@@ -2,7 +2,7 @@
 """Headline benchmark: DDIM images/sec, CIFAR-10 class-conditional UNet, CFG w=1 (cond/uncond batched as 2B
 rows in one UNet call), 100-step DDIM, batch 4096 per GPU (BASELINE.json configs[1]).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 A "step" is one denoising step of the real sampling loop over the whole per-GPU batch: one UNet forward on
 2*B rows plus the fused sampler update (diffusion.py:360-392).  100 such steps make B images, so
@@ -400,6 +400,24 @@ def train_step_block(timeout_s=120):
         return {"error": repr(e)[:400]}
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, x):
+    """--dump-outputs: the images the timed path left in x after its last step (what a caller of it receives), written
+    as out_dir/samples.npy in float32 so that two builds can be compared on the same seeded inputs.  A batch above
+    DUMP_MAX_BYTES is cut to a fixed, seeded subset of its images, kept in batch order."""
+    import numpy as np
+    import torch
+    x = x.detach().float().cpu()
+    per_image = x[0].numel() * 4
+    if x.shape[0] * per_image > DUMP_MAX_BYTES:
+        keep = torch.randperm(x.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_MAX_BYTES // per_image]
+        x = x[keep.sort().values]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "samples.npy"), x.numpy())
+
+
 def run_reference(args, rank):
     """--impl reference: the reference's own CPU implementation of the path on the host cores -- the unmodified
     reference staged under oracle/_ref (kind "reference"); the oracle port (kind "port") only if it is absent --
@@ -413,7 +431,9 @@ def run_reference(args, rank):
     g = torch.Generator().manual_seed(1234)
     x_t = torch.randn(B, 3, 32, 32, generator=g)
     label = torch.randint(10, (B,), generator=g) + 1
-    kind, _, dt, n = cpu_reference_trajectory(net.state_dict(), x_t, label, args.warmup, args.steps)
+    kind, x_last, dt, n = cpu_reference_trajectory(net.state_dict(), x_t, label, args.warmup, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x_last)
     val = B / (dt * T_STEPS)
     line = {"metric": METRIC, "value": val, "unit": "images/s", "n_gpus": args.gpus, "steps": n,
             "warmup": args.warmup, "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -493,6 +513,8 @@ def run_b200(args, rank, world, local_rank):
         ev1.record(stream)
         barrier()
     launches = L.vdt_kernel_launches() - n0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, x)
     ms = torch.tensor([ev0.elapsed_time(ev1)], device=device, dtype=torch.float64)
     per_rank = None
     if world > 1:
@@ -622,6 +644,8 @@ def main():
     ap.add_argument("--max-rows", type=int, default=int(os.environ.get("VDT_MAX_ROWS", "1024")))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train-step", action="store_true", help="skip the BASELINE configs[4] training-step block of the N=1 line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the images of the last timed step (rank 0) to DIR/samples.npy, float32, at most 64 MB")
     ap.add_argument("--train-step-child", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))

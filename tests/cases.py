@@ -5,7 +5,17 @@ the build container) and by the CPU / GPU tests (which run the oracle and the CU
 on the very same inputs).  Everything is regenerated from integer seeds with CPU
 generators, so only outputs need to be stored under ``tests/golden/``.
 """
+import zlib
+
+import numpy as np
 import torch
+
+
+def golden_sample_index(numel, n, key):
+    """Sorted flat positions of a fixed sample of n of an output's numel entries, seeded by ``key``: what a fixture keeps of
+    an output too large to store in full."""
+    g = torch.Generator().manual_seed(zlib.crc32(key.encode()) & 0x7fffffff)
+    return torch.randperm(numel, generator=g)[:n].sort().values.numpy().astype(np.int32)
 
 
 def _cfg(in_channels=3, hid=64, out_channels=3, mult=(1, 2), nrb=2, attn=(False, True),
@@ -27,7 +37,8 @@ CELEBA = _cfg(hid=192, out_channels=6, mult=(1, 2, 3, 4), nrb=3, attn=(False, Tr
 
 UNET_CASES = {
     # small: two levels, concat widths 192/256/128 (6-channel groups straddling the concat seam)
-    "small_cond": dict(cfg=_cfg(num_classes=10), seed=11, B=3, res=16, labels=[0, 3, 10],
+    # trace_keep: the fixture stores each traced feature map at that many seeded positions (golden_sample_index)
+    "small_cond": dict(cfg=_cfg(num_classes=10), seed=11, B=3, res=16, labels=[0, 3, 10], trace_keep=4096,
                        trace=["in_conv", "downsamples.level_0.0", "downsamples.level_0.2",
                               "downsamples.level_1.0", "middle", "upsamples.level_1.0",
                               "upsamples.level_1.3", "upsamples.level_0.2"]),
@@ -123,11 +134,12 @@ FULL_CASES = {
     # configs[0]: cifar10_uncond.json, x0-prediction, fixed_large, 10-step DDIM, batch 16
     "cifar10_uncond_ddim10": dict(cfg=CIFAR_UNCOND, init_seed=0, dezero_seed=7, B=16, T=10, model_out_type="x0",
                                   var_type="fixed_large", intp_frac=None, w_guide=0.0, use_ddim=True, noise_seed=1234,
-                                  labelled=False, keep_rows=16),
+                                  labelled=False, keep_rows=16, keep_entries=4096),
+    # (per-step model outputs: the first keep_rows rows, stored at keep_entries seeded positions of a step, golden_sample_index)
     # configs[1] at B=8: cifar10_cond.json, v-prediction, CFG w=1 (16 UNet rows per step), 100-step DDIM
     "cifar10_cond_cfg_ddim100": dict(cfg=CIFAR_COND, init_seed=0, dezero_seed=7, B=8, T=100, model_out_type="v",
                                      var_type="fixed_medium", intp_frac=0.3, w_guide=1.0, use_ddim=True, noise_seed=1234,
-                                     labelled=True, keep_rows=4),
+                                     labelled=True, keep_rows=4, keep_entries=1024),
 }
 
 

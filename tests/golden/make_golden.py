@@ -33,7 +33,7 @@ from v_diffusion.functions import get_timestep_embedding  # noqa: E402
 
 from oracle.unet_ref import make_state_dict, state_dict_shapes  # noqa: E402
 from tests.cases import (UNET_CASES, SAMPLE_CASES, FULL_CASES, TRAIN_CASES, build_inputs, build_sample_inputs,  # noqa: E402
-                         build_full_inputs, full_state_dict, build_train_inputs)
+                         build_full_inputs, full_state_dict, build_train_inputs, golden_sample_index)
 
 torch.set_num_threads(os.cpu_count())
 
@@ -67,7 +67,11 @@ def main():
             h.remove()
         arrs = {"out": out.numpy()}
         for k, v in feats.items():
-            arrs["trace:" + k] = v.numpy()
+            v = v.numpy()
+            if case.get("trace_keep"):                  # a seeded sample of the feature map keeps the fixture small
+                idx = golden_sample_index(v.size, case["trace_keep"], "trace:" + k)
+                arrs["trace_index:" + k], v = idx, v.reshape(-1)[idx]
+            arrs["trace:" + k] = v
         np.savez_compressed(os.path.join(HERE, f"unet_{name}.npz"), **arrs)
         print(name, tuple(out.shape), float(out.abs().mean()), float(out.abs().max()))
 
@@ -138,7 +142,9 @@ def main():
         x = diff.p_sample(rec, shape=tuple(noise.shape), noise=noise, label=label, device="cpu",
                           seed=case["noise_seed"], use_ddim=case["use_ddim"])
         mo = torch.stack(outs)
-        np.savez_compressed(os.path.join(HERE, f"full_{name}.npz"), out=x.numpy(), model_out=mo.numpy())
+        idx = golden_sample_index(mo[0].numel(), case["keep_entries"], f"full_{name}")
+        np.savez_compressed(os.path.join(HERE, f"full_{name}.npz"), out=x.numpy(), model_out=mo.reshape(len(mo), -1)[:, torch.from_numpy(idx).long()].numpy(),
+                            model_out_index=idx)
         print("full", name, tuple(x.shape), tuple(mo.shape), float(x.abs().mean()), float(x.abs().max()),
               f"{time.time() - t0:.1f}s")
 

@@ -500,7 +500,8 @@ def test_full_trajectory_vs_reference_golden(golden_dir, name, operand):
     validation mode (fp16x3): final samples within 1e-3."""
     case = FULL_CASES[name]
     g = np.load(os.path.join(golden_dir, f"full_{name}.npz"))
-    ref, ref_mo = torch.from_numpy(g["out"]), torch.from_numpy(g["model_out"])
+    ref, ref_mo = torch.from_numpy(g["out"]), torch.from_numpy(g["model_out"])       # model_out: seeded sample of each step
+    idx = torch.from_numpy(g["model_out_index"]).long()
     net = _full_model(case, operand)
     diff = _full_diffusion(case)
     noise, label = build_full_inputs(case)
@@ -515,7 +516,7 @@ def test_full_trajectory_vs_reference_golden(golden_dir, name, operand):
 
     def wrapped(x, t, y):
         o = net(x, t, y)
-        rec.append(o[:keep].cpu())
+        rec.append(o[:keep].cpu().reshape(-1)[idx])
         return o
     out2 = diff.p_sample(wrapped, tuple(noise.shape), noise=noise, label=label, device="cuda", use_ddim=True)
     assert (out2 - out).abs().max().item() <= 1e-5
@@ -776,3 +777,27 @@ def test_optimizer_step_vs_torch_adamw_and_reference_ema():
     assert worst <= 2e-6
     again = opt.step(grads).item()
     assert again == opt.step(grads).item()                              # fixed-order norm reduction
+
+
+def test_bench_dump_outputs_is_the_timed_trajectory(tmp_path):
+    """bench.py --dump-outputs writes what its timed loop computed: with --steps 100 the timed loop is exactly one 100-step DDIM
+    trajectory from the bench's seeded noise, so the dump equals GaussianDiffusion.p_sample on the bench's model and inputs."""
+    import subprocess
+    import sys
+    import bench
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    B = 4
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--batch", str(B), "--steps", "100", "--warmup", "3",
+                        "--no-cpu-baseline", "--no-train-step", "--dump-outputs", str(tmp_path)], cwd=root, capture_output=True,
+                       text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    got = torch.from_numpy(np.load(tmp_path / "samples.npy"))
+    device = torch.device("cuda", 0)
+    net, diff = bench.build_model(device, seed=0)
+    g = torch.Generator(device=device).manual_seed(1234)                # bench.run_b200's draws for rank 0
+    noise = torch.randn(B, 3, 32, 32, device=device, generator=g)
+    label = torch.randint(10, (B,), device=device, generator=g) + 1
+    want = diff.p_sample(net, (B, 3, 32, 32), noise=noise.cpu(), label=label.cpu(), device=device, use_ddim=True)
+    err = (got - want.cpu()).abs().max().item()
+    print(f"bench dump vs p_sample: max-abs {err:.3e}")
+    assert got.dtype == torch.float32 and got.shape == want.shape and err <= 1e-3

@@ -38,6 +38,8 @@ def test_unet_forward_matches_reference(golden_dir, name):
                 got = trace["middle.2"]
             elif got is None:
                 got = trace[mod + ".0"]
+            if "trace_index:" + mod in g.files:                 # stored at a seeded sample of positions (cases.golden_sample_index)
+                got = got.reshape(-1)[torch.from_numpy(g["trace_index:" + mod]).long()]
             r = torch.from_numpy(g[key])
             assert (got - r).abs().max().item() <= 2e-4 * max(1.0, r.abs().max().item()), mod
 
@@ -103,8 +105,10 @@ def test_full_trajectory_configs0_matches_reference(golden_dir):
                    T=case["T"], model_out_type=case["model_out_type"], w_guide=case["w_guide"], use_ddim=True,
                    var_type=case["var_type"], record=rec)
     assert (out - torch.from_numpy(g["out"])).abs().max().item() <= 5e-4
-    mo = torch.from_numpy(g["model_out"])
+    mo, idx = torch.from_numpy(g["model_out"]), torch.from_numpy(g["model_out_index"]).long()   # seeded sample of each step
+    assert len(rec) == mo.shape[0] == case["T"]
     for i, (ti, o) in enumerate(rec):
+        o = o[:case["keep_rows"]].reshape(-1)[idx]
         assert ((o - mo[i]).norm() / mo[i].norm()).item() <= 1e-4
 
 
@@ -122,9 +126,11 @@ def test_full_trajectory_configs1_matches_reference(golden_dir):
                    T=case["T"], model_out_type="v", w_guide=1.0, use_ddim=True, var_type="fixed_medium", intp_frac=0.3,
                    record=rec)
     assert (out - torch.from_numpy(g["out"])[:2]).abs().max().item() <= 1e-3
-    mo = torch.from_numpy(g["model_out"])                       # (100, 4, 3, 32, 32): rows of the first two images
+    mo = torch.from_numpy(g["model_out"])                       # (100, keep_entries): seeded sample of the rows of the first two images
+    idx = torch.from_numpy(g["model_out_index"]).long()
     assert len(rec) == 100
     for i, (ti, o) in enumerate(rec):
+        o = o.reshape(-1)[idx]
         assert ((o - mo[i]).norm() / mo[i].norm()).item() <= 2e-4, ti
 
 

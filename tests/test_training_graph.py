@@ -462,37 +462,36 @@ def test_autograd_mode_runs_the_reference_training_lines_unchanged(contract_ops)
         net(x0, t, y)
 
 
-def test_reference_train_loss_drives_the_autograd_unet(contract_ops):
-    """The UNMODIFIED reference's GaussianDiffusion.train_loss (oracle/_ref, staged from /root/reference in the build
-    container) called with this package's UNet (autograd mode, contract stand-in for the kernels) as its denoise_fn, then
-    loss.mean().backward() as in Trainer.step: same loss and same gradients as with the oracle UNet as denoise_fn."""
-    from oracle import stage_ref
-    if not stage_ref.staged():
-        pytest.skip("oracle/_ref is staged only where /root/reference exists")
-    ref = stage_ref.load()
-    cfg = _cfg(hid=64, mult=(1, 1), nrb=1, attn=(True, False), num_classes=10)
-    sd, net = _build(cfg, seed=6)
+def test_reference_train_loss_drives_the_autograd_unet(contract_ops, golden_dir):
+    """This package's UNet (autograd mode, contract stand-in for the kernels) as the denoise_fn of train_loss, then
+    loss.mean().backward() as in Trainer.step: the per-sample loss and every parameter's gradient against what the UNMODIFIED
+    reference's own UNet + GaussianDiffusion.train_loss + autograd produced on the same seeded inputs
+    (tests/golden/train_grads_small.npz, made by tests/golden/make_train_grad_golden.py).  train_loss is the oracle's
+    restatement, which test_oracle_golden.py pins to the reference's on its own fixtures."""
+    import numpy as np
+    from oracle import train_loss
+    from tests.cases import TRAIN_GRAD_CASE, build_train_grad_inputs, grad_probe
+    case = TRAIN_GRAD_CASE
+    g = np.load(os.path.join(golden_dir, "train_grads_small.npz"))
+    _, net = _build(case["cfg"], case["wseed"])
     net.autograd = True
     net.train()
-    diffusion = ref.GaussianDiffusion(logsnr_fn=ref.get_logsnr_schedule("cosine", logsnr_min=-20., logsnr_max=20.), sample_timesteps=100,
-                                      model_out_type="v", model_var_type="fixed_medium", reweight_type="snr_trunc", loss_type="mse",
-                                      intp_frac=0.3, w_guide=0.1, p_uncond=0.1)
-    g = torch.Generator().manual_seed(13)
-    x0 = torch.randn(2, 3, 8, 8, generator=g).clamp(-1, 1)
-    t = torch.rand(2, generator=g, dtype=torch.float64)
-    noise = torch.randn(2, 3, 8, 8, generator=g)
-    y = torch.tensor([7, 1])
-    loss = diffusion.train_loss(lambda a, b, c: net(a.double(), b, c).float(), x_0=x0, t=t, y=y.clone(), noise=noise)
-    assert loss.shape == (2,)
+    x0, t, noise, y = build_train_grad_inputs(case)
+    loss, _ = train_loss(lambda a, b, c: net(a.double(), b, c).float(), x0, t, y.clone(), noise,
+                         model_out_type=case["model_out_type"], reweight_type=case["reweight_type"])
+    assert loss.shape == (case["B"],)
     loss.mean().backward()
-    ref_p = {k: v.clone().requires_grad_(True) for k, v in sd.items()}
-    want = diffusion.train_loss(lambda a, b, c: _unet_forward(ref_p, cfg, a, b, c, None), x_0=x0, t=t, y=y.clone(), noise=noise)
-    want.mean().backward()
-    assert torch.allclose(loss.detach(), want.detach(), rtol=1e-5)
-    for k, p in net.named_parameters():
-        w = ref_p[k].grad
-        err = (p.grad.double() - w.double()).norm().item() / (w.double().norm().item() + 2e-5 * math.sqrt(w.numel()))
-        assert err <= 2e-4, (k, err)
+    np.testing.assert_allclose(loss.detach().numpy(), g["loss"], rtol=1e-5)
+    params = dict(net.named_parameters())
+    names = [str(n) for n in g["names"]]
+    assert sorted(names) == sorted(params)
+    for k in names:
+        gr = params[k].grad.double()
+        n_ref = float(g["norm/" + k])
+        assert abs(gr.norm().item() - n_ref) <= 1e-4 * n_ref + 1e-9, k
+        assert abs((gr * grad_probe(k, gr.shape)).sum().item() - float(g["proj/" + k])) <= 1e-3 * n_ref + 1e-9, k
+        if ("full/" + k) in g.files:
+            assert (gr - torch.from_numpy(g["full/" + k]).double()).norm().item() <= 1e-4 * n_ref + 1e-9, k
 
 
 def test_gpu_worker_and_bench_block_dry_run():
@@ -596,3 +595,21 @@ def test_bench_train_step_block_never_breaks_the_bench_line():
     import bench
     out = bench.train_step_block(timeout_s=120)
     assert set(out) == {"error"} and "child rc=" in out["error"], out
+
+
+def test_bench_dump_outputs_is_float32_and_a_fixed_sample_under_the_cap(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 whatever the input dtype; above the size cap, the same seeded subset of the images on
+    every call, kept in batch order."""
+    import numpy as np
+    import bench
+    x = torch.randn(12, 3, 8, 8, generator=torch.Generator().manual_seed(3), dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path / "all"), x)
+    full = np.load(tmp_path / "all" / "samples.npy")
+    assert full.dtype == np.float32 and np.array_equal(full, x.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 5 * x[0].numel() * 4)
+    bench.dump_outputs(str(tmp_path / "a"), x)
+    bench.dump_outputs(str(tmp_path / "b"), x)
+    a, b = np.load(tmp_path / "a" / "samples.npy"), np.load(tmp_path / "b" / "samples.npy")
+    assert a.shape == (5, 3, 8, 8) and np.array_equal(a, b)
+    rows = [next(i for i in range(12) if np.array_equal(full[i], r)) for r in a]
+    assert rows == sorted(rows) and len(set(rows)) == 5

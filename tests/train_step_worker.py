@@ -152,24 +152,14 @@ def dropout(case, B, operand):
     return dict(reproducible=same, finite=finite, seed_changes_output=rel(c, a), eval_differs=rel(e, a), out_bias_grad_rel=bias_rel)
 
 
-def grad_golden(case, B, operand):
-    """TrainingStep.loss_and_grads on the kernels against the gradients the UNMODIFIED reference's own UNet / train_loss /
-    autograd produced (tests/golden/train_grads_small.npz, made by tests/golden/make_train_grad_golden.py): per-sample loss,
-    every parameter gradient's norm and probe projection, the small tensors in full.  (B comes from the fixture.)"""
+def vs_grad_fixture(case, loss, grads):
+    """Per-sample loss and parameter gradients against tests/golden/train_grads_<case>.npz, made by the UNMODIFIED reference's own
+    UNet / train_loss / autograd (tests/golden/make_train_grad_golden.py): every gradient's norm and probe projection, the small
+    tensors in full."""
     import numpy as np
-    from tests.cases import TRAIN_GRAD_CASES, build_train_grad_inputs, grad_probe
-    c = TRAIN_GRAD_CASES[case]                                         # "small" | "cifar" (cifar10_cond.json's own network)
-    cfg = c["cfg"]
+    from tests.cases import grad_probe
     g = np.load(os.path.join(ROOT, "tests", "golden", f"train_grads_{case}.npz"))
-    sd, net = build(cfg, c["wseed"], operand)
-    net.train()
-    diff = GaussianDiffusion(get_logsnr_schedule("cosine", -20., 20.), 1000, c["model_out_type"], "fixed_medium", c["reweight_type"],
-                             "mse", intp_frac=0.3, p_uncond=0.1)
-    ts = TrainingStep(net, diff, timesteps=0)
-    x0, t, noise, y = build_train_grad_inputs(c)
-    loss, grads = ts.loss_and_grads(x0.cuda(), y.cuda(), t=t.cuda(), noise=noise.cuda())
-    torch.cuda.synchronize()
-    loss_rel = float(np.abs(loss.cpu().numpy() - g["loss"]).max() / np.abs(g["loss"]).max())
+    loss_rel = float(np.abs(loss.detach().cpu().numpy() - g["loss"]).max() / np.abs(g["loss"]).max())
     norm_err, proj_err, full_err = {}, {}, {}
     for k in (str(n) for n in g["names"]):
         gr = grads[k].detach().double().cpu()
@@ -184,43 +174,41 @@ def grad_golden(case, B, operand):
                 worst=dict(norm=top(norm_err), proj=top(proj_err), full=top(full_err)))
 
 
+def grad_golden(case, B, operand):
+    """TrainingStep.loss_and_grads on the kernels against the reference's gradient fixture (vs_grad_fixture).  (B comes from the
+    fixture.)"""
+    from tests.cases import TRAIN_GRAD_CASES, build_train_grad_inputs
+    c = TRAIN_GRAD_CASES[case]                                         # "small" | "cifar" (cifar10_cond.json's own network)
+    sd, net = build(c["cfg"], c["wseed"], operand)
+    net.train()
+    diff = GaussianDiffusion(get_logsnr_schedule("cosine", -20., 20.), 1000, c["model_out_type"], "fixed_medium", c["reweight_type"],
+                             "mse", intp_frac=0.3, p_uncond=0.1)
+    ts = TrainingStep(net, diff, timesteps=0)
+    x0, t, noise, y = build_train_grad_inputs(c)
+    loss, grads = ts.loss_and_grads(x0.cuda(), y.cuda(), t=t.cuda(), noise=noise.cuda())
+    torch.cuda.synchronize()
+    return vs_grad_fixture(case, loss, grads)
+
+
 def autograd_step(case, B, operand):
-    """UNet.autograd = True: the UNMODIFIED reference's GaussianDiffusion.train_loss (oracle/_ref) with this package's UNet
-    as denoise_fn on the GPU, then loss.mean().backward() as in Trainer.step (train_utils.py:149-151) -- loss and every
-    parameter's .grad against the same lines with the oracle UNet on the CPU."""
-    from oracle import stage_ref
-    if not stage_ref.staged():
-        return dict(skipped="oracle/_ref not staged")
-    ref = stage_ref.load()
-    cfg, R = CASES[case]["cfg"], CASES[case]["res"]
-    sd, net = build(cfg, 37, operand)
+    """UNet.autograd = True on the GPU as the denoise_fn of train_loss (the oracle's restatement, pinned to the reference's), then
+    loss.mean().backward() as in Trainer.step (train_utils.py:149-151): loss and every parameter's .grad against the reference's
+    gradient fixture (vs_grad_fixture).  (B comes from the fixture.)"""
+    from tests.cases import TRAIN_GRAD_CASES, build_train_grad_inputs
+    c = TRAIN_GRAD_CASES[case]
+    sd, net = build(c["cfg"], c["wseed"], operand)
     net.autograd = True
     net.train()
-    diffusion = ref.GaussianDiffusion(logsnr_fn=ref.get_logsnr_schedule("cosine", logsnr_min=-20., logsnr_max=20.), sample_timesteps=100,
-                                      model_out_type="v", model_var_type="fixed_medium", reweight_type="snr_trunc", loss_type="mse",
-                                      intp_frac=0.3, w_guide=0.1, p_uncond=0.1)
-    g = torch.Generator().manual_seed(55)
-    x0 = torch.randn(B, cfg["in_channels"], R, R, generator=g).clamp(-1, 1)
-    t = torch.rand(B, generator=g, dtype=torch.float64)
-    noise = torch.randn(x0.shape, generator=g)
-    y = torch.randint(1, cfg["num_classes"] + 1, (B,), generator=g)
+    x0, t, noise, y = build_train_grad_inputs(c)
     with torch.enable_grad():
-        loss = diffusion.train_loss(net, x_0=x0.cuda(), t=t.cuda(), y=y.clone().cuda(), noise=noise.cuda())
+        loss, _ = oracle_train_loss(lambda a, b, yy: net(a.cuda(), b.cuda(), yy.cuda()).cpu(), x0, t, y.clone(), noise,
+                                    model_out_type=c["model_out_type"], reweight_type=c["reweight_type"])
         loss.mean().backward()
     torch.cuda.synchronize()
-    ref_p = {k: v.clone().requires_grad_(True) for k, v in sd.items()}
-    with torch.enable_grad():
-        want = diffusion.train_loss(lambda a, b, c: _unet_forward(ref_p, cfg, a, b, c, None), x_0=x0, t=t, y=y.clone(), noise=noise)
-        want.mean().backward()
-    errs = {}
-    for k, p in net.named_parameters():
-        w = ref_p[k].grad
-        errs[k] = rel(p.grad, w, floor=1e-7 * math.sqrt(w.numel()))
-    worst = sorted(errs.items(), key=lambda kv: -kv[1])[:3]
+    res = vs_grad_fixture(case, loss, {k: p.grad for k, p in net.named_parameters()})
     with torch.no_grad():
         sampled = net(x0.cuda(), t.cuda(), y.cuda())                       # no grad mode: still the plan path (dropout 0 here)
-    return dict(loss_rel=rel(loss, want), grad_rel_worst=worst[0][1], worst=worst, grad_rel_median=sorted(errs.values())[len(errs) // 2],
-                plan_path_finite=bool(torch.isfinite(sampled).all()))
+    return dict(res, plan_path_finite=bool(torch.isfinite(sampled).all()))
 
 
 if __name__ == "__main__":
