@@ -190,7 +190,7 @@ int vdt_op_conv(const void* x_16_nhwc, int32_t batch, int32_t h, int32_t w, int3
  *        dy 16-bit NHWC [B, H, W, cout], w fp32 OIHW [cout, cin, k, k].
  * wgrad: dW fp32 OIHW [cout, cin, k, k] = sum over pixels of dY[p][co] * X[p + tap][ci] (tcgen05, both operands MN-major,
  *        K split over CTAs with a fixed-order reduction); optional dbias fp32 [cout] = sum over pixels of dY.  x, dy 16-bit
- *        NHWC.  Needs cout % 128 == 0, cin % 64 == 0 and feature maps that tile into 128-pixel boxes. */
+ *        NHWC.  Needs cout % 64 == 0, cin % 64 == 0 and feature maps that tile into 128-pixel boxes. */
 int vdt_op_conv_dgrad(const void* dy_16_nhwc, int32_t batch, int32_t h, int32_t w, int32_t cin, const float* w_oihw, int32_t cout,
                       int32_t ksize, float* dx_nhwc, int32_t f16, void* stream);
 int vdt_op_conv_wgrad(const void* x_16_nhwc, const void* dy_16_nhwc, int32_t batch, int32_t h, int32_t w, int32_t cin, int32_t cout,
@@ -213,7 +213,7 @@ int vdt_op_groupnorm_dropout(const void* src1, int32_t c1, int32_t batch, int32_
                              const float* beta, int32_t silu, void* out_act_16, int32_t f16, float drop_p, uint64_t seed,
                              int32_t layer, void* stream);
 /* Backward of norm -> FiLM -> SiLU -> dropout (the activation chain of a ResidualBlock, unet.py:131-135, 143-146): x and
- * grad_out fp32 [batch, h*w, c] (c in 128 / 256 / 512 / 1024), grad_out = gradient at the activation; film = null or
+ * grad_out fp32 [batch, h*w, c] (c % 64 == 0, c <= 2048), grad_out = gradient at the activation; film = null or
  * [batch][2c] (shift | scale per sample); (drop_p, seed, layer) name the forward's dropout stream (drop_p = 0: none).
  * Writes grad_x [batch, h*w, c], grad_gamma / grad_beta [c] and, when given, grad_film [batch][2c] (d shift | d scale).
  * Replaces autograd through F.group_norm / F.silu / F.dropout (torch/nn/functional.py) on this chain. */

@@ -13,6 +13,11 @@
 // The 16-bit rounding of the forward output is treated as the identity (straight-through).  The dropout mask is
 // regenerated from the forward's Philox stream (same counter / key / word per element), never stored.
 // All reductions run in a fixed order: results are bit-reproducible run to run.
+//
+// Channel layout (as the forward, groupnorm.cu: launch_groupnorm): a thread owns VEC channels of one group -- 4 when the
+// group width is a multiple of 4, else 2 -- and a row of CV = CB / VEC threads covers one channel block of CB channels
+// (whole groups); the kThreads / CV rows of a CTA stride over the pixels.  C up to 256 four-wide vectors is one channel
+// block; wider C, or a row that would leave more than a quarter of the CTA idle, is split over gridDim.z channel blocks.
 #include "kernels.cuh"
 #include "ptx.cuh"
 
@@ -23,24 +28,43 @@ constexpr int kGroups = 32;
 constexpr float kEps = 1e-6f;
 constexpr int kThreads = 256;
 
-// (mean, rstd) of every group of one sample: fp32 partial sums per thread, combined in fp64 (as the forward's fallback pass)
-__global__ void __launch_bounds__(kThreads) gn_stats_kernel(const float* __restrict__ x, float2* __restrict__ meanrstd, int HW, int C) {
+template <int VEC>
+__device__ __forceinline__ void load_vec(const float* src, float (&v)[VEC]) {
+    if constexpr (VEC == 4) {
+        const float4 t = *reinterpret_cast<const float4*>(src);
+        v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+    } else {
+        const float2 t = *reinterpret_cast<const float2*>(src);
+        v[0] = t.x; v[1] = t.y;
+    }
+}
+
+// (mean, rstd) of every group of one channel block of one sample: fp32 partial sums per thread, combined in fp64 (as the
+// forward's fallback pass).  grid (B, channel blocks)
+template <int VEC>
+__global__ void __launch_bounds__(kThreads) gn_stats_kernel(const float* __restrict__ x, float2* __restrict__ meanrstd, int HW, int C, int CB) {
     extern __shared__ float2 part[];                       // [kThreads]
     const int b = blockIdx.x, tid = threadIdx.x;
-    const int CV = C / 4, PPH = kThreads / CV;             // channel vectors, pixel phases (host: CV divides kThreads)
+    const int CV = CB / VEC, PPH = kThreads / CV;          // channel vectors, pixel phases (host: CV <= kThreads)
     const int cv = tid % CV, pp = tid / CV;
-    const float* src = x + static_cast<size_t>(b) * HW * C + cv * 4;
+    const float* src = x + static_cast<size_t>(b) * HW * C + blockIdx.y * CB + cv * VEC;
     float s = 0.f, ss = 0.f;
     if (pp < PPH)
         for (int pix = pp; pix < HW; pix += PPH) {
-            const float4 v = *reinterpret_cast<const float4*>(src + static_cast<size_t>(pix) * C);
-            s += (v.x + v.y) + (v.z + v.w);
-            ss = fmaf(v.x, v.x, fmaf(v.y, v.y, fmaf(v.z, v.z, fmaf(v.w, v.w, ss))));
+            float v[VEC];
+            load_vec<VEC>(src + static_cast<size_t>(pix) * C, v);
+            if constexpr (VEC == 4) {
+                s += (v[0] + v[1]) + (v[2] + v[3]);
+                ss = fmaf(v[0], v[0], fmaf(v[1], v[1], fmaf(v[2], v[2], fmaf(v[3], v[3], ss))));
+            } else {
+                s += v[0] + v[1];
+                ss = fmaf(v[0], v[0], fmaf(v[1], v[1], ss));
+            }
         }
     part[tid] = make_float2(s, ss);
     __syncthreads();
-    if (tid < kGroups) {
-        const int cpg = C / kGroups, vpg = cpg / 4;
+    const int cpg = C / kGroups, vpg = cpg / VEC, G = CB / cpg;
+    if (tid < G) {
         double ds = 0.0, dss = 0.0;
         for (int ph = 0; ph < PPH; ++ph)
             for (int j = 0; j < vpg; ++j) {
@@ -51,29 +75,33 @@ __global__ void __launch_bounds__(kThreads) gn_stats_kernel(const float* __restr
         const double mean = ds / n;
         double var = dss / n - mean * mean;
         if (var < 0.0) var = 0.0;
-        meanrstd[b * kGroups + tid] = make_float2(static_cast<float>(mean), static_cast<float>(1.0 / sqrt(var + static_cast<double>(kEps))));
+        meanrstd[b * kGroups + blockIdx.y * G + tid] = make_float2(static_cast<float>(mean), static_cast<float>(1.0 / sqrt(var + static_cast<double>(kEps))));
     }
 }
 
-struct Elem { float xhat[4], dz[4]; };
+template <int VEC>
+struct Elem { float xhat[VEC], dz[VEC]; };
 
 // The per-element chain shared by both passes: recompute xhat, z and the activation's derivative, apply the mask.
+template <int VEC>
 struct Chain {
     float rstd, mean;
-    float ga[4], be[4], fs[4], fb[4];
+    float ga[VEC], be[VEC], fs[VEC], fb[VEC];
     int silu;
+    int word0;                  // 2-wide vectors: 1 -> Philox words 2, 3 (word ((c >> 1) & 1) * 2 + i, as groupnorm.cu)
     bool drop; uint32_t thr; float dscale; unsigned long long seed; int layer;
-    __device__ __forceinline__ Elem eval(const float4 xv, const float4 gv, unsigned long long e) const {
-        const float x[4] = {xv.x, xv.y, xv.z, xv.w}, g[4] = {gv.x, gv.y, gv.z, gv.w};
+    // e: element index of the vector's first channel; one Philox call per 4 elements (counter e >> 2) as in the forward
+    __device__ __forceinline__ Elem<VEC> eval(const float (&x)[VEC], const float (&g)[VEC], unsigned long long e) const {
         uint32_t w[4] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu};
         if (drop) {
             const uint4 r = philox4x32(make_uint4(static_cast<uint32_t>(e >> 2), static_cast<uint32_t>(e >> 34), static_cast<uint32_t>(layer), 0x44524f50u),
                                        make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)));
             w[0] = r.x; w[1] = r.y; w[2] = r.z; w[3] = r.w;
+            if (VEC == 2 && word0) { w[0] = r.z; w[1] = r.w; }
         }
-        Elem o;
+        Elem<VEC> o;
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
+        for (int i = 0; i < VEC; ++i) {
             o.xhat[i] = (x[i] - mean) * rstd;
             const float z = fs[i] * (ga[i] * o.xhat[i] + be[i]) + fb[i];
             float d = g[i];
@@ -91,7 +119,7 @@ struct Chain {
 struct BwdArgs {
     const float* x; const float* grad_out; const float2* meanrstd;
     const float* gamma; const float* beta; const float* film;      // film: [B][2C] (shift | scale) or null
-    int B, HW, C, silu, slabs;
+    int B, HW, C, CB, silu, slabs;                                 // CB: channels of one channel block (gridDim.z = C / CB)
     float drop_p; unsigned long long seed; int layer;
     float2* partial;            // [B][slabs][C] (sum dz, sum dz * xhat)
     float2* ab;                 // [B][C] the same, summed over the slabs
@@ -99,17 +127,19 @@ struct BwdArgs {
     float* grad_x; float* grad_gamma; float* grad_beta; float* grad_film;
 };
 
-__device__ __forceinline__ Chain make_chain(const BwdArgs& p, int b, int c) {
-    Chain ch;
+template <int VEC>
+__device__ __forceinline__ Chain<VEC> make_chain(const BwdArgs& p, int b, int c) {
+    Chain<VEC> ch;
     const float2 st = p.meanrstd[b * kGroups + c / (p.C / kGroups)];
     ch.mean = st.x; ch.rstd = st.y;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < VEC; ++i) {
         ch.ga[i] = p.gamma[c + i]; ch.be[i] = p.beta[c + i];
         ch.fb[i] = p.film ? p.film[static_cast<size_t>(b) * 2 * p.C + c + i] : 0.f;
         ch.fs[i] = p.film ? 1.f + p.film[static_cast<size_t>(b) * 2 * p.C + p.C + c + i] : 1.f;
     }
     ch.silu = p.silu;
+    ch.word0 = VEC == 4 ? 0 : (c >> 1) & 1;
     ch.drop = p.drop_p > 0.f;
     ch.thr = ch.drop ? static_cast<uint32_t>(fminf(p.drop_p, 0.99999994f) * 4294967296.0f) : 0u;
     ch.dscale = ch.drop ? 1.f / (1.f - p.drop_p) : 1.f;
@@ -117,32 +147,38 @@ __device__ __forceinline__ Chain make_chain(const BwdArgs& p, int b, int c) {
     return ch;
 }
 
-// pass 1: grid (slabs, B); a CTA owns the pixels [slab * HW / slabs, ...) of one sample
+// pass 1: grid (slabs, B, channel blocks); a CTA owns the pixels [slab * HW / slabs, ...) of one sample's channel block
+template <int VEC>
 __global__ void __launch_bounds__(kThreads) gn_bwd_reduce_kernel(const BwdArgs p) {
-    extern __shared__ float2 red[];                        // [kThreads][4]
+    extern __shared__ float2 red[];                        // [kThreads][VEC]
     const int b = blockIdx.y, slab = blockIdx.x, tid = threadIdx.x;
-    const int CV = p.C / 4, PPH = kThreads / CV;
-    const int cv = tid % CV, pp = tid / CV, c = cv * 4;
+    const int CV = p.CB / VEC, PPH = kThreads / CV;
+    const int cv = tid % CV, pp = tid / CV, c = blockIdx.z * p.CB + cv * VEC;
     const int p0 = static_cast<int>(static_cast<long long>(slab) * p.HW / p.slabs), p1 = static_cast<int>(static_cast<long long>(slab + 1) * p.HW / p.slabs);
-    float a[4] = {0.f, 0.f, 0.f, 0.f}, bc[4] = {0.f, 0.f, 0.f, 0.f};
+    float a[VEC], bc[VEC];
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) { a[i] = 0.f; bc[i] = 0.f; }
     if (pp < PPH) {
-        const Chain ch = make_chain(p, b, c);
+        const Chain<VEC> ch = make_chain<VEC>(p, b, c);
         for (int pix = p0 + pp; pix < p1; pix += PPH) {
             const size_t off = (static_cast<size_t>(b) * p.HW + pix) * p.C + c;
-            const Elem e = ch.eval(*reinterpret_cast<const float4*>(p.x + off), *reinterpret_cast<const float4*>(p.grad_out + off), off);
+            float xv[VEC], gv[VEC];
+            load_vec<VEC>(p.x + off, xv);
+            load_vec<VEC>(p.grad_out + off, gv);
+            const Elem<VEC> e = ch.eval(xv, gv, off);
 #pragma unroll
-            for (int i = 0; i < 4; ++i) { a[i] += e.dz[i]; bc[i] = fmaf(e.dz[i], e.xhat[i], bc[i]); }
+            for (int i = 0; i < VEC; ++i) { a[i] += e.dz[i]; bc[i] = fmaf(e.dz[i], e.xhat[i], bc[i]); }
         }
     }
 #pragma unroll
-    for (int i = 0; i < 4; ++i) red[tid * 4 + i] = make_float2(a[i], bc[i]);
+    for (int i = 0; i < VEC; ++i) red[tid * VEC + i] = make_float2(a[i], bc[i]);
     __syncthreads();
     if (tid < CV) {                                        // fixed order over the pixel phases
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
+        for (int i = 0; i < VEC; ++i) {
             float sa = 0.f, sb = 0.f;
-            for (int ph = 0; ph < PPH; ++ph) { const float2 t = red[(ph * CV + tid) * 4 + i]; sa += t.x; sb += t.y; }
-            p.partial[(static_cast<size_t>(b) * p.slabs + slab) * p.C + tid * 4 + i] = make_float2(sa, sb);
+            for (int ph = 0; ph < PPH; ++ph) { const float2 t = red[(ph * CV + tid) * VEC + i]; sa += t.x; sb += t.y; }
+            p.partial[(static_cast<size_t>(b) * p.slabs + slab) * p.C + c + i] = make_float2(sa, sb);
         }
     }
 }
@@ -191,28 +227,62 @@ __global__ void __launch_bounds__(256) gn_bwd_param_kernel(const BwdArgs p) {
     if (lane == 0) { p.grad_gamma[c] = static_cast<float>(dg); p.grad_beta[c] = static_cast<float>(db); }
 }
 
-// pass 2: dx
+// pass 2: dx; grid as pass 1
+template <int VEC>
 __global__ void __launch_bounds__(kThreads) gn_bwd_apply_kernel(const BwdArgs p) {
     const int b = blockIdx.y, slab = blockIdx.x, tid = threadIdx.x;
-    const int CV = p.C / 4, PPH = kThreads / CV;
-    const int cv = tid % CV, pp = tid / CV, c = cv * 4;
+    const int CV = p.CB / VEC, PPH = kThreads / CV;
+    const int cv = tid % CV, pp = tid / CV, c = blockIdx.z * p.CB + cv * VEC;
     if (pp >= PPH) return;
     const int p0 = static_cast<int>(static_cast<long long>(slab) * p.HW / p.slabs), p1 = static_cast<int>(static_cast<long long>(slab + 1) * p.HW / p.slabs);
-    const Chain ch = make_chain(p, b, c);
+    const Chain<VEC> ch = make_chain<VEC>(p, b, c);
     const float2 m = p.m12[b * kGroups + c / (p.C / kGroups)];
-    float k[4];
+    float k[VEC];
 #pragma unroll
-    for (int i = 0; i < 4; ++i) k[i] = ch.ga[i] * ch.fs[i];
+    for (int i = 0; i < VEC; ++i) k[i] = ch.ga[i] * ch.fs[i];
     for (int pix = p0 + pp; pix < p1; pix += PPH) {
         const size_t off = (static_cast<size_t>(b) * p.HW + pix) * p.C + c;
-        const Elem e = ch.eval(*reinterpret_cast<const float4*>(p.x + off), *reinterpret_cast<const float4*>(p.grad_out + off), off);
-        float4 o;
-        o.x = ch.rstd * (k[0] * e.dz[0] - m.x - e.xhat[0] * m.y);
-        o.y = ch.rstd * (k[1] * e.dz[1] - m.x - e.xhat[1] * m.y);
-        o.z = ch.rstd * (k[2] * e.dz[2] - m.x - e.xhat[2] * m.y);
-        o.w = ch.rstd * (k[3] * e.dz[3] - m.x - e.xhat[3] * m.y);
-        *reinterpret_cast<float4*>(p.grad_x + off) = o;
+        float xv[VEC], gv[VEC];
+        load_vec<VEC>(p.x + off, xv);
+        load_vec<VEC>(p.grad_out + off, gv);
+        const Elem<VEC> e = ch.eval(xv, gv, off);
+        if constexpr (VEC == 4) {
+            float4 o;
+            o.x = ch.rstd * (k[0] * e.dz[0] - m.x - e.xhat[0] * m.y);
+            o.y = ch.rstd * (k[1] * e.dz[1] - m.x - e.xhat[1] * m.y);
+            o.z = ch.rstd * (k[2] * e.dz[2] - m.x - e.xhat[2] * m.y);
+            o.w = ch.rstd * (k[3] * e.dz[3] - m.x - e.xhat[3] * m.y);
+            *reinterpret_cast<float4*>(p.grad_x + off) = o;
+        } else {
+            float2 o;
+            o.x = ch.rstd * (k[0] * e.dz[0] - m.x - e.xhat[0] * m.y);
+            o.y = ch.rstd * (k[1] * e.dz[1] - m.x - e.xhat[1] * m.y);
+            *reinterpret_cast<float2*>(p.grad_x + off) = o;
+        }
     }
+}
+
+// Vector width and channel block of a width C (C % 64 == 0: whole, even-width groups): the fewest channel blocks (whole
+// groups, at most kThreads vectors wide) whose pixel-phase rows keep at least 3/4 of a CTA's threads busy.  C = 128, 256,
+// 512 and 1024 (four-wide vectors dividing kThreads) take one block, the layout this kernel had before wider C existed.
+struct BwdLayout { int vec, cb; };
+BwdLayout bwd_layout(int C) {
+    const int cpg = C / kGroups, vec = (cpg % 4 == 0) ? 4 : 2;
+    int nblk = 1;
+    for (; nblk < kGroups; nblk *= 2) {
+        const int cv = C / nblk / vec;
+        if (cv <= kThreads && (kThreads / cv) * cv * 4 >= kThreads * 3) break;
+    }
+    return BwdLayout{vec, C / nblk};
+}
+
+template <int VEC>
+void launch_passes(const BwdArgs& p, const float* x, float2* mr, int nblk, cudaStream_t stream) {
+    gn_stats_kernel<VEC><<<dim3(p.B, nblk), kThreads, kThreads * sizeof(float2), stream>>>(x, mr, p.HW, p.C, p.CB);
+    gn_bwd_reduce_kernel<VEC><<<dim3(p.slabs, p.B, nblk), kThreads, kThreads * VEC * sizeof(float2), stream>>>(p);
+    gn_bwd_finalize_kernel<<<p.B, kThreads, p.C * sizeof(double2), stream>>>(p);
+    gn_bwd_param_kernel<<<(p.C + 7) / 8, 256, 0, stream>>>(p);
+    gn_bwd_apply_kernel<VEC><<<dim3(p.slabs, p.B, nblk), kThreads, 0, stream>>>(p);
 }
 
 }  // namespace
@@ -225,13 +295,14 @@ size_t groupnorm_backward_scratch_bytes(int B, int HW, int C, int* slabs_out) {
 }
 
 cudaError_t launch_groupnorm_backward(const GroupNormBwdParams& q, cudaStream_t stream) {
-    // a thread owns 4 channels of one group, a CTA row of threads covers all channels: C in {128, 256, 512, 1024}
-    if (q.C % (4 * kGroups) != 0 || q.C / 4 > kThreads || kThreads % (q.C / 4) != 0) return cudaErrorInvalidValue;
+    // every width the forward takes from one source: groups of an even channel count, at most 2048 channels
+    if (q.C < 2 * kGroups || q.C % (2 * kGroups) != 0 || q.C > 2048) return cudaErrorInvalidValue;
+    const BwdLayout lay = bwd_layout(q.C);
     int slabs = 1;
     groupnorm_backward_scratch_bytes(q.B, q.HW, q.C, &slabs);
     BwdArgs p{};
     p.x = q.x; p.grad_out = q.grad_out; p.gamma = q.gamma; p.beta = q.beta; p.film = q.film;
-    p.B = q.B; p.HW = q.HW; p.C = q.C; p.silu = q.silu; p.slabs = slabs;
+    p.B = q.B; p.HW = q.HW; p.C = q.C; p.CB = lay.cb; p.silu = q.silu; p.slabs = slabs;
     p.drop_p = q.drop_p; p.seed = q.drop_seed; p.layer = q.drop_layer;
     float2* s = static_cast<float2*>(q.scratch);
     p.partial = s; s += static_cast<size_t>(q.B) * slabs * q.C;
@@ -240,11 +311,9 @@ cudaError_t launch_groupnorm_backward(const GroupNormBwdParams& q, cudaStream_t 
     float2* mr = s;
     p.meanrstd = mr;
     p.grad_x = q.grad_x; p.grad_gamma = q.grad_gamma; p.grad_beta = q.grad_beta; p.grad_film = q.grad_film;
-    gn_stats_kernel<<<q.B, kThreads, kThreads * sizeof(float2), stream>>>(q.x, mr, q.HW, q.C);
-    gn_bwd_reduce_kernel<<<dim3(slabs, q.B), kThreads, kThreads * 4 * sizeof(float2), stream>>>(p);
-    gn_bwd_finalize_kernel<<<q.B, kThreads, q.C * sizeof(double2), stream>>>(p);
-    gn_bwd_param_kernel<<<(q.C + 7) / 8, 256, 0, stream>>>(p);
-    gn_bwd_apply_kernel<<<dim3(slabs, q.B), kThreads, 0, stream>>>(p);
+    const int nblk = q.C / lay.cb;
+    if (lay.vec == 4) launch_passes<4>(p, q.x, mr, nblk, stream);
+    else launch_passes<2>(p, q.x, mr, nblk, stream);
     return cudaGetLastError();
 }
 

@@ -134,8 +134,8 @@ struct GroupNormParams {
 };
 cudaError_t launch_groupnorm(const GroupNormParams& p, cudaStream_t stream);
 
-// Backward of GroupNorm -> FiLM -> SiLU -> dropout (gn_backward.cu) for an fp32 [B, HW, C] input with C in
-// {128, 256, 512, 1024}; grad_out is the gradient at the activation (the forward's 16-bit rounding is straight-through).
+// Backward of GroupNorm -> FiLM -> SiLU -> dropout (gn_backward.cu) for an fp32 [B, HW, C] input with C % 64 == 0,
+// C <= 2048; grad_out is the gradient at the activation (the forward's 16-bit rounding is straight-through).
 struct GroupNormBwdParams {
     const float* x; const float* grad_out;
     const float* gamma; const float* beta;
@@ -269,7 +269,7 @@ struct alignas(64) WgradParams {
     CUtensorMap x_map;                 // 4-D (Cin, W, H, N) 16-bit, same box
     int taps;                          // 9 or 1
     int Cout, Cin;
-    int co_blocks;                     // Cout / 128
+    int co_blocks;                     // ceil(Cout / 128); with Cout % 128 == 64 the last block holds 64 channels
     int ci_block, ci_blocks;           // input channels per accumulator (<= 256, multiple of 64), Cin / ci_block
     int tap_groups;                    // ceil(taps / 2): two taps' accumulators fill TMEM
     int splits;                        // K splits (pixel-tile ranges)

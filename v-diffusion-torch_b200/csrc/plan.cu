@@ -1817,7 +1817,7 @@ extern "C" int vdt_op_conv_dgrad(const void* dy, int32_t batch, int32_t h, int32
 extern "C" int vdt_op_conv_wgrad(const void* x, const void* dy, int32_t batch, int32_t h, int32_t w, int32_t cin, int32_t cout,
                                  int32_t ksize, float* dw_oihw, float* dbias, int32_t f16, void* stream) {
     if (ksize != 1 && ksize != 3) return fail("ksize must be 1 or 3");
-    if (cout % 128 || cin % 64) return fail("wgrad needs cout %% 128 == 0 and cin %% 64 == 0 (got %d -> %d)", cin, cout);
+    if (cout % 64 || cin % 64) return fail("wgrad needs cout %% 64 == 0 and cin %% 64 == 0 (got %d -> %d)", cin, cout);
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     ConvGeom g;
     CKI(conv_geom(batch, h, w, &g));
@@ -1826,7 +1826,7 @@ extern "C" int vdt_op_conv_wgrad(const void* x, const void* dy, int32_t batch, i
     memset(wp.get(), 0, sizeof(WgradParams));
     CKI(make_map_nhwc(&wp->dy_map, dy, batch, h, w, cout, g.box_h, g.box_n));
     CKI(make_map_nhwc(&wp->x_map, x, batch, h, w, cin, g.box_h, g.box_n));
-    wp->taps = ksize * ksize; wp->Cout = cout; wp->Cin = cin; wp->co_blocks = cout / 128;
+    wp->taps = ksize * ksize; wp->Cout = cout; wp->Cin = cin; wp->co_blocks = (cout + 127) / 128;
     wp->ci_block = cin <= 256 ? cin : (cin % 256 == 0 ? 256 : (cin % 192 == 0 ? 192 : (cin % 128 == 0 ? 128 : 64)));
     wp->ci_blocks = cin / wp->ci_block;
     wp->tap_groups = (wp->taps + 1) / 2;
@@ -1877,8 +1877,8 @@ extern "C" int vdt_op_groupnorm_backward(const float* x, const float* grad_out, 
                                          float* grad_film, void* stream) {
     if (!x || !grad_out || !gamma || !beta || !grad_x || !grad_gamma || !grad_beta) return fail("null argument");
     if (batch < 1 || h < 1 || w < 1) return fail("empty input");
-    if (c % 128 != 0 || c > 1024 || 256 % (c / 4) != 0)
-        return fail("groupnorm backward takes 128, 256, 512 or 1024 channels (got %d)", c);
+    if (c < 64 || c % 64 != 0 || c > 2048)
+        return fail("groupnorm backward takes a multiple of 64 channels up to 2048 (got %d)", c);
     if (!(drop_p >= 0.f && drop_p < 1.f)) return fail("drop_p must lie in [0, 1)");
     GroupNormBwdParams q{};
     q.x = x; q.grad_out = grad_out; q.gamma = gamma; q.beta = beta; q.film = film;

@@ -13,6 +13,10 @@
 // bounds zero fill = padding); the two taps' 128 x 256 fp32 accumulators fill TMEM's 512 columns.  Partial sums go to
 // partial[split][tap][co][ci]; a second kernel adds the splits in a fixed order (deterministic) and writes OIHW.
 //
+// Cout % 128 == 64 (192, 576, ...): the last output-channel block holds 64 channels.  Its CTAs never load the second
+// 64-channel dY chunk; that chunk's shared memory is zeroed once in both stages, so the M = 128 MMA multiplies zero rows
+// (half of that block's tensor work is spent on zeros) and the epilogue warps of the missing channels write nothing.
+//
 //   warp 0   TMA producer      warp 1   MMA issuer      warps 2-5   epilogue (TMEM -> partial sums)
 #include <atomic>
 
@@ -50,6 +54,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
     const int t_begin = static_cast<int>(static_cast<long long>(split) * p.num_tiles / p.splits);
     const int t_end = static_cast<int>(static_cast<long long>(split + 1) * p.num_tiles / p.splits);
     const int bn = p.ci_block, bchunks = bn / 64;
+    const int achunks = (co_blk * 128 + 128 <= p.Cout) ? 2 : 1;         // 1: tail block of 64 output channels
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < 2; ++s) { mbar_init(&a_full[s], 1); mbar_init(&a_empty[s], 1); mbar_init(&b_full[s], 1); mbar_init(&b_empty[s], 1); }
@@ -58,6 +63,13 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
         tma_prefetch_desc(&p.dy_map); tma_prefetch_desc(&p.x_map);
     }
     if (warp == 1) tmem_alloc(tmem_slot, 512);
+    if (achunks == 1) {                                       // zero rows for the missing 64 output channels, both stages
+        for (int i = threadIdx.x; i < kChunk / 16; i += blockDim.x) {
+            reinterpret_cast<uint4*>(a_smem + kChunk)[i] = make_uint4(0u, 0u, 0u, 0u);
+            reinterpret_cast<uint4*>(a_smem + kABytes + kChunk)[i] = make_uint4(0u, 0u, 0u, 0u);
+        }
+        fence_proxy_async_smem();                             // generic-proxy writes -> visible to UMMA after the barrier
+    }
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -71,8 +83,8 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
                 const int sa = ia & 1;
                 mbar_wait(&a_empty[sa], ((ia >> 1) & 1) ^ 1);
                 if (elect_one()) {
-                    mbar_expect_tx(&a_full[sa], static_cast<uint32_t>(2 * p.rows_per_tile * 128));
-                    for (int c = 0; c < 2; ++c)
+                    mbar_expect_tx(&a_full[sa], static_cast<uint32_t>(achunks * p.rows_per_tile * 128));
+                    for (int c = 0; c < achunks; ++c)
                         tma_load_4d(a_smem + sa * kABytes + c * kChunk, &p.dy_map, &a_full[sa], co_blk * 128 + c * 64, 0, y0, n0);
                 }
                 __syncwarp();
@@ -126,7 +138,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
         const int q = warp & 3;
         mbar_wait(acc_full, 0);
         tc_fence_after();
-        if (t_end > t_begin) {
+        if (t_end > t_begin && co_blk * 128 + q * 32 < p.Cout) {     // TMEM lanes of the tail block's missing channels: none
             const int co = co_blk * 128 + q * 32 + lane;
             for (int k = 0; k < ntaps; ++k) {
                 float* dst = p.partial + ((static_cast<size_t>(split) * p.taps + tap0 + k) * p.Cout + co) * p.Cin + ci_blk * bn;
