@@ -190,7 +190,8 @@ int vdt_op_conv(const void* x_16_nhwc, int32_t batch, int32_t h, int32_t w, int3
  *        dy 16-bit NHWC [B, H, W, cout], w fp32 OIHW [cout, cin, k, k].
  * wgrad: dW fp32 OIHW [cout, cin, k, k] = sum over pixels of dY[p][co] * X[p + tap][ci] (tcgen05, both operands MN-major,
  *        K split over CTAs with a fixed-order reduction); optional dbias fp32 [cout] = sum over pixels of dY.  x, dy 16-bit
- *        NHWC.  Needs cout % 64 == 0, cin % 64 == 0 and feature maps that tile into 128-pixel boxes. */
+ *        NHWC.  Needs cout % 64 == 0 and cin % 64 == 0; takes any feature map the forward conv takes (width <= 128), including
+ *        those whose tile holds fewer than 128 pixels (28x28, 14x14, 7x7, ...). */
 int vdt_op_conv_dgrad(const void* dy_16_nhwc, int32_t batch, int32_t h, int32_t w, int32_t cin, const float* w_oihw, int32_t cout,
                       int32_t ksize, float* dx_nhwc, int32_t f16, void* stream);
 int vdt_op_conv_wgrad(const void* x_16_nhwc, const void* dy_16_nhwc, int32_t batch, int32_t h, int32_t w, int32_t cin, int32_t cout,

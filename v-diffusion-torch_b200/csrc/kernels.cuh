@@ -273,7 +273,7 @@ struct alignas(64) WgradParams {
     int ci_block, ci_blocks;           // input channels per accumulator (<= 256, multiple of 64), Cin / ci_block
     int tap_groups;                    // ceil(taps / 2): two taps' accumulators fill TMEM
     int splits;                        // K splits (pixel-tile ranges)
-    int num_tiles, tiles_per_image, box_h, box_n, rows_per_tile;   // the forward conv's 128-pixel tiling (rows_per_tile == 128)
+    int num_tiles, tiles_per_image, box_h, box_n, rows_per_tile;   // the forward conv's 128-pixel tiling (rows_per_tile <= 128)
     int f16;
     float* partial;                    // fp32 [splits][taps][Cout][Cin]
 };

@@ -1821,7 +1821,6 @@ extern "C" int vdt_op_conv_wgrad(const void* x, const void* dy, int32_t batch, i
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     ConvGeom g;
     CKI(conv_geom(batch, h, w, &g));
-    if (g.rows_per_tile != 128) return fail("wgrad needs feature maps that tile into 128-pixel boxes (got %dx%d)", h, w);
     std::unique_ptr<WgradParams> wp(new WgradParams());
     memset(wp.get(), 0, sizeof(WgradParams));
     CKI(make_map_nhwc(&wp->dy_map, dy, batch, h, w, cout, g.box_h, g.box_n));

@@ -9,13 +9,20 @@
 // UMMA reads them through MN-major descriptors (tcgen05 transposes on the fly; nothing is transposed in memory).
 //
 // Work item = (block of 128 output channels, block of <= 256 input channels, group of <= 2 taps, K split): the CTA walks
-// its share of the 128-pixel tiles; per tile the dY tile is fetched once and one X tile per tap (shifted box, out-of-
+// its share of the (up to) 128-pixel tiles; per tile the dY tile is fetched once and one X tile per tap (shifted box, out-of-
 // bounds zero fill = padding); the two taps' 128 x 256 fp32 accumulators fill TMEM's 512 columns.  Partial sums go to
 // partial[split][tap][co][ci]; a second kernel adds the splits in a fixed order (deterministic) and writes OIHW.
 //
 // Cout % 128 == 64 (192, 576, ...): the last output-channel block holds 64 channels.  Its CTAs never load the second
 // 64-channel dY chunk; that chunk's shared memory is zeroed once in both stages, so the M = 128 MMA multiplies zero rows
 // (half of that block's tensor work is spent on zeros) and the epilogue warps of the missing channels write nothing.
+//
+// Ragged K tiles (28x28, 14x14, 7x7, 24x24, 5x5 ...: the forward conv's box holds rows_per_tile < 128 pixels): the pixels
+// are the contraction, so a stale row would be multiplied into every dW entry (in both operands: 0 * NaN is NaN).  Rows
+// rows_per_tile .. 127 of every dY and X chunk are zeroed once per CTA in both stages: TMA fills exactly rows_per_tile rows
+// and never touches them, and zeroing whole 128-byte rows commutes with the 128B swizzle, which permutes 16-byte pieces
+// within a row.  Each tap issues ceil(rows_per_tile / 16) MMAs instead of 8.  Boxes past the batch end are zero-filled by
+// TMA, as in the forward conv.
 //
 //   warp 0   TMA producer      warp 1   MMA issuer      warps 2-5   epilogue (TMEM -> partial sums)
 #include <atomic>
@@ -33,7 +40,8 @@ constexpr int kBBytesMax = 4 * kChunk;           // X tile: up to 256 input chan
 constexpr int kWgThreads = 32 * 6;
 constexpr int kWgSmem = 2 * kABytes + 2 * kBBytesMax + 1024 + 256;
 
-template <bool F16>
+// kRagged: rows_per_tile < kPix.  A separate instantiation, so full tiles keep their instruction stream unchanged
+template <bool F16, bool kRagged>
 __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_constant__ WgradParams p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -69,6 +77,16 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
             reinterpret_cast<uint4*>(a_smem + kABytes + kChunk)[i] = make_uint4(0u, 0u, 0u, 0u);
         }
         fence_proxy_async_smem();                             // generic-proxy writes -> visible to UMMA after the barrier
+    }
+    if (kRagged) {                                            // zero pixel rows rows_per_tile .. 127 of every loaded chunk
+        const int tail16 = (kPix - p.rows_per_tile) * 8;      // 16-byte pieces per chunk
+        const int per_stage = achunks + bchunks;              // dY chunks (a missing one is zeroed whole above) + X chunks
+        for (int i = threadIdx.x; i < 2 * per_stage * tail16; i += blockDim.x) {
+            const int c = i / tail16, s = c / per_stage, j = c % per_stage;
+            uint8_t* chunk = (j < achunks) ? a_smem + s * kABytes + j * kChunk : b_smem + s * kBBytesMax + (j - achunks) * kChunk;
+            reinterpret_cast<uint4*>(chunk + p.rows_per_tile * 128)[i % tail16] = make_uint4(0u, 0u, 0u, 0u);
+        }
+        fence_proxy_async_smem();
     }
     tc_fence_before();
     __syncthreads();
@@ -107,6 +125,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
             // D[co 128][ci bn] += A^T B with A = dY tile, B = X tile, both MN-major (bits 15 / 16 of the descriptor).  The whole
             // warp walks the loop; one elected lane issues each instruction (ptx.cuh: elect_one)
             const uint32_t idesc = umma_idesc_16(128, bn, (F16 ? 1 : 0)) | kIdescBMajorMN | (1u << 15);
+            const int kmma = kRagged ? (p.rows_per_tile + 15) / 16 : kPix / 16;
             int ia = 0, ib = 0;
             for (int t = t_begin; t < t_end; ++t, ++ia) {
                 const int sa = ia & 1;
@@ -120,7 +139,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_kernel(const __grid_const
                     const uint64_t bdesc = umma_desc_sw128_mn(smem_u32(b_smem + sb * kBBytesMax), kChunk);
                     if (elect_one()) {
 #pragma unroll
-                        for (int kk = 0; kk < kPix / 16; ++kk)   // 16 pixels per MMA: +2048 bytes (= 128 descriptor units) in both operands
+                        for (int kk = 0; kk < kmma; ++kk)        // 16 pixels per MMA: +2048 bytes (= 128 descriptor units) in both operands
                             umma_16(tmem_base + static_cast<uint32_t>(k * 256), adesc + static_cast<uint64_t>(kk * 128),
                                     bdesc + static_cast<uint64_t>(kk * 128), idesc, (t > t_begin || kk > 0) ? 1u : 0u);
                         umma_commit(&b_empty[sb]);
@@ -216,15 +235,19 @@ cudaError_t launch_wgrad(const WgradParams& p, float* dw, float* dbias, const h1
     if (e != cudaSuccess) return e;
     if (dev < 0 || dev >= kMaxDevices) return cudaErrorInvalidDevice;
     if (!attr_set[dev].load(std::memory_order_acquire)) {
-        e = cudaFuncSetAttribute(wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem);
+        e = cudaFuncSetAttribute(wgrad_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(wgrad_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(wgrad_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(wgrad_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem);
         if (e != cudaSuccess) return e;
         attr_set[dev].store(true, std::memory_order_release);
     }
     const int grid = p.co_blocks * p.ci_blocks * p.tap_groups * p.splits;
     if (grid <= 0 || p.num_tiles <= 0) return cudaErrorInvalidValue;
-    if (p.f16) wgrad_kernel<true><<<grid, kWgThreads, kWgSmem, stream>>>(p);
-    else wgrad_kernel<false><<<grid, kWgThreads, kWgSmem, stream>>>(p);
+    const bool ragged = p.rows_per_tile < kPix;
+    void (*kernel)(WgradParams) = p.f16 ? (ragged ? wgrad_kernel<true, true> : wgrad_kernel<true, false>)
+                                        : (ragged ? wgrad_kernel<false, true> : wgrad_kernel<false, false>);
+    kernel<<<grid, kWgThreads, kWgSmem, stream>>>(p);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const long long n = static_cast<long long>(p.taps) * p.Cout * p.Cin;
