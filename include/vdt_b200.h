@@ -49,6 +49,11 @@ typedef struct vdt_unet_config {
 enum { VDT_OUT_X0 = 0, VDT_OUT_EPS = 1, VDT_OUT_BOTH = 2, VDT_OUT_V = 3 };
 enum { VDT_VAR_FIXED_SMALL = 0, VDT_VAR_FIXED_LARGE = 1, VDT_VAR_FIXED_MEDIUM = 2 };
 enum { VDT_SCHED_COSINE = 0, VDT_SCHED_LINEAR = 1, VDT_SCHED_SIGMOID = 2, VDT_SCHED_LEGACY = 3 };
+/* Solver of the reverse loop.  FIRST_ORDER: the reference's DDIM / ancestral step.  DPMPP_2M: DPM-Solver++(2M) (Lu et al.,
+ * 2022) on the same time grid t = i/T, DDIM only (use_ddim = 1, x0eps_coef = 0): the first step is DDIM, every later step
+ * but the last adds c2k * (pred_x0 - pred_x0 of the previous step) to the DDIM mean (vdt_step_coefficients slot 15), and
+ * the last step returns the guided x0 like DDIM. */
+enum { VDT_SOLVER_FIRST_ORDER = 0, VDT_SOLVER_DPMPP_2M = 1 };
 typedef struct vdt_sampler_config {
     int32_t sample_timesteps;     /* T */
     int32_t model_out_type;       /* VDT_OUT_* */
@@ -58,7 +63,7 @@ typedef struct vdt_sampler_config {
     int32_t x0eps_coef;           /* GaussianDiffusion(x0eps_coef=): posterior mean as c1*eps + c2*x0 (diffusion.py:137-140, 335-343) */
     int32_t t_fp32;               /* 1: the step tensor is fp32 as in p_sample_progressive (diffusion.py:421): s, t are fp32
                                      quotients and the timestep embedding is evaluated in fp32; 0: fp64 as in p_sample (:399) */
-    int32_t reserved;             /* 0 */
+    int32_t solver;               /* VDT_SOLVER_*; 0 = the reference's first-order step */
     double intp_frac;
     double logsnr_min, logsnr_max;
     double w_guide;
@@ -110,7 +115,9 @@ int vdt_p_sample(vdt_plan* plan, const vdt_sampler_config* sc, const float* nois
 int vdt_p_sample_range(vdt_plan* plan, const vdt_sampler_config* sc, float* x, const void* label,
                        const float* step_noise, int32_t batch, int32_t first_step, int32_t num_steps,
                        float* pred_x0 /* optional [B, C, R, R]: guided x0 prediction of the last step run
-                                         (p_sample_step(return_pred=True); used by p_sample_progressive, 416-441) */,
+                                         (p_sample_step(return_pred=True); used by p_sample_progressive, 416-441).
+                                         solver = DPMPP_2M: in/out -- on entry the guided x0 of step first_step + 1,
+                                         read when first_step < T-1 (then it must be given) */,
                        void* stream);
 /* Same with HOST buffers (pinned or pageable); copies in/out inside the call and synchronises. */
 int vdt_p_sample_host(vdt_plan* plan, const vdt_sampler_config* sc, const float* noise, const void* label,
@@ -136,7 +143,10 @@ int vdt_images_to_uint8(const float* x_nchw, uint8_t* out_nhwc, int32_t batch, i
 
 /* logsnr schedule + posterior coefficients — diffusion.py:42-112, 126-203 (host, fp64 with the reference's
  * fp32 rounding points).  out: [T][16] floats: alpha_t, sigma_t, rsqrt(sigmoid l_t), exp(-l_t/2), sigmoid(l_t),
- * sigmoid(-l_t), c1, c2, std, logvar, logsnr_s, logsnr_t, rsqrt(sigmoid -l_t), exp(l_t/2), x0eps_coef (0/1), 0.
+ * sigmoid(-l_t), c1, c2, std, logvar, logsnr_s, logsnr_t, rsqrt(sigmoid -l_t), exp(l_t/2), x0eps_coef (0/1), c2k.
+ * c2k (slot 15) is 0 unless solver = DPMPP_2M; there, for 0 < i < T-1, c2k = c2 * h_i / (2 h_{i+1}) with h_i = (l_s - l_t)/2
+ * of step i (fp64 from the fp32-rounded log-SNRs, rounded once), and 0 in rows 0 and T-1.  The solver is refused for
+ * use_ddim = 0 and for x0eps_coef = 1.
  * With x0eps_coef and DDIM, c1/c2 are the LOGARITHMS 0.5*logsigmoid(-+l_s): the reference only exponentiates
  * them for eta != 0 (diffusion.py:180-182 vs 199) and p_sample always runs eta = 0; reproduced as is. */
 int vdt_step_coefficients(const vdt_sampler_config* sc, float* out);
@@ -248,6 +258,12 @@ int vdt_op_attention_backward(const float* qkv, const float* grad_out, float* gr
 int vdt_op_sampler_step(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
                         int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step, const float* coef_host,
                         float w, void* stream);
+/* The same update with a history buffer, for DPM-Solver++(2M) rows: pred_hist fp32 [B, C, H, W] holds the guided x0 of
+ * the previous step on entry when coef[15] != 0 (it is not read otherwise) and this step's guided x0 on return.
+ * vdt_op_sampler_step refuses a row with coef[15] != 0. */
+int vdt_op_sampler_step_hist(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
+                             int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step, const float* coef_host,
+                             float w, float* pred_hist, void* stream);
 
 #ifdef __cplusplus
 }

@@ -22,6 +22,7 @@ SCHEDULES = {"cosine": 0, "linear": 1, "sigmoid": 2, "legacy": 3}
 COEF_STRIDE = 16
 OPERAND_DTYPES = {"fp16": 0, "bf16": 1, "fp16x3": 2}
 REWEIGHT_TYPES = {"constant": 0, "snr": 1, "snr_trunc": 2, "snr_1plus": 3}
+SOLVERS = {None: 0, "dpmpp_2m": 1}                # include/vdt_b200.h VDT_SOLVER_*
 
 
 class UNetConfig(C.Structure):
@@ -36,7 +37,7 @@ class UNetConfig(C.Structure):
 class SamplerConfig(C.Structure):
     _fields_ = [("sample_timesteps", C.c_int32), ("model_out_type", C.c_int32), ("model_var_type", C.c_int32),
                 ("logsnr_schedule", C.c_int32), ("use_ddim", C.c_int32), ("x0eps_coef", C.c_int32),
-                ("t_fp32", C.c_int32), ("reserved", C.c_int32), ("intp_frac", C.c_double), ("logsnr_min", C.c_double), ("logsnr_max", C.c_double),
+                ("t_fp32", C.c_int32), ("solver", C.c_int32), ("intp_frac", C.c_double), ("logsnr_min", C.c_double), ("logsnr_max", C.c_double),
                 ("w_guide", C.c_double), ("seed", C.c_uint64)]
 
 
@@ -110,6 +111,7 @@ def lib():
     L.vdt_op_groupnorm.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, i32, vp, vp, i32, i32, vp]
     L.vdt_op_attention.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp]
     L.vdt_op_sampler_step.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, C.c_float, vp]
+    L.vdt_op_sampler_step_hist.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, C.c_float, vp, vp]
     L.vdt_stat_slabs_per_image.argtypes = [i32, i32]
     L.vdt_unet_forward_train.argtypes = [vp, vp, vp, vp, vp, i32, C.c_float, C.c_uint64, vp]
     L.vdt_op_groupnorm_dropout.argtypes = [vp, i32, i32, i32, i32, vp, vp, i32, vp, i32, C.c_float, C.c_uint64, i32, vp]
@@ -139,7 +141,8 @@ EXPORTS = ["vdt_last_error", "vdt_version", "vdt_kernel_launches", "vdt_plan_cre
            "vdt_plan_num_weights", "vdt_plan_weight_name", "vdt_plan_weight_shape", "vdt_plan_load_weight",
            "vdt_plan_finalize", "vdt_unet_forward", "vdt_p_sample", "vdt_p_sample_range", "vdt_p_sample_host",
            "vdt_step_coefficients", "vdt_plan_flops", "vdt_profile_enable", "vdt_profile_read",
-           "vdt_op_conv", "vdt_op_groupnorm", "vdt_op_attention", "vdt_op_sampler_step", "vdt_stat_slabs_per_image",
+           "vdt_op_conv", "vdt_op_groupnorm", "vdt_op_attention", "vdt_op_sampler_step", "vdt_op_sampler_step_hist",
+           "vdt_stat_slabs_per_image",
            "vdt_plan_saturations", "vdt_images_to_uint8",
            "vdt_train_coefficients", "vdt_q_sample", "vdt_train_loss", "vdt_unet_forward_train", "vdt_op_groupnorm_dropout",
            "vdt_op_conv_dgrad", "vdt_op_conv_wgrad", "vdt_op_groupnorm_backward",

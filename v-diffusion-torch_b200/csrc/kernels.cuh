@@ -235,7 +235,9 @@ struct SamplerStepParams {
     const float* x_t;                  // fp32 NCHW [B, C, HW]
     float* x_s;                        // fp32 NCHW [B, C, HW]  (may alias x_t)
     float* pred_x0;                    // optional fp32 NCHW [B, C, HW]: the (guided) x0 prediction of this step
-                                       // (p_sample_step(return_pred=True), diffusion.py:385, 392)
+                                       // (p_sample_step(return_pred=True), diffusion.py:385, 392).  Required when the
+                                       // coefficient row's c2k (slot 15, DPM-Solver++(2M)) is non-zero: it then holds the
+                                       // previous step's prediction on entry
     const SamplerState* st;            // step index, coefficient row, injected noise / seed of this call
     int B, C, HW;
     int cfg;                           // 1: classifier-free guidance pair per sample

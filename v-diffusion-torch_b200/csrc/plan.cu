@@ -1405,11 +1405,24 @@ static int logsnr_d(const vdt_sampler_config& sc, double t, double* out) {
     return fail("unknown logsnr schedule %d", sc.logsnr_schedule);   // NotImplementedError, diffusion.py:96
 }
 
+// DPM-Solver++(2M) is defined here on the data prediction of the DDIM (eta = 0) step only.
+static int check_solver(const vdt_sampler_config& sc) {
+    if (sc.solver == VDT_SOLVER_FIRST_ORDER) return 0;
+    if (sc.solver != VDT_SOLVER_DPMPP_2M) return fail("unknown solver %d", sc.solver);
+    if (!sc.use_ddim) return fail("the DPM-Solver++(2M) solver needs use_ddim = 1 (it is not defined for ancestral sampling)");
+    if (sc.x0eps_coef)
+        return fail("the DPM-Solver++(2M) solver needs x0eps_coef = 0 (under DDIM the reference's (eps, x0) coefficients are "
+                    "logarithms, so there is no data-prediction step to extend)");
+    return 0;
+}
+
 extern "C" int vdt_step_coefficients(const vdt_sampler_config* scp, float* out) {
     if (!scp || !out) return fail("null argument");
     const vdt_sampler_config& sc = *scp;
     const int T = sc.sample_timesteps;
     if (T < 1) return fail("sample_timesteps must be >= 1");
+    CKI(check_solver(sc));
+    std::vector<double> h(T), c2d(T);                           // lambda_s - lambda_t and the fp64 c2 of every step
     for (int i = 0; i < T; ++i) {
         double ls_d, lt_d;
         // s = step / T, t = (step + 1) / T: fp64 tensors in p_sample (diffusion.py:399), fp32 in p_sample_progressive
@@ -1466,7 +1479,14 @@ extern "C" int vdt_step_coefficients(const vdt_sampler_config* scp, float* out) 
         o[13] = std::exp(0.5f * lt32);
         o[14] = sc.x0eps_coef ? 1.0f : 0.0f;         // lets vdt_op_sampler_step pick the (eps, x0) form from the row alone
         o[15] = 0.0f;
+        h[i] = 0.5 * (ls - lt);
+        c2d[i] = c2;
     }
+    // DPM-Solver++(2M): with lambda = l / 2 and h_i = lambda_s - lambda_t of step i, D = pred + k (pred - pred_prev) with
+    // k = h_i / (2 h_{i+1}) (step i + 1 runs just before step i), written as the DDIM mean plus c2k (pred - pred_prev).
+    // The first step (i = T-1) is DDIM; the last (i = 0) returns the guided x0 like DDIM.
+    if (sc.solver == VDT_SOLVER_DPMPP_2M)
+        for (int i = 1; i < T - 1; ++i) out[(size_t)i * kCoefStride + 15] = (float)(c2d[i] * (h[i] / (2.0 * h[i + 1])));
     return 0;
 }
 
@@ -1548,10 +1568,10 @@ static int get_sampler_exec(vdt_plan* p, const vdt_sampler_config& sc, int imgs,
     // the key holds what shapes the workspace, the coefficient table and the kernel parameters baked into the graph;
     // per-call values (seed, injected-noise tensor, fp32-t mode of p_sample_progressive) live in the device-side
     // SamplerState and are rewritten before every call
-    char key[192];
-    snprintf(key, sizeof(key), "smp%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%.17g:%.17g:%.17g:%.17g", lane, imgs, (int)has_label,
+    char key[208];
+    snprintf(key, sizeof(key), "smp%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%.17g:%.17g:%.17g:%.17g", lane, imgs, (int)has_label,
              sc.sample_timesteps, sc.model_out_type, sc.model_var_type, sc.logsnr_schedule, sc.use_ddim, sc.x0eps_coef, sc.t_fp32,
-             sc.intp_frac, sc.logsnr_min, sc.logsnr_max, sc.w_guide);
+             sc.solver, sc.intp_frac, sc.logsnr_min, sc.logsnr_max, sc.w_guide);
     CKI(exec_cache_lookup(p, key, out));
     if (*out) return 0;
     CKI(exec_cache_make_room(p));
@@ -1604,10 +1624,17 @@ extern "C" int vdt_p_sample_range(vdt_plan* p, const vdt_sampler_config* scp, fl
                                   const float* step_noise, int32_t batch, int32_t first_step, int32_t num_steps,
                                   float* pred_x0, void* stream) {
     if (!p || !scp || !x) return fail("null argument");
-    if (!p->finalized) return fail("plan not finalized (load every state_dict key, then vdt_plan_finalize)");
     const vdt_sampler_config& sc = *scp;
-    if (sc.model_out_type < 0 || sc.model_out_type > 3) return fail("unknown model_out_type %d", sc.model_out_type);
     const int T = sc.sample_timesteps;
+    CKI(check_solver(sc));
+    // DPM-Solver++(2M) steps after the first read the previous step's guided x0: a range that starts inside the trajectory
+    // takes it from pred_x0 (written by the call that ran step first_step + 1), since the exec's pred buffer is shared by
+    // every chunk of its lane
+    const bool carry_pred = sc.solver == VDT_SOLVER_DPMPP_2M && first_step < T - 1 && num_steps > 0;
+    if (carry_pred && !pred_x0)
+        return fail("DPM-Solver++(2M) from step %d < T-1 needs pred_x0 holding the guided x0 of step %d", first_step, first_step + 1);
+    if (!p->finalized) return fail("plan not finalized (load every state_dict key, then vdt_plan_finalize)");
+    if (sc.model_out_type < 0 || sc.model_out_type > 3) return fail("unknown model_out_type %d", sc.model_out_type);
     if (first_step < 0 || first_step >= T || num_steps < 0 || first_step - num_steps < -1)
         return fail("step range [%d, %d) steps leaves the trajectory of %d steps", first_step, num_steps, T);
     cudaStream_t user = reinterpret_cast<cudaStream_t>(stream);
@@ -1641,6 +1668,7 @@ extern "C" int vdt_p_sample_range(vdt_plan* p, const vdt_sampler_config* scp, fl
         Exec* ex;
         CKI(get_sampler_exec(p, sc, imgs, label != nullptr, lane, &ex));
         CK(cudaMemcpyAsync(ex->xin, x + (size_t)i0 * CHW, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
+        if (carry_pred) CK(cudaMemcpyAsync(ex->pred, pred_x0 + (size_t)i0 * CHW, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
         if (mt) {
             const int n = ex->rows * c.num_classes;
             multitag_rows_kernel<<<(n + 127) / 128, 128, 0, st>>>(static_cast<const float*>(label) + (size_t)i0 * c.num_classes,
@@ -1939,9 +1967,13 @@ extern "C" int vdt_images_to_uint8(const float* x, uint8_t* out, int32_t batch, 
     return 0;
 }
 
-extern "C" int vdt_op_sampler_step(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
-                                   int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step,
-                                   const float* coef_host, float w, void* stream) {
+static int op_sampler_step_impl(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
+                                int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step,
+                                const float* coef_host, float w, float* pred_hist, void* stream) {
+    if (!coef_host) return fail("null argument");
+    if (coef_host[15] != 0.0f && !pred_hist)
+        return fail("coefficient row %d is a DPM-Solver++(2M) row (c2k != 0): use vdt_op_sampler_step_hist with the previous "
+                    "step's guided x0", step);
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     SamplerState hs{};
     hs.next_step = step - 1; hs.step = step; hs.img0 = 0; hs.noise = noise; hs.noise_step_stride = 0; hs.seed = 0;
@@ -1951,7 +1983,7 @@ extern "C" int vdt_op_sampler_step(const float* model_out, const float* x_t, con
     CK(cudaMemcpy(ds, &hs, sizeof(hs), cudaMemcpyHostToDevice));
     SamplerStepParams sp{};
     sp.model_out = model_out; sp.x_t = x_t; sp.x_s = x_s;
-    sp.st = ds; sp.pred_x0 = nullptr; sp.B = batch; sp.C = c; sp.HW = hw; sp.cfg = cfg;
+    sp.st = ds; sp.pred_x0 = pred_hist; sp.B = batch; sp.C = c; sp.HW = hw; sp.cfg = cfg;
     sp.model_out_type = model_out_type; sp.w = w; sp.x0eps = coef_host[14] != 0.0f ? 1 : 0;
     cudaError_t e = launch_sampler_step(sp, st);
     ++g_launches;
@@ -1960,6 +1992,19 @@ extern "C" int vdt_op_sampler_step(const float* model_out, const float* x_t, con
     if (e != cudaSuccess) return fail("sampler_step launch failed: %s", cudaGetErrorString(e));
     if (e2 != cudaSuccess) return fail("sampler_step failed: %s", cudaGetErrorString(e2));
     return 0;
+}
+
+extern "C" int vdt_op_sampler_step(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
+                                   int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step,
+                                   const float* coef_host, float w, void* stream) {
+    return op_sampler_step_impl(model_out, x_t, noise, x_s, batch, c, hw, cfg, model_out_type, step, coef_host, w, nullptr, stream);
+}
+
+extern "C" int vdt_op_sampler_step_hist(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
+                                        int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step,
+                                        const float* coef_host, float w, float* pred_hist, void* stream) {
+    if (!pred_hist) return fail("null pred_hist");
+    return op_sampler_step_impl(model_out, x_t, noise, x_s, batch, c, hw, cfg, model_out_type, step, coef_host, w, pred_hist, stream);
 }
 
 // ---- entry points the composed training step (v-diffusion-torch_b200/training.py) adds to the kernel-level hooks ----------

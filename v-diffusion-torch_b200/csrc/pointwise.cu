@@ -315,6 +315,17 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const SamplerStepPara
         if (noisy) mean += sd * z[k];
         out[k] = mean; pr[k] = pred;
     }
+    // DPM-Solver++(2M): x_s = DDIM mean + c2k (pred - pred of the previous step), i.e. c1 x_t + c2 D with
+    // D = pred + k (pred - pred_prev).  The previous pred is read only for a non-zero c2k: the buffer may hold stale values
+    // from another chunk or call (0 * NaN is NaN), and DDIM / ancestral rows (c2k = 0) keep exactly their instructions.
+    // This thread owns these elements, so the read precedes the store below without a race.
+    const float c2k = cf[15];
+    if (c2k != 0.f) {
+        float pp[VEC];
+        ldv(p.pred_x0 + i, pp);
+#pragma unroll
+        for (int k = 0; k < VEC; ++k) out[k] = fmaf(c2k, pr[k] - pp[k], out[k]);
+    }
     if (p.pred_x0) stv(p.pred_x0 + i, pr);
     stv(p.x_s + i, out);
 }

@@ -63,7 +63,19 @@ class GaussianDiffusion:
         self.intp_frac, self.w_guide, self.p_uncond, self.x0eps_coef = intp_frac, w_guide, p_uncond, x0eps_coef
 
     # ------------------------------------------------------------------ C structs
-    def sampler_config(self, use_ddim, seed=None, t_fp32=False):
+    def _check_solver(self, solver, use_ddim):
+        """``solver`` (extension): None, the reference's first-order step, or "dpmpp_2m", DPM-Solver++(2M) (Lu et al., 2022)
+        on the same time grid -- defined for DDIM (use_ddim=True) with x0eps_coef=False only."""
+        if solver not in _lib.SOLVERS:
+            raise NotImplementedError(f"unknown solver {solver!r} (choices: None, 'dpmpp_2m')")
+        if solver is not None and not use_ddim:
+            raise NotImplementedError(f"solver={solver!r} needs use_ddim=True (it is not defined for ancestral sampling)")
+        if solver is not None and self.x0eps_coef:
+            raise NotImplementedError(f"solver={solver!r} needs x0eps_coef=False (under DDIM the reference's (eps, x0) "
+                                      "coefficients are logarithms, diffusion.py:180-182)")
+
+    def sampler_config(self, use_ddim, seed=None, t_fp32=False, solver=None):
+        self._check_solver(solver, use_ddim)
         if not use_ddim and self.model_var_type not in _lib.VAR_TYPES:
             raise NotImplementedError(self.model_var_type)          # diffusion.py:161
         if not use_ddim and self.model_var_type == "fixed_medium" and not isinstance(self.intp_frac, float):
@@ -76,6 +88,7 @@ class GaussianDiffusion:
         sc.use_ddim = int(bool(use_ddim))
         sc.x0eps_coef = int(bool(self.x0eps_coef))                  # diffusion.py:137-140, 180-182, 335-343
         sc.t_fp32 = int(bool(t_fp32))                               # diffusion.py:421 vs :399
+        sc.solver = _lib.SOLVERS[solver]
         sc.intp_frac = float(self.intp_frac or 0.)
         sc.logsnr_min, sc.logsnr_max = self.logsnr_fn.logsnr_min, self.logsnr_fn.logsnr_max
         sc.w_guide = float(self.w_guide)
@@ -114,9 +127,9 @@ class GaussianDiffusion:
                     raise RuntimeError(f"class ids must lie in [0, {num_classes}] (0 = unconditional), got [{lo}, {hi}]")
         return label
 
-    def step_coefficients(self, use_ddim):
-        """[T, 16] fp32 host table (include/vdt_b200.h: vdt_step_coefficients)."""
-        sc = self.sampler_config(use_ddim)
+    def step_coefficients(self, use_ddim, solver=None):
+        """[T, 16] fp32 host table (include/vdt_b200.h: vdt_step_coefficients); slot 15 holds DPM-Solver++(2M)'s c2k."""
+        sc = self.sampler_config(use_ddim, solver=solver)
         out = torch.empty((self.sample_timesteps, _lib.COEF_STRIDE), dtype=torch.float32)
         _lib.check(_lib.lib().vdt_step_coefficients(C.byref(sc), _lib.ptr(out)))
         return out
@@ -124,9 +137,11 @@ class GaussianDiffusion:
     # ------------------------------------------------------------------ p_sample (diffusion.py:394-414)
     @torch.no_grad()
     def p_sample(self, denoise_fn, shape, noise=None, label=None, device="cpu", seed=None, use_ddim=False,
-                 step_noise=None):
+                 step_noise=None, solver=None):
         """``step_noise`` (extension): optional (T, B, C, H, W) tensor of the per-step normal draws the
-        reference takes from its generator (diffusion.py:389), so both sides inject identical noise."""
+        reference takes from its generator (diffusion.py:389), so both sides inject identical noise.
+        ``solver`` (extension): None (the reference's step) or "dpmpp_2m" (DPM-Solver++(2M), with use_ddim=True)."""
+        self._check_solver(solver, use_ddim)
         device = torch.device(device)
         if device.type != "cuda":
             raise RuntimeError("v_diffusion_b200 samples on CUDA (sm_100a) only; there is no CPU fallback")
@@ -151,7 +166,8 @@ class GaussianDiffusion:
         L = _lib.lib()
         if isinstance(denoise_fn, UNet):
             # fused path: the per-step normals come from the library's own Philox stream keyed by this call's seed
-            sc = self.sampler_config(use_ddim, self._noise_seed(seed) if (not use_ddim and step_noise is None) else seed)
+            sc = self.sampler_config(use_ddim, self._noise_seed(seed) if (not use_ddim and step_noise is None) else seed,
+                                     solver=solver)
             plan = denoise_fn.plan_for(shape[2], device)
             out = torch.empty_like(x_t)
             with torch.cuda.device(device):
@@ -160,14 +176,17 @@ class GaussianDiffusion:
             return out.cpu()
         # generic callable: same fused update kernel, one step at a time; the per-step normals continue the generator
         # that produced x_T, like the reference's single generator (diffusion.py:401-405, 389)
-        sc = self.sampler_config(use_ddim, seed)
-        return self._p_sample_generic(denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim).cpu()
+        sc = self.sampler_config(use_ddim, seed, solver=solver)
+        return self._p_sample_generic(denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver).cpu()
 
     @torch.no_grad()
     def p_sample_progressive(self, denoise_fn, shape, noise=None, label=None, device="cpu", seed=None, use_ddim=False,
-                             pred_freq=50, step_noise=None):
+                             pred_freq=50, step_noise=None, solver=None):
         """diffusion.py:416-441: returns (x_0, preds) where preds[k] is the (guided) x0 prediction made at the
-        steps ti with (ti + 1) % pred_freq == 0, ordered like the reference (index L-1 = earliest).  Fused path only."""
+        steps ti with (ti + 1) % pred_freq == 0, ordered like the reference (index L-1 = earliest).  Fused path only.
+        ``solver`` as in p_sample; under "dpmpp_2m" the ``pred`` buffer every range call shares carries the previous
+        step's guided x0 into the next call."""
+        self._check_solver(solver, use_ddim)
         if not isinstance(denoise_fn, UNet):
             raise TypeError("p_sample_progressive needs the v_diffusion_b200 UNet")
         device = torch.device(device)
@@ -182,7 +201,8 @@ class GaussianDiffusion:
         if step_noise is not None:
             step_noise = step_noise.to(device=device, dtype=torch.float32).contiguous()
         # the reference's progressive loop carries an fp32 step tensor (diffusion.py:421): fp32 s / t and an fp32 sinusoid
-        sc = self.sampler_config(use_ddim, self._noise_seed(seed) if (not use_ddim and step_noise is None) else seed, t_fp32=True)
+        sc = self.sampler_config(use_ddim, self._noise_seed(seed) if (not use_ddim and step_noise is None) else seed, t_fp32=True,
+                                 solver=solver)
         plan = denoise_fn.plan_for(shape[2], device)
         Lp = T // pred_freq
         preds = torch.zeros((Lp, B) + tuple(shape[1:]), dtype=torch.float32)
@@ -254,10 +274,12 @@ class GaussianDiffusion:
                                         _lib.REWEIGHT_TYPES[self.reweight_type], _lib.current_stream_ptr()))
         return (loss, grad) if return_grad else loss
 
-    def _p_sample_generic(self, denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim):
+    def _p_sample_generic(self, denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver=None):
         L = _lib.lib()
         B = shape[0]
-        coefs = self.step_coefficients(use_ddim)
+        coefs = self.step_coefficients(use_ddim, solver)
+        # DPM-Solver++(2M): the guided x0 of the previous step, read by every step whose c2k is non-zero
+        hist = torch.empty_like(x_t) if solver is not None else None
         use_cfg = (self.w_guide > 0) and (label is not None)        # diffusion.py:368
         T = self.sample_timesteps
         hw = shape[2] * shape[3]
@@ -276,9 +298,15 @@ class GaussianDiffusion:
                     z = step_noise[ti] if step_noise is not None else torch.randn(shape, device=device, generator=gen)
                     z = z.contiguous()
                 x_s = torch.empty_like(x_t)
-                _lib.check(L.vdt_op_sampler_step(_lib.ptr(model_out), _lib.ptr(x_t), _lib.ptr(z), _lib.ptr(x_s), B,
-                                                 shape[1], hw, int(use_cfg), sc.model_out_type, ti,
-                                                 _lib.ptr(coefs[ti].contiguous()), float(self.w_guide),
-                                                 _lib.current_stream_ptr()))
+                if hist is None:
+                    _lib.check(L.vdt_op_sampler_step(_lib.ptr(model_out), _lib.ptr(x_t), _lib.ptr(z), _lib.ptr(x_s), B,
+                                                     shape[1], hw, int(use_cfg), sc.model_out_type, ti,
+                                                     _lib.ptr(coefs[ti].contiguous()), float(self.w_guide),
+                                                     _lib.current_stream_ptr()))
+                else:
+                    _lib.check(L.vdt_op_sampler_step_hist(_lib.ptr(model_out), _lib.ptr(x_t), _lib.ptr(z), _lib.ptr(x_s), B,
+                                                          shape[1], hw, int(use_cfg), sc.model_out_type, ti,
+                                                          _lib.ptr(coefs[ti].contiguous()), float(self.w_guide), _lib.ptr(hist),
+                                                          _lib.current_stream_ptr()))
                 x_t = x_s
         return x_t

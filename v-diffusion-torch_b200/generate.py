@@ -145,6 +145,9 @@ def main():
     ap.add_argument("--ckpt-path", default=None, help="reference checkpoint (.pt); random init when omitted")
     ap.add_argument("--use-ema", action="store_true")
     ap.add_argument("--use-ddim", action="store_true")
+    ap.add_argument("--solver", choices=["ddim", "dpmpp_2m"], default="ddim",
+                    help="ddim: the reference's first-order step; dpmpp_2m: DPM-Solver++(2M) on the same time grid "
+                         "(needs --use-ddim; fewer --sample-timesteps for a comparable trajectory)")
     ap.add_argument("--sample-timesteps", type=int, default=1024)      # generate.py:25
     ap.add_argument("--uncond", action="store_true")
     ap.add_argument("--w-guide", type=float, default=0.1)              # generate.py:27
@@ -158,6 +161,9 @@ def main():
     ap.add_argument("--warmup-batches", type=int, default=0, help="untimed batches before the reported wall-clock")
     ap.add_argument("--label-path", default=None, help="multitag models: torch-saved (N, num_classes) attribute table")
     args = ap.parse_args()
+    if args.solver == "dpmpp_2m" and not args.use_ddim:
+        ap.error("--solver dpmpp_2m needs --use-ddim (DPM-Solver++(2M) is not defined for ancestral sampling)")
+    solver = None if args.solver == "ddim" else args.solver
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -207,7 +213,7 @@ def main():
         # would replay the same per-step normals for every batch (ancestral sampling, no injected noise)
         seed = int(torch.randint(0, 2 ** 62, (1,), device=device, generator=gen).item())
         return diffusion.p_sample(model, (n,) + chw, noise=noise, label=label, device=device, seed=seed,
-                                  use_ddim=args.use_ddim).to(device)
+                                  use_ddim=args.use_ddim, solver=solver).to(device)
 
     run = sample_balanced if args.schedule == "dynamic" else sample_sharded
     calls = [0]
