@@ -119,6 +119,28 @@ int vdt_p_sample_range(vdt_plan* plan, const vdt_sampler_config* sc, float* x, c
                                          solver = DPMPP_2M: in/out -- on entry the guided x0 of step first_step + 1,
                                          read when first_step < T-1 (then it must be given) */,
                        void* stream);
+/* Inpainting by replacement (Song et al., 2021, "Score-based generative modeling through SDEs", App. I; RePaint without
+ * resampling).  known fp32 [B, C, R, R]: the image in model space ([-1, 1]); mask fp32 [B, C, R, R] in [0, 1], 1 = known
+ * (the Python layer expands a [B, 1, R, R] mask over channels); known_noise NULL or fp32 [T, B, C, R, R], indexed by step
+ * like step_noise.  known and mask come together; known_noise needs both.  Device pointers, any 4-byte alignment.
+ * After step i has produced x_s (and stored the guided x0 in pred_x0, which is never replaced):
+ *   i > 0:  x_s = m * k_s + (1 - m) * x_s,  k_s = alpha_s * known + sigma_s * z', with alpha_s, sigma_s = slots 0, 1 of
+ *           coefficient row i - 1 (whose t is this step's s) and z' = known_noise[i], or else a standard normal from this
+ *           library's Philox4x32-10 stream keyed by sc->seed with counter word 3 = 1 (the ancestral draws use 0);
+ *   i = 0:  x_0 = m * known + (1 - m) * x_0.
+ * m = 0 leaves x_s unchanged and m = 1 gives k_s exactly.  x_T is the caller's noise.  Every solver and output type is
+ * allowed.  Under DDIM without known_noise the caller picks the seed of the z' stream. */
+typedef struct vdt_inpaint {
+    const float* known;
+    const float* mask;
+    const float* known_noise;
+} vdt_inpaint;
+/* vdt_p_sample / vdt_p_sample_range with inpainting; inpaint = NULL (or all three NULL) is the plain call. */
+int vdt_p_sample_inpaint(vdt_plan* plan, const vdt_sampler_config* sc, const vdt_inpaint* inpaint, const float* noise,
+                         const void* label, const float* step_noise, float* out, int32_t batch, void* stream);
+int vdt_p_sample_range_inpaint(vdt_plan* plan, const vdt_sampler_config* sc, const vdt_inpaint* inpaint, float* x,
+                               const void* label, const float* step_noise, int32_t batch, int32_t first_step,
+                               int32_t num_steps, float* pred_x0, void* stream);
 /* Same with HOST buffers (pinned or pageable); copies in/out inside the call and synchronises. */
 int vdt_p_sample_host(vdt_plan* plan, const vdt_sampler_config* sc, const float* noise, const void* label,
                       const float* step_noise, float* out, int32_t batch);
@@ -264,6 +286,13 @@ int vdt_op_sampler_step(const float* model_out, const float* x_t, const float* n
 int vdt_op_sampler_step_hist(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
                              int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step, const float* coef_host,
                              float w, float* pred_hist, void* stream);
+/* The same update followed by the inpainting replacement of vdt_inpaint: known, mask fp32 [B, C, H, W]; known_noise this
+ * step's z' [B, C, H, W] or NULL (then the Philox stream 1 keyed by seed); coef_prev_host = coefficient row step - 1 (host;
+ * NULL at step 0).  pred_hist may be NULL for a first-order row.  known = mask = NULL is the plain step. */
+int vdt_op_sampler_step_known(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
+                              int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step, const float* coef_host,
+                              float w, float* pred_hist, const float* known, const float* mask, const float* known_noise,
+                              uint64_t seed, const float* coef_prev_host, void* stream);
 
 #ifdef __cplusplus
 }

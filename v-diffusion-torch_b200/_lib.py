@@ -41,6 +41,10 @@ class SamplerConfig(C.Structure):
                 ("w_guide", C.c_double), ("seed", C.c_uint64)]
 
 
+class Inpaint(C.Structure):                               # include/vdt_b200.h vdt_inpaint
+    _fields_ = [("known", C.c_void_p), ("mask", C.c_void_p), ("known_noise", C.c_void_p)]
+
+
 def nvcc_path():
     for cand in (os.environ.get("NVCC"), shutil.which("nvcc"), "/usr/local/cuda/bin/nvcc"):
         if cand and os.path.exists(cand):
@@ -102,6 +106,8 @@ def lib():
     L.vdt_unet_forward.argtypes = [vp, vp, vp, vp, vp, i32, vp]
     L.vdt_p_sample.argtypes = [vp, C.POINTER(SamplerConfig), vp, vp, vp, vp, i32, vp]
     L.vdt_p_sample_range.argtypes = [vp, C.POINTER(SamplerConfig), vp, vp, vp, i32, i32, i32, vp, vp]
+    L.vdt_p_sample_inpaint.argtypes = [vp, C.POINTER(SamplerConfig), C.POINTER(Inpaint), vp, vp, vp, vp, i32, vp]
+    L.vdt_p_sample_range_inpaint.argtypes = [vp, C.POINTER(SamplerConfig), C.POINTER(Inpaint), vp, vp, vp, i32, i32, i32, vp, vp]
     L.vdt_plan_flops.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double)]
     L.vdt_profile_enable.argtypes = [C.c_int]
     L.vdt_profile_read.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_uint64)]
@@ -112,6 +118,8 @@ def lib():
     L.vdt_op_attention.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp]
     L.vdt_op_sampler_step.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, C.c_float, vp]
     L.vdt_op_sampler_step_hist.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, C.c_float, vp, vp]
+    L.vdt_op_sampler_step_known.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, C.c_float, vp, vp, vp, vp,
+                                            C.c_uint64, vp, vp]
     L.vdt_stat_slabs_per_image.argtypes = [i32, i32]
     L.vdt_unet_forward_train.argtypes = [vp, vp, vp, vp, vp, i32, C.c_float, C.c_uint64, vp]
     L.vdt_op_groupnorm_dropout.argtypes = [vp, i32, i32, i32, i32, vp, vp, i32, vp, i32, C.c_float, C.c_uint64, i32, vp]
@@ -140,9 +148,10 @@ def lib():
 EXPORTS = ["vdt_last_error", "vdt_version", "vdt_kernel_launches", "vdt_plan_create", "vdt_plan_destroy",
            "vdt_plan_num_weights", "vdt_plan_weight_name", "vdt_plan_weight_shape", "vdt_plan_load_weight",
            "vdt_plan_finalize", "vdt_unet_forward", "vdt_p_sample", "vdt_p_sample_range", "vdt_p_sample_host",
+           "vdt_p_sample_inpaint", "vdt_p_sample_range_inpaint",
            "vdt_step_coefficients", "vdt_plan_flops", "vdt_profile_enable", "vdt_profile_read",
            "vdt_op_conv", "vdt_op_groupnorm", "vdt_op_attention", "vdt_op_sampler_step", "vdt_op_sampler_step_hist",
-           "vdt_stat_slabs_per_image",
+           "vdt_op_sampler_step_known",           "vdt_stat_slabs_per_image",
            "vdt_plan_saturations", "vdt_images_to_uint8",
            "vdt_train_coefficients", "vdt_q_sample", "vdt_train_loss", "vdt_unet_forward_train", "vdt_op_groupnorm_dropout",
            "vdt_op_conv_dgrad", "vdt_op_conv_wgrad", "vdt_op_groupnorm_backward",

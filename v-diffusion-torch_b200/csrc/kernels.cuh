@@ -221,12 +221,19 @@ struct SamplerState {
                                        // p_sample_progressive does (diffusion.py:421: `t = torch.empty(B)`)
     const float* noise;                // injected per-step noise [T, Btotal, C, HW] or null
     long long noise_step_stride;       // elements between steps (Btotal*C*HW)
-    unsigned long long seed;           // on-device Philox noise when `noise` is null and std > 0
-    unsigned long long pad;
+    unsigned long long seed;           // on-device Philox noise when `noise` is null and std > 0; stream 1 of the same key
+                                       // gives the inpainting draws when `known_noise` is null
+    float known_a, known_s;            // inpainting: alpha_s, sigma_s of this step's s (slots 0, 1 of row step - 1)
     float coef[16];                    // one row of vdt_step_coefficients (include/vdt_b200.h)
+    // Inpainting by replacement (include/vdt_b200.h vdt_inpaint): null mask = off.  Full-batch tensors indexed like
+    // `noise` (img0 * CHW + element; known_noise also by step * noise_step_stride), possibly at odd offsets.
+    const float* known;                // [Btotal, C, HW] known image in model space
+    const float* mask;                 // [Btotal, C, HW] in [0, 1], 1 = known
+    const float* known_noise;          // [T, Btotal, C, HW] injected z' or null
 };
 constexpr int kCoefStride = 16;
-// single-thread kernel: st->step = st->next_step--, copies the coefficient row, writes t_rows[r] = (step+1)/T
+// single-thread kernel: st->step = st->next_step--, copies the coefficient row (and slots 0, 1 of row step - 1 into
+// known_a / known_s when step > 0), writes t_rows[r] = (step+1)/T
 cudaError_t launch_sampler_begin_step(SamplerState* st, const float* coef_table, double* t_rows, int nrows, int T,
                                       cudaStream_t stream);
 

@@ -219,11 +219,14 @@ __global__ void multitag_rows_kernel(const float* __restrict__ label, float* __r
     const int r = i / ncls, k = i % ncls;
     y_rows[i] = (rep == 2 && (r & 1)) ? 0.f : label[(size_t)(r / rep) * ncls + k];
 }
+// every per-call field is written, the inpainting pointers too (null when the call has none): execs are reused across calls
 __global__ void sampler_init_state_kernel(SamplerState* st, int next_step, int img0, int t_fp32, const float* noise,
-                                          long long noise_stride, unsigned long long seed) {
+                                          long long noise_stride, unsigned long long seed, vdt_inpaint inp) {
     if (threadIdx.x == 0 && blockIdx.x == 0) {
         st->next_step = next_step; st->step = next_step; st->img0 = img0; st->t_fp32 = t_fp32;
-        st->noise = noise; st->noise_step_stride = noise_stride; st->seed = seed; st->pad = 0;
+        st->noise = noise; st->noise_step_stride = noise_stride; st->seed = seed;
+        st->known_a = 0.f; st->known_s = 0.f;
+        st->known = inp.known; st->mask = inp.mask; st->known_noise = inp.known_noise;
     }
 }
 __global__ void set_u64_kernel(unsigned long long* p, unsigned long long v) {
@@ -1620,10 +1623,20 @@ static int get_sampler_exec(vdt_plan* p, const vdt_sampler_config& sc, int imgs,
     return 0;
 }
 
-extern "C" int vdt_p_sample_range(vdt_plan* p, const vdt_sampler_config* scp, float* x, const void* label,
-                                  const float* step_noise, int32_t batch, int32_t first_step, int32_t num_steps,
-                                  float* pred_x0, void* stream) {
+// known and mask come together; known_noise only with both
+static int check_inpaint(const float* known, const float* mask, const float* known_noise) {
+    if ((known == nullptr) != (mask == nullptr))
+        return fail("inpainting needs both known and mask (got %s without %s)", known ? "known" : "mask", known ? "mask" : "known");
+    if (known_noise && !mask) return fail("inpainting known_noise needs known and mask");
+    return 0;
+}
+
+extern "C" int vdt_p_sample_range_inpaint(vdt_plan* p, const vdt_sampler_config* scp, const vdt_inpaint* inpaint, float* x,
+                                          const void* label, const float* step_noise, int32_t batch, int32_t first_step,
+                                          int32_t num_steps, float* pred_x0, void* stream) {
     if (!p || !scp || !x) return fail("null argument");
+    const vdt_inpaint inp = inpaint ? *inpaint : vdt_inpaint{nullptr, nullptr, nullptr};
+    CKI(check_inpaint(inp.known, inp.mask, inp.known_noise));
     const vdt_sampler_config& sc = *scp;
     const int T = sc.sample_timesteps;
     CKI(check_solver(sc));
@@ -1679,7 +1692,7 @@ extern "C" int vdt_p_sample_range(vdt_plan* p, const vdt_sampler_config* scp, fl
         }
         CK(cudaGetLastError());
         sampler_init_state_kernel<<<1, 32, 0, st>>>(ex->state, first_step, i0, sc.t_fp32 ? 1 : 0, step_noise,
-                                                    (long long)batch * (long long)CHW, (unsigned long long)sc.seed);
+                                                    (long long)batch * (long long)CHW, (unsigned long long)sc.seed, inp);
         CK(cudaGetLastError());
         g_launches += 2;
         for (int step = 0; step < num_steps; ++step) CKI(run_exec(p, ex, st));
@@ -1694,13 +1707,26 @@ extern "C" int vdt_p_sample_range(vdt_plan* p, const vdt_sampler_config* scp, fl
     return leave_work(p, user);
 }
 
-extern "C" int vdt_p_sample(vdt_plan* p, const vdt_sampler_config* scp, const float* noise, const void* label,
-                            const float* step_noise, float* out, int32_t batch, void* stream) {
+extern "C" int vdt_p_sample_range(vdt_plan* p, const vdt_sampler_config* scp, float* x, const void* label,
+                                  const float* step_noise, int32_t batch, int32_t first_step, int32_t num_steps,
+                                  float* pred_x0, void* stream) {
+    return vdt_p_sample_range_inpaint(p, scp, nullptr, x, label, step_noise, batch, first_step, num_steps, pred_x0, stream);
+}
+
+extern "C" int vdt_p_sample_inpaint(vdt_plan* p, const vdt_sampler_config* scp, const vdt_inpaint* inpaint, const float* noise,
+                                    const void* label, const float* step_noise, float* out, int32_t batch, void* stream) {
     if (!p || !scp || !noise || !out) return fail("null argument");
+    if (inpaint) CKI(check_inpaint(inpaint->known, inpaint->mask, inpaint->known_noise));
     const size_t CHW = (size_t)p->cfg.in_channels * p->cfg.resolution * p->cfg.resolution;
     cudaStream_t user = reinterpret_cast<cudaStream_t>(stream);
     if (out != noise) CK(cudaMemcpyAsync(out, noise, (size_t)batch * CHW * 4, cudaMemcpyDeviceToDevice, user));
-    return vdt_p_sample_range(p, scp, out, label, step_noise, batch, scp->sample_timesteps - 1, scp->sample_timesteps, nullptr, stream);
+    return vdt_p_sample_range_inpaint(p, scp, inpaint, out, label, step_noise, batch, scp->sample_timesteps - 1,
+                                      scp->sample_timesteps, nullptr, stream);
+}
+
+extern "C" int vdt_p_sample(vdt_plan* p, const vdt_sampler_config* scp, const float* noise, const void* label,
+                            const float* step_noise, float* out, int32_t batch, void* stream) {
+    return vdt_p_sample_inpaint(p, scp, nullptr, noise, label, step_noise, out, batch, stream);
 }
 
 extern "C" int vdt_p_sample_host(vdt_plan* p, const vdt_sampler_config* scp, const float* noise, const void* label,
@@ -1969,15 +1995,21 @@ extern "C" int vdt_images_to_uint8(const float* x, uint8_t* out, int32_t batch, 
 
 static int op_sampler_step_impl(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
                                 int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step,
-                                const float* coef_host, float w, float* pred_hist, void* stream) {
+                                const float* coef_host, float w, float* pred_hist, const float* known, const float* mask,
+                                const float* known_noise, uint64_t seed, const float* coef_prev_host, void* stream) {
     if (!coef_host) return fail("null argument");
     if (coef_host[15] != 0.0f && !pred_hist)
         return fail("coefficient row %d is a DPM-Solver++(2M) row (c2k != 0): use vdt_op_sampler_step_hist with the previous "
                     "step's guided x0", step);
+    CKI(check_inpaint(known, mask, known_noise));
+    if (mask && step > 0 && !coef_prev_host)
+        return fail("inpainting at step %d > 0 needs coefficient row %d (alpha_s, sigma_s of this step's s)", step, step - 1);
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     SamplerState hs{};
-    hs.next_step = step - 1; hs.step = step; hs.img0 = 0; hs.noise = noise; hs.noise_step_stride = 0; hs.seed = 0;
+    hs.next_step = step - 1; hs.step = step; hs.img0 = 0; hs.noise = noise; hs.noise_step_stride = 0; hs.seed = seed;
     for (int i = 0; i < kCoefStride; ++i) hs.coef[i] = coef_host[i];
+    hs.known = known; hs.mask = mask; hs.known_noise = known_noise;
+    if (mask && step > 0) { hs.known_a = coef_prev_host[0]; hs.known_s = coef_prev_host[1]; }
     SamplerState* ds = nullptr;
     CK(cudaMalloc(&ds, sizeof(SamplerState)));
     CK(cudaMemcpy(ds, &hs, sizeof(hs), cudaMemcpyHostToDevice));
@@ -1997,14 +2029,24 @@ static int op_sampler_step_impl(const float* model_out, const float* x_t, const 
 extern "C" int vdt_op_sampler_step(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
                                    int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step,
                                    const float* coef_host, float w, void* stream) {
-    return op_sampler_step_impl(model_out, x_t, noise, x_s, batch, c, hw, cfg, model_out_type, step, coef_host, w, nullptr, stream);
+    return op_sampler_step_impl(model_out, x_t, noise, x_s, batch, c, hw, cfg, model_out_type, step, coef_host, w, nullptr,
+                                nullptr, nullptr, nullptr, 0, nullptr, stream);
 }
 
 extern "C" int vdt_op_sampler_step_hist(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
                                         int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step,
                                         const float* coef_host, float w, float* pred_hist, void* stream) {
     if (!pred_hist) return fail("null pred_hist");
-    return op_sampler_step_impl(model_out, x_t, noise, x_s, batch, c, hw, cfg, model_out_type, step, coef_host, w, pred_hist, stream);
+    return op_sampler_step_impl(model_out, x_t, noise, x_s, batch, c, hw, cfg, model_out_type, step, coef_host, w, pred_hist,
+                                nullptr, nullptr, nullptr, 0, nullptr, stream);
+}
+
+extern "C" int vdt_op_sampler_step_known(const float* model_out, const float* x_t, const float* noise, float* x_s, int32_t batch,
+                                         int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step,
+                                         const float* coef_host, float w, float* pred_hist, const float* known, const float* mask,
+                                         const float* known_noise, uint64_t seed, const float* coef_prev_host, void* stream) {
+    return op_sampler_step_impl(model_out, x_t, noise, x_s, batch, c, hw, cfg, model_out_type, step, coef_host, w, pred_hist,
+                                known, mask, known_noise, seed, coef_prev_host, stream);
 }
 
 // ---- entry points the composed training step (v-diffusion-torch_b200/training.py) adds to the kernel-level hooks ----------

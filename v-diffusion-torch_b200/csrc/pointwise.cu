@@ -198,6 +198,11 @@ __global__ void sampler_begin_step_kernel(SamplerState* st, const float* __restr
         st->step = step;
         st->next_step = step - 1;
         for (int i = 0; i < kCoefStride; ++i) st->coef[i] = coef_table[step * kCoefStride + i];
+        // inpainting: the known image is diffused to this step's s = step / T, which is row step - 1's t (in both t modes)
+        if (step > 0) {
+            st->known_a = coef_table[(step - 1) * kCoefStride + 0];
+            st->known_s = coef_table[(step - 1) * kCoefStride + 1];
+        }
         // t = (step + 1) / T: fp64 in p_sample (diffusion.py:399, 364), fp32 in p_sample_progressive (diffusion.py:421)
         const double t = st->t_fp32 ? static_cast<double>(__fdiv_rn(static_cast<float>(step + 1), static_cast<float>(T)))
                                     : static_cast<double>(step + 1) / static_cast<double>(T);
@@ -207,9 +212,10 @@ __global__ void sampler_begin_step_kernel(SamplerState* st, const float* __restr
 
 // Philox4x32-10 counter RNG + Box-Muller for on-device ancestral noise (used only when no noise
 // tensor is injected; the stream is this library's own, not torch's).  One counter value yields the four
-// normals of elements 4q .. 4q+3.
-__device__ __forceinline__ float4 philox_normal4(unsigned long long seed, uint32_t step, unsigned long long quad) {
-    const uint4 r = philox4x32(make_uint4(static_cast<uint32_t>(quad), static_cast<uint32_t>(quad >> 32), step, 0u),
+// normals of elements 4q .. 4q+3.  Counter word 3 selects the stream: 0 ancestral noise, 1 inpainting's z'.
+__device__ __forceinline__ float4 philox_normal4(unsigned long long seed, uint32_t step, unsigned long long quad,
+                                                 uint32_t stream = 0u) {
+    const uint4 r = philox4x32(make_uint4(static_cast<uint32_t>(quad), static_cast<uint32_t>(quad >> 32), step, stream),
                                make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)));
     const float k = 1.0f / 16777216.0f;
     const float u1 = (static_cast<float>(r.x >> 8) + 0.5f) * k, u2 = (static_cast<float>(r.y >> 8) + 0.5f) * k;
@@ -236,8 +242,10 @@ template <> struct SVec<1> { typedef float type; };
 
 // One thread owns VEC (4 or 1) consecutive elements of one image: every tensor is read / written once with 16-byte
 // (VEC = 4) fully coalesced accesses; the per-step scalars come from the device-side SamplerState.
+// Six 256-thread blocks per SM (<= 42 registers): the occupancy the kernel had before inpainting added its branch, which a
+// memory-bound kernel needs to keep its latency hidden (without the bound: 48 registers, five blocks, ~12 % slower).
 template <int VEC>
-__global__ void __launch_bounds__(256) sampler_step_kernel(const SamplerStepParams p) {
+__global__ void __launch_bounds__(256, 6) sampler_step_kernel(const SamplerStepParams p) {
     typedef typename SVec<VEC>::type vec_t;
     const long long n = static_cast<long long>(p.B) * p.C * p.HW;
     const long long i = (blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x) * VEC;
@@ -250,6 +258,8 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const SamplerStepPara
         cf[k] = c4.x; cf[k + 1] = c4.y; cf[k + 2] = c4.z; cf[k + 3] = c4.w;
     }
     const int step = st->step;
+    // read with the other state fields: the stores below may alias *st, so a later read could not be hoisted above them
+    const float* const mask = st->mask;
     const int chw = p.C * p.HW;
     const int b = static_cast<int>(i / chw), e = static_cast<int>(i % chw);
     const int Cm = (p.model_out_type == 2) ? 2 * p.C : p.C;
@@ -270,6 +280,14 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const SamplerStepPara
         for (int k = 0; k < VEC; ++k) f[k] = v[k];
         *reinterpret_cast<vec_t*>(q) = t;
     };
+    auto ldu = [&ldv](const float* q, float (&v)[VEC]) {            // caller-owned tensors may sit at odd offsets
+        if (VEC == 1 || (reinterpret_cast<uintptr_t>(q) & 15u) == 0) {
+            ldv(q, v);
+        } else {
+#pragma unroll
+            for (int k = 0; k < VEC; ++k) v[k] = q[k];
+        }
+    };
     ldv(p.x_t + i, x);
     ldv(mo, o);
     if (p.model_out_type == 2) ldv(mo + second, o2);
@@ -281,16 +299,10 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const SamplerStepPara
     const bool last = (step == 0);
     const bool noisy = !last && sd > 0.f;
     float z[VEC];
+    const long long gi = static_cast<long long>(st->img0) * chw + i;          // element index inside the whole batch
     if (noisy) {
-        const long long gi = static_cast<long long>(st->img0) * chw + i;      // element index inside the whole batch
         if (st->noise) {
-            const float* zp = st->noise + static_cast<long long>(step) * st->noise_step_stride + gi;
-            if (VEC == 1 || (reinterpret_cast<uintptr_t>(zp) & 15u) == 0) {
-                ldv(zp, z);
-            } else {                                                   // caller-owned tensor at an odd offset
-#pragma unroll
-                for (int k = 0; k < VEC; ++k) z[k] = zp[k];
-            }
+            ldu(st->noise + static_cast<long long>(step) * st->noise_step_stride + gi, z);
         } else {
             const float4 g = philox_normal4(st->seed, static_cast<uint32_t>(step), static_cast<unsigned long long>(gi) >> 2);
             const float gv[4] = {g.x, g.y, g.z, g.w};
@@ -327,6 +339,30 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const SamplerStepPara
         for (int k = 0; k < VEC; ++k) out[k] = fmaf(c2k, pr[k] - pp[k], out[k]);
     }
     if (p.pred_x0) stv(p.pred_x0 + i, pr);
+    // Inpainting by replacement (Song et al., 2021, App. I): x_s = m k_s + (1 - m) x_s with k_s = alpha_s known + sigma_s z'
+    // (z' fresh per step, independent of the ancestral draws), and k_0 = known at the last step.  Written as m k + (1 - m) x
+    // so m = 0 returns x_s and m = 1 returns k_s bit for bit.  pred (above) stays the model's guided x0.
+    if (mask) {
+        float m[VEC], kn[VEC];
+        ldu(mask + gi, m);
+        ldu(st->known + gi, kn);
+        if (!last) {
+            float zk[VEC];
+            if (st->known_noise) {
+                ldu(st->known_noise + static_cast<long long>(step) * st->noise_step_stride + gi, zk);
+            } else {
+                const float4 g = philox_normal4(st->seed, static_cast<uint32_t>(step), static_cast<unsigned long long>(gi) >> 2, 1u);
+                const float gv[4] = {g.x, g.y, g.z, g.w};
+#pragma unroll
+                for (int k = 0; k < VEC; ++k) zk[k] = gv[(VEC == 4) ? k : static_cast<int>(gi & 3)];
+            }
+            const float a = st->known_a, s = st->known_s;
+#pragma unroll
+            for (int k = 0; k < VEC; ++k) kn[k] = fmaf(a, kn[k], s * zk[k]);
+        }
+#pragma unroll
+        for (int k = 0; k < VEC; ++k) out[k] = fmaf(m[k], kn[k], (1.f - m[k]) * out[k]);
+    }
     stv(p.x_s + i, out);
 }
 

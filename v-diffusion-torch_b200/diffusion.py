@@ -127,6 +127,47 @@ class GaussianDiffusion:
                     raise RuntimeError(f"class ids must lie in [0, {num_classes}] (0 = unconditional), got [{lo}, {hi}]")
         return label
 
+    def _check_inpaint(self, shape, known, mask, known_noise):
+        """Inpainting inputs (extension; include/vdt_b200.h vdt_inpaint) as fp32 tensors on the caller's devices, or None when
+        there are none.  ``known``: the image in model space, shaped like the batch; ``mask``: 1 = known pixel, values in
+        [0, 1], shaped like the batch or (B, 1, R, R); ``known_noise``: optional (T,) + shape draws of z'.  Everything is
+        checked here because the library only sees raw pointers; the value checks share one device synchronisation."""
+        if known is None and mask is None:
+            if known_noise is not None:
+                raise ValueError("known_noise needs known and mask")
+            return None
+        if (known is None) != (mask is None):
+            raise ValueError("inpainting needs both known and mask")
+        shape = tuple(shape)
+        if tuple(known.shape) != shape:
+            raise ValueError(f"known has shape {tuple(known.shape)}, expected {shape}")
+        if tuple(mask.shape) not in (shape, shape[:1] + (1,) + shape[2:]):
+            raise ValueError(f"mask has shape {tuple(mask.shape)}, expected {shape} or {shape[:1] + (1,) + shape[2:]}")
+        if known_noise is not None and tuple(known_noise.shape) != (self.sample_timesteps,) + shape:
+            raise ValueError(f"known_noise has shape {tuple(known_noise.shape)}, expected {(self.sample_timesteps,) + shape}")
+        known, mask = known.to(torch.float32), mask.to(torch.float32)
+        flags = [torch.isfinite(known).all(), ((mask >= 0) & (mask <= 1)).all()]
+        if known_noise is not None:
+            known_noise = known_noise.to(torch.float32)
+            flags.append(torch.isfinite(known_noise).all())
+        ok = torch.stack([f.to(known.device) for f in flags]).tolist()
+        if not ok[0]:
+            raise ValueError("known must be finite")
+        if not ok[1]:
+            raise ValueError("mask values must lie in [0, 1]")
+        if known_noise is not None and not ok[2]:
+            raise ValueError("known_noise must be finite")
+        return known, mask, known_noise
+
+    @staticmethod
+    def _inpaint_on(inp, shape, device):
+        """The checked inputs as contiguous device tensors (the mask expanded over channels) and their vdt_inpaint struct."""
+        known, mask, known_noise = inp
+        known = known.to(device).contiguous()
+        mask = mask.to(device).expand(tuple(shape)).contiguous()
+        known_noise = None if known_noise is None else known_noise.to(device).contiguous()
+        return (known, mask, known_noise), _lib.Inpaint(_lib.ptr(known), _lib.ptr(mask), _lib.ptr(known_noise))
+
     def step_coefficients(self, use_ddim, solver=None):
         """[T, 16] fp32 host table (include/vdt_b200.h: vdt_step_coefficients); slot 15 holds DPM-Solver++(2M)'s c2k."""
         sc = self.sampler_config(use_ddim, solver=solver)
@@ -137,11 +178,16 @@ class GaussianDiffusion:
     # ------------------------------------------------------------------ p_sample (diffusion.py:394-414)
     @torch.no_grad()
     def p_sample(self, denoise_fn, shape, noise=None, label=None, device="cpu", seed=None, use_ddim=False,
-                 step_noise=None, solver=None):
+                 step_noise=None, solver=None, known=None, mask=None, known_noise=None):
         """``step_noise`` (extension): optional (T, B, C, H, W) tensor of the per-step normal draws the
         reference takes from its generator (diffusion.py:389), so both sides inject identical noise.
-        ``solver`` (extension): None (the reference's step) or "dpmpp_2m" (DPM-Solver++(2M), with use_ddim=True)."""
+        ``solver`` (extension): None (the reference's step) or "dpmpp_2m" (DPM-Solver++(2M), with use_ddim=True).
+        ``known``, ``mask``, ``known_noise`` (extension): inpainting by replacement.  After every step the pixels with mask 1
+        are set to ``known`` diffused to the step's time (alpha_s known + sigma_s z'), and the last step sets them to ``known``;
+        a soft mask blends.  z' comes from ``known_noise`` or else from the library's noise stream keyed by ``seed`` (a fresh
+        seed when None, under DDIM too).  See include/vdt_b200.h vdt_inpaint."""
         self._check_solver(solver, use_ddim)
+        inp = self._check_inpaint(shape, known, mask, known_noise)
         device = torch.device(device)
         if device.type != "cuda":
             raise RuntimeError("v_diffusion_b200 samples on CUDA (sm_100a) only; there is no CPU fallback")
@@ -164,29 +210,39 @@ class GaussianDiffusion:
             if tuple(step_noise.shape) != (self.sample_timesteps,) + tuple(shape):
                 raise ValueError(f"step_noise must have shape {(self.sample_timesteps,) + tuple(shape)}")
         L = _lib.lib()
+        # inpainting without injected z' draws it from the library's stream keyed by the call's seed, under DDIM too
+        inp_seed = inp is not None and known_noise is None
         if isinstance(denoise_fn, UNet):
             # fused path: the per-step normals come from the library's own Philox stream keyed by this call's seed
-            sc = self.sampler_config(use_ddim, self._noise_seed(seed) if (not use_ddim and step_noise is None) else seed,
-                                     solver=solver)
+            sc = self.sampler_config(use_ddim, self._noise_seed(seed) if ((not use_ddim and step_noise is None) or inp_seed)
+                                     else seed, solver=solver)
             plan = denoise_fn.plan_for(shape[2], device)
             out = torch.empty_like(x_t)
             with torch.cuda.device(device):
-                _lib.check(L.vdt_p_sample(plan, C.byref(sc), _lib.ptr(x_t), _lib.ptr(label), _lib.ptr(step_noise),
-                                          _lib.ptr(out), B, _lib.current_stream_ptr()))
+                if inp is None:
+                    _lib.check(L.vdt_p_sample(plan, C.byref(sc), _lib.ptr(x_t), _lib.ptr(label), _lib.ptr(step_noise),
+                                              _lib.ptr(out), B, _lib.current_stream_ptr()))
+                else:
+                    held, ip = self._inpaint_on(inp, shape, device)      # `held` keeps the tensors alive for the call
+                    _lib.check(L.vdt_p_sample_inpaint(plan, C.byref(sc), C.byref(ip), _lib.ptr(x_t), _lib.ptr(label),
+                                                      _lib.ptr(step_noise), _lib.ptr(out), B, _lib.current_stream_ptr()))
             return out.cpu()
         # generic callable: same fused update kernel, one step at a time; the per-step normals continue the generator
         # that produced x_T, like the reference's single generator (diffusion.py:401-405, 389)
-        sc = self.sampler_config(use_ddim, seed, solver=solver)
-        return self._p_sample_generic(denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver).cpu()
+        sc = self.sampler_config(use_ddim, self._noise_seed(seed) if inp_seed else seed, solver=solver)
+        held = None if inp is None else self._inpaint_on(inp, shape, device)[0]
+        return self._p_sample_generic(denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver, held).cpu()
 
     @torch.no_grad()
     def p_sample_progressive(self, denoise_fn, shape, noise=None, label=None, device="cpu", seed=None, use_ddim=False,
-                             pred_freq=50, step_noise=None, solver=None):
+                             pred_freq=50, step_noise=None, solver=None, known=None, mask=None, known_noise=None):
         """diffusion.py:416-441: returns (x_0, preds) where preds[k] is the (guided) x0 prediction made at the
         steps ti with (ti + 1) % pred_freq == 0, ordered like the reference (index L-1 = earliest).  Fused path only.
         ``solver`` as in p_sample; under "dpmpp_2m" the ``pred`` buffer every range call shares carries the previous
-        step's guided x0 into the next call."""
+        step's guided x0 into the next call.  ``known``, ``mask``, ``known_noise`` as in p_sample; the previews stay the
+        model's guided x0 predictions."""
         self._check_solver(solver, use_ddim)
+        inp = self._check_inpaint(shape, known, mask, known_noise)
         if not isinstance(denoise_fn, UNet):
             raise TypeError("p_sample_progressive needs the v_diffusion_b200 UNet")
         device = torch.device(device)
@@ -201,8 +257,10 @@ class GaussianDiffusion:
         if step_noise is not None:
             step_noise = step_noise.to(device=device, dtype=torch.float32).contiguous()
         # the reference's progressive loop carries an fp32 step tensor (diffusion.py:421): fp32 s / t and an fp32 sinusoid
-        sc = self.sampler_config(use_ddim, self._noise_seed(seed) if (not use_ddim and step_noise is None) else seed, t_fp32=True,
-                                 solver=solver)
+        inp_seed = inp is not None and known_noise is None
+        sc = self.sampler_config(use_ddim, self._noise_seed(seed) if ((not use_ddim and step_noise is None) or inp_seed) else seed,
+                                 t_fp32=True, solver=solver)
+        held, ip = self._inpaint_on(inp, shape, device) if inp is not None else (None, None)   # `held` keeps them alive
         plan = denoise_fn.plan_for(shape[2], device)
         Lp = T // pred_freq
         preds = torch.zeros((Lp, B) + tuple(shape[1:]), dtype=torch.float32)
@@ -215,8 +273,13 @@ class GaussianDiffusion:
                 record = stop >= 0
                 if not record:
                     stop = 0
-                _lib.check(lib.vdt_p_sample_range(plan, C.byref(sc), _lib.ptr(x), _lib.ptr(label), _lib.ptr(step_noise), B,
-                                                  first, first - stop + 1, _lib.ptr(pred), _lib.current_stream_ptr()))
+                if ip is None:
+                    _lib.check(lib.vdt_p_sample_range(plan, C.byref(sc), _lib.ptr(x), _lib.ptr(label), _lib.ptr(step_noise), B,
+                                                      first, first - stop + 1, _lib.ptr(pred), _lib.current_stream_ptr()))
+                else:
+                    _lib.check(lib.vdt_p_sample_range_inpaint(plan, C.byref(sc), C.byref(ip), _lib.ptr(x), _lib.ptr(label),
+                                                              _lib.ptr(step_noise), B, first, first - stop + 1, _lib.ptr(pred),
+                                                              _lib.current_stream_ptr()))
                 if record and idx > 0:
                     idx -= 1
                     preds[idx] = pred.cpu()
@@ -274,7 +337,7 @@ class GaussianDiffusion:
                                         _lib.REWEIGHT_TYPES[self.reweight_type], _lib.current_stream_ptr()))
         return (loss, grad) if return_grad else loss
 
-    def _p_sample_generic(self, denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver=None):
+    def _p_sample_generic(self, denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver=None, inp=None):
         L = _lib.lib()
         B = shape[0]
         coefs = self.step_coefficients(use_ddim, solver)
@@ -298,7 +361,14 @@ class GaussianDiffusion:
                     z = step_noise[ti] if step_noise is not None else torch.randn(shape, device=device, generator=gen)
                     z = z.contiguous()
                 x_s = torch.empty_like(x_t)
-                if hist is None:
+                if inp is not None:
+                    known, mask, known_noise = inp
+                    _lib.check(L.vdt_op_sampler_step_known(
+                        _lib.ptr(model_out), _lib.ptr(x_t), _lib.ptr(z), _lib.ptr(x_s), B, shape[1], hw, int(use_cfg),
+                        sc.model_out_type, ti, _lib.ptr(coefs[ti].contiguous()), float(self.w_guide), _lib.ptr(hist),
+                        _lib.ptr(known), _lib.ptr(mask), None if known_noise is None else _lib.ptr(known_noise[ti]), sc.seed,
+                        _lib.ptr(coefs[ti - 1].contiguous()) if ti > 0 else None, _lib.current_stream_ptr()))
+                elif hist is None:
                     _lib.check(L.vdt_op_sampler_step(_lib.ptr(model_out), _lib.ptr(x_t), _lib.ptr(z), _lib.ptr(x_s), B,
                                                      shape[1], hw, int(use_cfg), sc.model_out_type, ti,
                                                      _lib.ptr(coefs[ti].contiguous()), float(self.w_guide),
