@@ -217,6 +217,44 @@ int vdt_adamw_ema_step(float* param, const float* grad, float* exp_avg, float* e
 int vdt_op_conv(const void* x_16_nhwc, int32_t batch, int32_t h, int32_t w, int32_t cin, const float* w_oihw,
                 int32_t cout, int32_t ksize, const float* bias, const float* residual, float* out_nhwc, int32_t f16,
                 void* out16, void* stats_out, int32_t stat_cols, void* stream);
+/* One conv of the UNet plan in any of the modes the sampler runs, packed by the plan's own weight packers and launched
+ * through the same setup: sub-pixel 2x-upsampling conv (ups), fused 1x1 skip conv (a1 / w1 appended as extra K),
+ * split-precision operands (a3_lo / a1_lo, operand_dtype 2), upsampled or pair-shared residuals, 16-bit output, GroupNorm
+ * statistics and the fp16 saturation counter.  H, W = 2h, 2w when ups = 1, else h, w.  Refused (before any CUDA call):
+ * ups with a1 or a residual; resid_mode 1 with odd H or W; resid_mode 2 with an odd batch; a3_lo without a1_lo when a1 is
+ * given, or the reverse; c3, c1 or cout off the multiples of 64; stats where vdt_op_conv has no layout for H x W, and for
+ * ups also where 4 * slabs(h, w) != slabs(H, W) (e.g. 14 -> 28). */
+typedef struct vdt_conv_op {
+    const void* a3;               /* 16-bit NHWC [batch, h, w, c3]: the 3x3 operand (the low-resolution input when ups = 1) */
+    const void* a3_lo;            /* NULL, or the lo halves of a3: split-precision mode, round16(x - round16(x)) */
+    const void* a1;               /* NULL, or 16-bit NHWC [batch, H, W, c1]: operand of the fused 1x1 skip conv */
+    const void* a1_lo;            /* lo halves of a1, given exactly when a1 and a3_lo are */
+    const float* w3;              /* fp32 OIHW [cout, c3, 3, 3] */
+    const float* w1;              /* fp32 OIHW [cout, c1, 1, 1], given exactly when a1 is */
+    const float* bias;            /* fp32 [cout]: the conv bias (plus the skip conv's, which the plan adds into it) */
+    const float* residual;        /* NULL or fp32 NHWC, read per resid_mode */
+    float* out_f32;               /* fp32 NHWC [batch, H, W, cout]; exactly one of out_f32 and out16 */
+    void* out16;                  /* 16-bit NHWC [batch, H, W, cout] in the operand format (fp16 saturates at +-65504) */
+    void* stats;                  /* NULL or float2 [batch * vdt_stat_slabs_per_image(H, W) + 4][cout / stat_cols] */
+    uint64_t* sat_count;          /* NULL or a device counter: +1 per (warp, 32x32 chunk) whose fp16 store saturated */
+    int32_t batch, h, w;          /* a3's shape */
+    int32_t c3, c1, cout;
+    int32_t ups;                  /* 1: conv3x3(nearest_upsample_2x(a3)) in the sub-pixel form */
+    int32_t resid_mode;           /* 0: residual [batch, H, W, cout]; 1: [batch, H/2, W/2, cout], output pixel (y, x) adds
+                                     (y/2, x/2); 2: [batch/2, H, W, cout], output image i adds residual image i/2 */
+    int32_t stat_cols;            /* 4 or 2 columns per statistics entry */
+    int32_t f16;                  /* 1 fp16 operands, 0 bf16 */
+} vdt_conv_op;
+int vdt_op_conv_ex(const vdt_conv_op* op, void* stream);
+/* The network's first conv as the plan runs it (im2col into 64 patch columns, then a pointwise GEMM): x fp32 NCHW
+ * [batch, c, h, w] with 1 <= c <= 7, w fp32 OIHW [hid, c, 3, 3], bias [hid] -> out fp32 NHWC [batch * rep, h, w, hid], where
+ * output image i reads input image i / rep (rep = 2: the CFG pair interleave); stats_out as for vdt_op_conv. */
+int vdt_op_in_conv(const float* x_nchw, int32_t batch, int32_t rep, int32_t c, int32_t h, int32_t w, const float* w_oihw,
+                   const float* bias, int32_t hid, float* out_nhwc, void* stats_out, int32_t stat_cols, int32_t f16, void* stream);
+/* The network's last conv as the plan runs it (a pointwise GEMM over tap-major weight rows, then a tap-sum gather): a 16-bit
+ * NHWC [batch, h, w, c0], w fp32 OIHW [cout, c0, 3, 3] with 1 <= cout <= 16, bias [cout] -> out fp32 NCHW [batch, cout, h, w]. */
+int vdt_op_out_conv(const void* a_16_nhwc, int32_t batch, int32_t h, int32_t w, int32_t c0, const float* w_oihw, int32_t cout,
+                    const float* bias, float* out_nchw, int32_t f16, void* stream);
 /* Backward of a conv layer (F.conv2d under autograd, modules.py:141-144).
  * dgrad: dX fp32 NHWC [B, H, W, cin] = conv(dY, W rotated 180 degrees with its channel axes swapped) on the forward kernel;
  *        dy 16-bit NHWC [B, H, W, cout], w fp32 OIHW [cout, cin, k, k].

@@ -23,6 +23,7 @@ def test_library_exports_every_declared_symbol():
 def test_struct_layout_matches_header():
     assert C.sizeof(_lib.UNetConfig) == 4 * (4 + 8 + 1 + 8 + 8)
     assert C.sizeof(_lib.SamplerConfig) == 8 * 4 + 4 * 8 + 8
+    assert C.sizeof(_lib.ConvOp) == 12 * 8 + 10 * 4               # vdt_conv_op: 12 pointers, 10 int32
 
 
 def test_step_coefficients_match_reference(golden_dir):

@@ -45,6 +45,15 @@ class Inpaint(C.Structure):                               # include/vdt_b200.h v
     _fields_ = [("known", C.c_void_p), ("mask", C.c_void_p), ("known_noise", C.c_void_p)]
 
 
+class ConvOp(C.Structure):                                # include/vdt_b200.h vdt_conv_op
+    _fields_ = [("a3", C.c_void_p), ("a3_lo", C.c_void_p), ("a1", C.c_void_p), ("a1_lo", C.c_void_p),
+                ("w3", C.c_void_p), ("w1", C.c_void_p), ("bias", C.c_void_p), ("residual", C.c_void_p),
+                ("out_f32", C.c_void_p), ("out16", C.c_void_p), ("stats", C.c_void_p), ("sat_count", C.c_void_p),
+                ("batch", C.c_int32), ("h", C.c_int32), ("w", C.c_int32), ("c3", C.c_int32), ("c1", C.c_int32),
+                ("cout", C.c_int32), ("ups", C.c_int32), ("resid_mode", C.c_int32), ("stat_cols", C.c_int32),
+                ("f16", C.c_int32)]
+
+
 def nvcc_path():
     for cand in (os.environ.get("NVCC"), shutil.which("nvcc"), "/usr/local/cuda/bin/nvcc"):
         if cand and os.path.exists(cand):
@@ -114,6 +123,9 @@ def lib():
     L.vdt_p_sample_host.argtypes = [vp, C.POINTER(SamplerConfig), vp, vp, vp, vp, i32]
     L.vdt_step_coefficients.argtypes = [C.POINTER(SamplerConfig), vp]
     L.vdt_op_conv.argtypes = [vp, i32, i32, i32, i32, vp, i32, i32, vp, vp, vp, i32, vp, vp, i32, vp]
+    L.vdt_op_conv_ex.argtypes = [C.POINTER(ConvOp), vp]
+    L.vdt_op_in_conv.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, i32, vp, vp, i32, i32, vp]
+    L.vdt_op_out_conv.argtypes = [vp, i32, i32, i32, i32, vp, i32, vp, vp, i32, vp]
     L.vdt_op_groupnorm.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, i32, vp, vp, i32, i32, vp]
     L.vdt_op_attention.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp]
     L.vdt_op_sampler_step.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, C.c_float, vp]
@@ -150,7 +162,7 @@ EXPORTS = ["vdt_last_error", "vdt_version", "vdt_kernel_launches", "vdt_plan_cre
            "vdt_plan_finalize", "vdt_unet_forward", "vdt_p_sample", "vdt_p_sample_range", "vdt_p_sample_host",
            "vdt_p_sample_inpaint", "vdt_p_sample_range_inpaint",
            "vdt_step_coefficients", "vdt_plan_flops", "vdt_profile_enable", "vdt_profile_read",
-           "vdt_op_conv", "vdt_op_groupnorm", "vdt_op_attention", "vdt_op_sampler_step", "vdt_op_sampler_step_hist",
+           "vdt_op_conv", "vdt_op_conv_ex", "vdt_op_in_conv", "vdt_op_out_conv", "vdt_op_groupnorm", "vdt_op_attention", "vdt_op_sampler_step", "vdt_op_sampler_step_hist",
            "vdt_op_sampler_step_known",           "vdt_stat_slabs_per_image",
            "vdt_plan_saturations", "vdt_images_to_uint8",
            "vdt_train_coefficients", "vdt_q_sample", "vdt_train_loss", "vdt_unet_forward_train", "vdt_op_groupnorm_dropout",

@@ -617,6 +617,35 @@ static int pack_conv_ups(const float* src, h16* dst, int O, int I, int f16, int 
     return 0;
 }
 
+// 3x3 conv with an optional fused 1x1 skip conv (w1 != null) as extra K: columns [3x3 segments | skip segments at 9 * I3 * km]
+static int pack_conv_skip(const float* w3, const float* w1, h16* dst, int O, int I3, int I1, int f16, int split) {
+    const int km = split ? 3 : 1, ktot = (9 * I3 + (w1 ? I1 : 0)) * km;
+    CKI(pack_conv(w3, dst, O, I3, 9, ktot, 0, f16, split));
+    if (w1) CKI(pack_conv(w1, dst, O, I1, 1, ktot, 9 * I3 * km, f16, split));
+    return 0;
+}
+
+// in_conv: [O][64 * km], the 64 patch columns of launch_im2col3x3 per segment
+static int pack_inconv(const float* src, h16* dst, int O, int C, int f16, int split) {
+    const int km = split ? 3 : 1;
+    for (int part = 0; part < km; ++part) {
+        pack_inconv_w_kernel<<<(O * 64 + 255) / 256, 256>>>(src, dst, O, C, f16, 64 * km, 64 * part, part == 2 ? 1 : 0);
+        CK(cudaGetLastError());
+    }
+    return 0;
+}
+
+// out_conv as a pointwise GEMM over tap-major weight rows (9 * Cout, padded with zero rows to a multiple of 32)
+static int outconv_rows(int cout) { return (9 * cout + 31) / 32 * 32; }
+static int pack_outconv(const float* src, h16* dst, int O, int C, int f16, int split) {
+    const int km = split ? 3 : 1;
+    for (int part = 0; part < km; ++part) {            // split mode: K segments W_hi | W_hi | W_lo
+        pack_outconv_t_kernel<<<(9 * O * C + 255) / 256, 256>>>(src, dst, O, C, f16, C * km, C * part, part == 2 ? 1 : 0);
+        CK(cudaGetLastError());
+    }
+    return 0;
+}
+
 extern "C" int vdt_plan_finalize(vdt_plan* p) {
     if (!p) return fail("null plan");
     for (auto& w : p->weights)
@@ -631,11 +660,7 @@ extern "C" int vdt_plan_finalize(vdt_plan* p) {
     const int sp = p->split, km = sp ? 3 : 1;          // K multiplier of the split mode
     CKI(dev_alloc(p, &p->sat_count, 1));
     CKI(dev_alloc(p, &p->w_in, (size_t)hid * 64 * km));
-    for (int part = 0; part < km; ++part) {
-        pack_inconv_w_kernel<<<(hid * 64 + 255) / 256, 256>>>(p->W("in_conv.weight"), p->w_in, hid, c.in_channels, p->f16, 64 * km,
-                                                             64 * part, part == 2 ? 1 : 0);
-        CK(cudaGetLastError());
-    }
+    CKI(pack_inconv(p->W("in_conv.weight"), p->w_in, hid, c.in_channels, p->f16, sp));
     CKI(dev_alloc(p, &p->w_fc_all, (size_t)p->film_total * E));
     CKI(dev_alloc(p, &p->b_fc_all, (size_t)p->film_total));
     for (auto& b : p->blocks) {
@@ -651,8 +676,8 @@ extern "C" int vdt_plan_finalize(vdt_plan* p) {
             const bool skipconv = b.cin != b.cout;
             const int k2 = (9 * b.cout + (skipconv ? b.cin : 0)) * km;
             CKI(dev_alloc(p, &b.w2, (size_t)b.cout * k2));
-            CKI(pack_conv(p->W(n + ".conv2.weight"), b.w2, b.cout, b.cout, 9, k2, 0, p->f16, sp));
-            if (skipconv) CKI(pack_conv(p->W(n + ".skip.weight"), b.w2, b.cout, b.cin, 1, k2, 9 * b.cout * km, p->f16, sp));
+            CKI(pack_conv_skip(p->W(n + ".conv2.weight"), skipconv ? p->W(n + ".skip.weight") : nullptr, b.w2, b.cout, b.cout, b.cin,
+                               p->f16, sp));
             CKI(dev_alloc(p, &b.bias2, (size_t)b.cout));
             add_vec_kernel<<<(b.cout + 255) / 256, 256>>>(p->W(n + ".conv2.bias"), skipconv ? p->W(n + ".skip.bias") : nullptr,
                                                           b.bias2, b.cout);
@@ -671,15 +696,10 @@ extern "C" int vdt_plan_finalize(vdt_plan* p) {
         }
     }
     const int c0 = hid * c.ch_multipliers[0];
-    // out_conv as a pointwise GEMM over tap-major weight rows (9 * Cout, padded with zero rows to a multiple of 32)
-    p->out_rows = (9 * c.out_channels + 31) / 32 * 32;
+    p->out_rows = outconv_rows(c.out_channels);
     CKI(dev_alloc(p, &p->w_out, (size_t)p->out_rows * c0 * km));
     CKI(dev_alloc(p, &p->zero_bias, (size_t)p->out_rows));
-    for (int part = 0; part < km; ++part) {            // split mode: K segments W_hi | W_hi | W_lo
-        pack_outconv_t_kernel<<<(9 * c.out_channels * c0 + 255) / 256, 256>>>(p->W("out_conv.2.weight"), p->w_out, c.out_channels, c0, p->f16,
-                                                                              c0 * km, c0 * part, part == 2 ? 1 : 0);
-        CK(cudaGetLastError());
-    }
+    CKI(pack_outconv(p->W("out_conv.2.weight"), p->w_out, c.out_channels, c0, p->f16, sp));
     CK(cudaDeviceSynchronize());
     p->finalized = true;
     return 0;
@@ -1802,6 +1822,177 @@ extern "C" int vdt_op_conv(const void* x, int32_t batch, int32_t h, int32_t w, i
     cudaError_t e = cudaStreamSynchronize(st);
     cudaFree(wp);
     if (rc == 0 && e != cudaSuccess) return fail("conv kernel failed: %s", cudaGetErrorString(e));
+    return rc;
+}
+
+static int device_sm_count() {
+    int dev = 0, nsm = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+    return nsm;
+}
+
+// One conv in any mode build_unet_steps gives it, with the plan's packers and setup_conv.  Every argument is checked
+// before the first CUDA call, so that none of setup_conv's internal refusals can be reached from here.
+extern "C" int vdt_op_conv_ex(const vdt_conv_op* op, void* stream) {
+    if (!op) return fail("null argument");
+    const vdt_conv_op& o = *op;
+    if (!o.a3 || !o.w3 || !o.bias) return fail("a3, w3 and bias are required");
+    if ((o.out_f32 != nullptr) == (o.out16 != nullptr)) return fail("give exactly one of out_f32 and out16");
+    if ((o.a1 != nullptr) != (o.w1 != nullptr)) return fail("a1 and w1 come together");
+    if (!o.a1 && o.a1_lo) return fail("a1_lo without a1");
+    if (o.a1 && (o.a3_lo != nullptr) != (o.a1_lo != nullptr))
+        return fail("split-precision mode packs every weight in three parts: give both a3_lo and a1_lo or neither");
+    if (o.f16 != 0 && o.f16 != 1) return fail("f16 must be 0 or 1 (got %d)", o.f16);
+    if (o.batch < 1 || o.h < 1 || o.w < 1) return fail("empty input (%d x %d x %d)", o.batch, o.h, o.w);
+    if (o.c3 < 64 || o.c3 % 64 || o.cout < 64 || o.cout % 64 || (o.a1 && (o.c1 < 64 || o.c1 % 64)))
+        return fail("channel counts must be positive multiples of 64 (c3 %d, c1 %d, cout %d)", o.c3, o.a1 ? o.c1 : 0, o.cout);
+    if (o.ups != 0 && o.ups != 1) return fail("ups must be 0 or 1 (got %d)", o.ups);
+    if (o.ups && o.a1) return fail("the sub-pixel upsampling conv takes no 1x1 skip operand");
+    if (o.ups && o.residual) return fail("the sub-pixel upsampling conv takes no residual");
+    if (o.resid_mode < 0 || o.resid_mode > 2) return fail("resid_mode must be 0, 1 or 2 (got %d)", o.resid_mode);
+    if (o.resid_mode != 0 && !o.residual) return fail("resid_mode %d needs a residual", o.resid_mode);
+    if (o.resid_mode == 1 && ((o.h | o.w) & 1)) return fail("an upsampled residual needs even output sides (got %dx%d)", o.h, o.w);
+    if (o.resid_mode == 2 && (o.batch & 1)) return fail("a residual shared by image pairs needs an even batch (got %d)", o.batch);
+    ConvGeom geom;
+    CKI(conv_geom(o.batch, o.h, o.w, &geom));
+    const int H = o.ups ? 2 * o.h : o.h, W = o.ups ? 2 * o.w : o.w;
+    if (o.stats) {
+        if (o.stat_cols != 2 && o.stat_cols != 4) return fail("stat_cols must be 2 or 4 (got %d)", o.stat_cols);
+        const int slabs = stat_slabs_per_image(o.h, o.w);
+        if (slabs <= 0 || (o.ups && 4 * slabs != stat_slabs_per_image(H, W)))
+            return fail("no conv-epilogue statistics layout for %dx%d feature maps%s", H, W, o.ups ? " from a sub-pixel conv" : "");
+    }
+    const int split = o.a3_lo ? 1 : 0, km = split ? 3 : 1;
+    const int ktot = o.ups ? 16 * o.c3 * km : (9 * o.c3 + (o.a1 ? o.c1 : 0)) * km;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    h16* wp = nullptr;
+    CK(cudaMalloc(&wp, (size_t)o.cout * ktot * 2));
+    int rc = 0;
+    cudaError_t e = cudaMemset(wp, 0, (size_t)o.cout * ktot * 2);
+    if (e != cudaSuccess) rc = fail("weight buffer: %s", cudaGetErrorString(e));
+    if (rc == 0) rc = o.ups ? pack_conv_ups(o.w3, wp, o.cout, o.c3, o.f16, split)
+                            : pack_conv_skip(o.w3, o.w1, wp, o.cout, o.c3, o.c1, o.f16, split);
+    if (rc == 0 && (e = cudaStreamSynchronize(nullptr)) != cudaSuccess) rc = fail("weight packing failed: %s", cudaGetErrorString(e));
+    if (rc == 0) {
+        ConvSpec s;
+        s.f16 = o.f16; s.stat_cols = o.stat_cols == 2 ? 2 : 4; s.sat_count = reinterpret_cast<unsigned long long*>(o.sat_count);
+        s.a3 = (const h16*)o.a3; s.a3_lo = (const h16*)o.a3_lo; s.c3 = o.c3;
+        if (o.a1) { s.a1 = (const h16*)o.a1; s.a1_lo = (const h16*)o.a1_lo; s.c1 = o.c1; s.ld1 = o.c1; }
+        s.n = o.batch; s.h = o.h; s.w = o.w; s.wpacked = wp; s.cout = o.cout; s.wrows = o.cout; s.ups = o.ups;
+        s.bias = o.bias; s.residual = o.residual; s.resid_up = o.resid_mode == 1; s.resid_rep = o.resid_mode == 2 ? 2 : 0;
+        if (o.out16) { s.out_mode = kOutBF16; s.out_bf16 = (h16*)o.out16; } else { s.out_mode = kOutF32; s.out_f32 = o.out_f32; }
+        s.ld = o.cout; s.stats = (float2*)o.stats;
+        std::unique_ptr<ConvParams> cp(new ConvParams());
+        rc = setup_conv(s, cp.get());
+        if (rc == 0 && o.stats && !cp->stats) rc = fail("internal: statistics dropped for %dx%d feature maps", H, W);
+        if (rc == 0) {
+            e = launch_conv_gemm(*cp, device_sm_count(), st);
+            ++g_launches;
+            if (e != cudaSuccess) rc = fail("conv launch failed: %s", cudaGetErrorString(e));
+        }
+    }
+    e = cudaStreamSynchronize(st);
+    cudaFree(wp);
+    if (rc == 0 && e != cudaSuccess) return fail("conv kernel failed: %s", cudaGetErrorString(e));
+    return rc;
+}
+
+// in_conv as the plan runs it: im2col of the fp32 NCHW input into 64 patch columns (image i reads input image i / rep),
+// then the pointwise GEMM against pack_inconv's weights, with optional GroupNorm statistics.
+extern "C" int vdt_op_in_conv(const float* x_nchw, int32_t batch, int32_t rep, int32_t c, int32_t h, int32_t w, const float* w_oihw,
+                              const float* bias, int32_t hid, float* out_nhwc, void* stats_out, int32_t stat_cols, int32_t f16,
+                              void* stream) {
+    if (!x_nchw || !w_oihw || !bias || !out_nhwc) return fail("null argument");
+    if (batch < 1 || h < 1 || w < 1) return fail("empty input (%d x %d x %d)", batch, h, w);
+    if (rep != 1 && rep != 2) return fail("rep must be 1 or 2 (got %d)", rep);
+    if (c < 1 || 9 * c > 64) return fail("in_conv takes 1 to 7 input channels (got %d)", c);
+    if (hid < 64 || hid % 64) return fail("channel counts must be positive multiples of 64 (hid %d)", hid);
+    if (f16 != 0 && f16 != 1) return fail("f16 must be 0 or 1 (got %d)", f16);
+    if (stats_out) {
+        if (stat_cols != 2 && stat_cols != 4) return fail("stat_cols must be 2 or 4 (got %d)", stat_cols);
+        if (stat_slabs_per_image(h, w) <= 0) return fail("no conv-epilogue statistics layout for %dx%d feature maps", h, w);
+    }
+    const int n = batch * rep;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    h16 *wp = nullptr, *patches = nullptr;
+    CK(cudaMalloc(&wp, (size_t)hid * 64 * 2));
+    int rc = 0;
+    cudaError_t e = cudaMalloc(&patches, (size_t)n * h * w * 64 * 2);
+    if (e != cudaSuccess) rc = fail("patch buffer: %s", cudaGetErrorString(e));
+    if (rc == 0) rc = pack_inconv(w_oihw, wp, hid, c, f16, 0);
+    if (rc == 0 && (e = cudaStreamSynchronize(nullptr)) != cudaSuccess) rc = fail("weight packing failed: %s", cudaGetErrorString(e));
+    if (rc == 0) {
+        e = launch_im2col3x3(x_nchw, patches, nullptr, batch, rep, c, h, w, f16, st);
+        ++g_launches;
+        if (e != cudaSuccess) rc = fail("im2col launch failed: %s", cudaGetErrorString(e));
+    }
+    if (rc == 0) {
+        ConvSpec s;
+        s.f16 = f16; s.stat_cols = stat_cols == 2 ? 2 : 4;
+        s.a1 = patches; s.c1 = 64; s.ld1 = 64; s.n = n; s.h = h; s.w = w; s.wpacked = wp; s.cout = hid; s.wrows = hid;
+        s.bias = bias; s.out_mode = kOutF32; s.out_f32 = out_nhwc; s.ld = hid; s.stats = (float2*)stats_out;
+        std::unique_ptr<ConvParams> cp(new ConvParams());
+        rc = setup_conv(s, cp.get());
+        if (rc == 0 && stats_out && !cp->stats) rc = fail("internal: statistics dropped for %dx%d feature maps", h, w);
+        if (rc == 0) {
+            e = launch_conv_gemm(*cp, device_sm_count(), st);
+            ++g_launches;
+            if (e != cudaSuccess) rc = fail("conv launch failed: %s", cudaGetErrorString(e));
+        }
+    }
+    e = cudaStreamSynchronize(st);
+    cudaFree(patches);
+    cudaFree(wp);
+    if (rc == 0 && e != cudaSuccess) return fail("in_conv kernels failed: %s", cudaGetErrorString(e));
+    return rc;
+}
+
+// out_conv as the plan runs it: the pointwise GEMM Y[pixel, tap * cout + co] over pack_outconv's tap-major rows (zero bias,
+// padded to outconv_rows), then the tap-sum gather + bias into fp32 NCHW.
+extern "C" int vdt_op_out_conv(const void* a_16_nhwc, int32_t batch, int32_t h, int32_t w, int32_t c0, const float* w_oihw,
+                               int32_t cout, const float* bias, float* out_nchw, int32_t f16, void* stream) {
+    if (!a_16_nhwc || !w_oihw || !bias || !out_nchw) return fail("null argument");
+    if (batch < 1 || h < 1 || w < 1) return fail("empty input (%d x %d x %d)", batch, h, w);
+    if (c0 < 64 || c0 % 64) return fail("channel counts must be positive multiples of 64 (c0 %d)", c0);
+    if (cout < 1 || cout > 16) return fail("out_conv takes 1 to 16 output channels (got %d)", cout);
+    if (f16 != 0 && f16 != 1) return fail("f16 must be 0 or 1 (got %d)", f16);
+    const int rows = outconv_rows(cout);
+    const size_t pixels = (size_t)batch * h * w;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    h16* wp = nullptr; float* zero = nullptr; float* ytap = nullptr;
+    CK(cudaMalloc(&wp, (size_t)rows * c0 * 2));
+    int rc = 0;
+    cudaError_t e = cudaMalloc(&zero, (size_t)rows * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&ytap, pixels * rows * 4);
+    if (e == cudaSuccess) e = cudaMemset(wp, 0, (size_t)rows * c0 * 2);
+    if (e == cudaSuccess) e = cudaMemset(zero, 0, (size_t)rows * 4);
+    if (e != cudaSuccess) rc = fail("out_conv buffers: %s", cudaGetErrorString(e));
+    if (rc == 0) rc = pack_outconv(w_oihw, wp, cout, c0, f16, 0);
+    if (rc == 0 && (e = cudaStreamSynchronize(nullptr)) != cudaSuccess) rc = fail("weight packing failed: %s", cudaGetErrorString(e));
+    if (rc == 0) {
+        ConvSpec s;
+        s.f16 = f16;
+        s.a1 = (const h16*)a_16_nhwc; s.c1 = c0; s.ld1 = c0; s.n = batch; s.h = h; s.w = w; s.wpacked = wp;
+        s.cout = rows; s.wrows = rows; s.bias = zero; s.out_mode = kOutF32; s.out_f32 = ytap; s.ld = rows;
+        std::unique_ptr<ConvParams> cp(new ConvParams());
+        rc = setup_conv(s, cp.get());
+        if (rc == 0) {
+            e = launch_conv_gemm(*cp, device_sm_count(), st);
+            ++g_launches;
+            if (e != cudaSuccess) rc = fail("conv launch failed: %s", cudaGetErrorString(e));
+        }
+    }
+    if (rc == 0) {
+        e = launch_tapsum3x3(ytap, bias, out_nchw, batch, h, w, cout, rows, st);
+        ++g_launches;
+        if (e != cudaSuccess) rc = fail("tapsum launch failed: %s", cudaGetErrorString(e));
+    }
+    e = cudaStreamSynchronize(st);
+    cudaFree(ytap);
+    cudaFree(zero);
+    cudaFree(wp);
+    if (rc == 0 && e != cudaSuccess) return fail("out_conv kernels failed: %s", cudaGetErrorString(e));
     return rc;
 }
 
