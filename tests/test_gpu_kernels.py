@@ -581,16 +581,3 @@ def test_attn_block_backward_composed_from_kernels(L, f16):
     print(f"AttentionBlock fwd+bwd {Cc}ch N={N} B={B} {'fp16' if f16 else 'bf16'}: " + ", ".join(f"{k} {v:.1e}" for k, v in errs.items()))
     assert max(errs.values()) <= 8e-3 * EPS[f16], errs          # measured: 7.7e-4 (fp16), 5.8e-3 (bf16)
 
-
-def test_attention_cta_pair_variant_matches():
-    """The opt-in cta_group::2 attention variant (VDT_ATTN_PAIR=1; measured slower, kept selectable) computes the same thing:
-    run the attention parity cases that qualify (even number of query tiles, d % 128 == 0) in a child process with it on."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, VDT_ATTN_PAIR="1", PYTHONPATH=root + os.pathsep + os.environ.get("PYTHONPATH", ""))
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_gpu_kernels.py"), "-q", "-m", "gpu", "-k",
-                        "test_attention and (1024 or 256 or 4096) and not pair"], cwd=root, env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-500:]
-    assert "passed" in r.stdout

@@ -17,21 +17,13 @@
 // as the current item's last S = Q K^T has retired, and its first two S tiles are issued while the
 // softmax warps are still finishing the current item (per-CTA set-up used to cost ~10 us per 128 rows).
 //
-// TWO = true (opt-in, VDT_ATTN_PAIR=1; even number of query tiles per image, d a multiple of 128): CTAs are paired in clusters of two and the
-// tensor cores run in cta_group::2 mode.  The pair owns two query tiles of the same image and head; every 64-key K tile
-// and V tile is fetched ONCE per pair, half by each CTA (K: 32 of the 64 keys, the N halves of S = Q K^T; V: 128 of the d
-// feature columns, the N halves of O += P V), so a ring stage costs half the shared memory -- four stages instead of two in
-// the same 64 + 64 KB -- and the L2 -> smem traffic per query tile halves.  The leader CTA issues every MMA; TMA completions
-// of both CTAs land on the leader's barriers, tcgen05.commit multicasts the consumer-side barriers to both CTAs.
-//
 //   warp 0     TMA producer for Q (per item) and the 64-key K tiles (ring slot freed when S retires)
 //   warp 10    TMA producer for the V tiles (ring slot freed when O += P V retires)
-//   warp 1     MMA issuer (leader CTA only when TWO)
+//   warp 1     MMA issuer
 //   warps 2-9  softmax + final normalise/store: two threads per query row (= TMEM lane), each owning 32
 //              of the tile's 64 key columns (and half of O's columns); row maxima are exchanged through
 //              shared memory once per tile between the two warps that share a TMEM lane quarter
 #include <atomic>
-#include <cstdlib>
 
 #include "kernels.cuh"
 #include "ptx.cuh"
@@ -44,11 +36,11 @@ constexpr int kKeys = 64;                      // keys per tile = one 128-byte s
 constexpr int kThreads = 64 + 256 + 32;
 constexpr float kRescaleThreshold = 8.0f;      // log2 units
 
-constexpr int kMaxStages = 4;
+constexpr int kStages = 2;                     // K / V ring stages
 struct Smem {          // stage pointers are computed, not indexed (no local-memory arrays)
     uint8_t* q; uint8_t* k0; uint8_t* v0; uint8_t* p0;
     int kv_stride;
-    uint64_t *q_full, *q_empty, *k_full, *v_full, *k_empty, *v_empty, *s_full, *p_full, *o_empty;   // k_/v_ arrays: [kMaxStages]
+    uint64_t *q_full, *q_empty, *k_full, *v_full, *k_empty, *v_empty, *s_full, *p_full, *o_empty;   // k_/v_ arrays: [kStages]
     uint32_t* tmem_slot;
     __device__ __forceinline__ uint8_t* k(int s) const { return k0 + s * kv_stride; }
     __device__ __forceinline__ uint8_t* v(int s) const { return v0 + s * kv_stride; }
@@ -57,7 +49,7 @@ struct Smem {          // stage pointers are computed, not indexed (no local-mem
 
 __host__ __device__ inline int attn_smem_bytes(int d) {
     // Q d/64 x 16K | K ring d/64 x 16K | V ring d/64 x 16K | P 2 x 16K | barriers | row max / sum exchange
-    // (ring = 2 stages of d/64 x 8K, or 4 stages of half that in the CTA-pair variant)
+    // (ring = 2 stages of d/64 x 8K)
     return (d / 64) * 16384 + 4 * (d / 64) * 8192 + 2 * 16384 + 256 + 2048;
 }
 
@@ -70,25 +62,22 @@ __device__ __forceinline__ Item decode_item(int w, int qtiles, int heads, int ip
     return it;
 }
 
-template <bool F16, bool TWO>
-__device__ __forceinline__ void attention_body(const AttnParams& p) {
+template <bool F16>
+__global__ void __launch_bounds__(kThreads, 1) attention_kernel(const __grid_constant__ AttnParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];   // 128B-swizzled tiles need 1024-byte alignment
     uint8_t* base = smem_raw;
     if ((smem_u32(base) & 1023u) != 0) __trap();
     const int d = p.d, dch = d / 64;
     Smem sm;
-    constexpr int S = TWO ? 4 : 2;                           // K / V ring stages
     sm.q = base; base += dch * 16384;
-    sm.kv_stride = dch * (TWO ? 4096 : 8192);               // a CTA of a pair holds half of every K / V tile
+    sm.kv_stride = dch * 8192;
     sm.k0 = base; base += 2 * dch * 8192;
     sm.v0 = base; base += 2 * dch * 8192;
     sm.p0 = base; base += 2 * 16384;
     uint64_t* bars = reinterpret_cast<uint64_t*>(base);
-    sm.q_full = bars; sm.q_empty = bars + 1; sm.k_full = bars + 2; sm.v_full = sm.k_full + kMaxStages; sm.k_empty = sm.v_full + kMaxStages;
-    sm.v_empty = sm.k_empty + kMaxStages; sm.s_full = sm.v_empty + kMaxStages; sm.p_full = sm.s_full + 2; sm.o_empty = sm.p_full + 2;
+    sm.q_full = bars; sm.q_empty = bars + 1; sm.k_full = bars + 2; sm.v_full = sm.k_full + kStages; sm.k_empty = sm.v_full + kStages;
+    sm.v_empty = sm.k_empty + kStages; sm.s_full = sm.v_empty + kStages; sm.p_full = sm.s_full + 2; sm.o_empty = sm.p_full + 2;
     sm.tmem_slot = reinterpret_cast<uint32_t*>(sm.o_empty + 1);
-    const int rank = TWO ? static_cast<int>(cluster_ctarank()) : 0;
-    constexpr int NC = TWO ? 2 : 1;                          // CTAs that arrive on the leader-side barriers
     float* xch = reinterpret_cast<float*>(base + 256);      // [2][2][128]: double-buffered row-max exchange; reused for l
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -101,31 +90,27 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
     const int qtiles = packed ? 1 : (N + kQRows - 1) / kQRows;
     const int nt = packed ? 2 : (N + kKeys - 1) / kKeys;    // key tiles per item
     const int groups = (p.B + ipc - 1) / ipc;
-    // an item of a CTA pair is two adjacent query tiles; cta / ncta = this CTA's (pair's) index among the resident ones
-    const int qsteps = TWO ? qtiles / 2 : qtiles;
-    const int total_items = groups * p.heads * qsteps;
-    const int cta = TWO ? (blockIdx.x >> 1) : blockIdx.x, ncta = TWO ? (gridDim.x >> 1) : gridDim.x;
+    const int total_items = groups * p.heads * qtiles;
+    const int cta = blockIdx.x, ncta = gridDim.x;           // persistent: this CTA takes items cta, cta + ncta, ...
     uint32_t tmem_cols = 128; while (tmem_cols < static_cast<uint32_t>(d + 2 * kKeys)) tmem_cols <<= 1;
 
     if (threadIdx.x == 0) {
-        // q_full / k_full / v_full / p_full / o_empty are only used in the leader CTA of a pair; the others in both
-        mbar_init(sm.q_full, 1); mbar_init(sm.q_empty, 1); mbar_init(sm.o_empty, 8 * NC);
-        for (int s = 0; s < S; ++s) { mbar_init(&sm.k_full[s], 1); mbar_init(&sm.v_full[s], 1); mbar_init(&sm.k_empty[s], 1);
-                                      mbar_init(&sm.v_empty[s], 1); }
-        for (int s = 0; s < 2; ++s) { mbar_init(&sm.p_full[s], 8 * NC); mbar_init(&sm.s_full[s], 1); }
+        mbar_init(sm.q_full, 1); mbar_init(sm.q_empty, 1); mbar_init(sm.o_empty, 8);
+        for (int s = 0; s < kStages; ++s) { mbar_init(&sm.k_full[s], 1); mbar_init(&sm.v_full[s], 1); mbar_init(&sm.k_empty[s], 1);
+                                            mbar_init(&sm.v_empty[s], 1); }
+        for (int s = 0; s < 2; ++s) { mbar_init(&sm.p_full[s], 8); mbar_init(&sm.s_full[s], 1); }
         fence_mbar_init();
-        tma_prefetch_desc(&p.q_map); tma_prefetch_desc(&p.kv_map); tma_prefetch_desc(&p.k2_map);
+        tma_prefetch_desc(&p.q_map); tma_prefetch_desc(&p.kv_map);
     }
-    if (warp == 1) { if (TWO) tmem_alloc_2cta(sm.tmem_slot, tmem_cols); else tmem_alloc(sm.tmem_slot, tmem_cols); }
+    if (warp == 1) tmem_alloc(sm.tmem_slot, tmem_cols);
     tc_fence_before();
     __syncthreads();
-    if (TWO) cluster_sync_all();                            // the peer's barriers are initialised before anything signals them
     tc_fence_after();
     const uint32_t tmem_base = *sm.tmem_slot;
     const uint32_t tmem_o = tmem_base;                      // columns [0, d)
     const uint32_t tmem_s = tmem_base + static_cast<uint32_t>(d);   // two S buffers: columns [d, d+64) and [d+64, d+128)
 
-    // g = running key-tile counter of this CTA across its items: ring slot g % S, barrier parity (g / S) & 1
+    // g = running key-tile counter of this CTA across its items: ring slot g % kStages, barrier parity (g / kStages) & 1
     // (the S / P buffers are double-buffered: slot g & 1, parity (g >> 1) & 1)
     if (warp == 0) {
         // ------------------------------------------------------------------ Q + K producer
@@ -133,32 +118,24 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
         {
             int g = 0, it_n = 0;
             for (int w = cta; w < total_items; w += ncta, ++it_n) {
-                const Item it = decode_item(w, qsteps, p.heads, ipc);
-                const int qt = TWO ? 2 * it.qt + rank : it.qt;
-                const long long row0 = static_cast<long long>(it.b0) * N + static_cast<long long>(qt) * kQRows;
+                const Item it = decode_item(w, qtiles, p.heads, ipc);
+                const long long row0 = static_cast<long long>(it.b0) * N + static_cast<long long>(it.qt) * kQRows;
                 const long long krow0 = static_cast<long long>(it.b0) * N;
                 mbar_wait(sm.q_empty, (it_n & 1) ^ 1);      // the previous item's last S = Q K^T has retired
                 if (elect_one()) {
-                    if (rank == 0) mbar_expect_tx(sm.q_full, static_cast<uint32_t>(NC * dch * 16384));
-                    for (int c = 0; c < dch; ++c) {
-                        if (TWO) tma_load_2d_2cta(sm.q + c * 16384, &p.q_map, sm.q_full, it.h * d + c * 64, static_cast<int>(row0));
-                        else tma_load_2d(sm.q + c * 16384, &p.q_map, sm.q_full, it.h * d + c * 64, static_cast<int>(row0));
-                    }
+                    mbar_expect_tx(sm.q_full, static_cast<uint32_t>(dch * 16384));
+                    for (int c = 0; c < dch; ++c)
+                        tma_load_2d(sm.q + c * 16384, &p.q_map, sm.q_full, it.h * d + c * 64, static_cast<int>(row0));
                 }
                 __syncwarp();
                 for (int j = 0; j < nt; ++j, ++g) {
-                    const int s = g % S;
-                    mbar_wait(&sm.k_empty[s], ((g / S) & 1) ^ 1);
+                    const int s = g % kStages;
+                    mbar_wait(&sm.k_empty[s], ((g / kStages) & 1) ^ 1);
                     if (elect_one()) {
-                        if (rank == 0) mbar_expect_tx(&sm.k_full[s], static_cast<uint32_t>(dch * 8192));
-                        for (int c = 0; c < dch; ++c) {
-                            if (TWO)                        // this CTA's 32 of the tile's 64 keys (its N half of S)
-                                tma_load_2d_2cta(sm.k(s) + c * 4096, &p.k2_map, &sm.k_full[s], p.hid + it.h * d + c * 64,
-                                                 static_cast<int>(krow0) + j * kKeys + rank * 32);
-                            else
-                                tma_load_2d(sm.k(s) + c * 8192, &p.kv_map, &sm.k_full[s], p.hid + it.h * d + c * 64,
-                                            static_cast<int>(krow0) + j * kKeys);
-                        }
+                        mbar_expect_tx(&sm.k_full[s], static_cast<uint32_t>(dch * 8192));
+                        for (int c = 0; c < dch; ++c)
+                            tma_load_2d(sm.k(s) + c * 8192, &p.kv_map, &sm.k_full[s], p.hid + it.h * d + c * 64,
+                                        static_cast<int>(krow0) + j * kKeys);
                     }
                     __syncwarp();
                 }
@@ -168,19 +145,17 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
         // ------------------------------------------------------------------ V producer
         {
             int g = 0;
-            const int vch = TWO ? dch / 2 : dch;            // 64-feature chunks this CTA holds: its N half of O += P V
             for (int w = cta; w < total_items; w += ncta) {
-                const Item it = decode_item(w, qsteps, p.heads, ipc);
+                const Item it = decode_item(w, qtiles, p.heads, ipc);
                 const long long krow0 = static_cast<long long>(it.b0) * N;
                 for (int j = 0; j < nt; ++j, ++g) {
-                    const int s = g % S;
-                    mbar_wait(&sm.v_empty[s], ((g / S) & 1) ^ 1);
+                    const int s = g % kStages;
+                    mbar_wait(&sm.v_empty[s], ((g / kStages) & 1) ^ 1);
                     if (elect_one()) {
-                        if (rank == 0) mbar_expect_tx(&sm.v_full[s], static_cast<uint32_t>(dch * 8192));
-                        for (int c = 0; c < vch; ++c) {    // chunk c: 64 keys x 64 features, one 128-byte row per key
-                            const int col = 2 * p.hid + it.h * d + (rank * vch + c) * 64;
-                            if (TWO) tma_load_2d_2cta(sm.v(s) + c * 8192, &p.kv_map, &sm.v_full[s], col, static_cast<int>(krow0) + j * kKeys);
-                            else tma_load_2d(sm.v(s) + c * 8192, &p.kv_map, &sm.v_full[s], col, static_cast<int>(krow0) + j * kKeys);
+                        mbar_expect_tx(&sm.v_full[s], static_cast<uint32_t>(dch * 8192));
+                        for (int c = 0; c < dch; ++c) {    // chunk c: 64 keys x 64 features, one 128-byte row per key
+                            const int col = 2 * p.hid + it.h * d + c * 64;
+                            tma_load_2d(sm.v(s) + c * 8192, &p.kv_map, &sm.v_full[s], col, static_cast<int>(krow0) + j * kKeys);
                         }
                     }
                     __syncwarp();
@@ -188,62 +163,59 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
             }
         }
     } else if (warp == 1) {
-        // ------------------------------------------------------------------ MMA issuer (the pair's leader when TWO)
+        // ------------------------------------------------------------------ MMA issuer
         // The whole warp walks the loop (warp-uniform control flow and operands); one elected lane issues each instruction.
-        if (rank == 0) {
-            const uint32_t idesc_s = umma_idesc_16(NC * kQRows, kKeys, (F16 ? 1 : 0));
-            const uint32_t idesc_o = umma_idesc_16(NC * kQRows, d, (F16 ? 1 : 0)) | kIdescBMajorMN;
-            const uint32_t v_lbo = 8192u;                   // next 64-feature chunk of a V stage
-            const int k_chunk = TWO ? 4096 : 8192;          // bytes of one 64-feature chunk of a K stage
-            auto mma = [&](uint32_t dt, uint64_t ad, uint64_t bd, uint32_t idesc, uint32_t acc) {
-                if (elect_one()) { if (TWO) umma_16_2cta(dt, ad, bd, idesc, acc); else umma_16(dt, ad, bd, idesc, acc); }
-            };
-            auto commit = [&](uint64_t* bar) {
-                if (elect_one()) { if (TWO) umma_commit_2cta(bar, static_cast<uint16_t>(3)); else umma_commit(bar); }
-            };
-            const uint64_t q_desc = umma_desc_sw128(smem_u32(sm.q));
-            int g = 0, it_n = 0;
-            for (int w = cta; w < total_items; w += ncta, ++it_n) {
-                auto issue_s = [&](int j) {                 // tile j of this item = running tile g + j
-                    const int gj = g + j, s = gj % S, sb = gj & 1;
-                    mbar_wait(&sm.k_full[s], (gj / S) & 1);
-                    tc_fence_after();
-                    const uint64_t k_desc = umma_desc_sw128(smem_u32(sm.k(s)));
-                    const uint32_t dst = tmem_s + static_cast<uint32_t>(sb * kKeys);
-                    for (int c = 0; c < dch; ++c) {         // 64-feature chunk c: 16 KB of Q, k_chunk bytes of K (descriptor units of 16 B)
-                        const uint64_t ad = q_desc + static_cast<uint64_t>(c * (16384 >> 4));
-                        const uint64_t bd = k_desc + static_cast<uint64_t>(c * (k_chunk >> 4));
+        const uint32_t idesc_s = umma_idesc_16(kQRows, kKeys, (F16 ? 1 : 0));
+        const uint32_t idesc_o = umma_idesc_16(kQRows, d, (F16 ? 1 : 0)) | kIdescBMajorMN;
+        const uint32_t v_lbo = 8192u;                       // next 64-feature chunk of a V stage
+        auto mma = [&](uint32_t dt, uint64_t ad, uint64_t bd, uint32_t idesc, uint32_t acc) {
+            if (elect_one()) umma_16(dt, ad, bd, idesc, acc);
+        };
+        auto commit = [&](uint64_t* bar) {
+            if (elect_one()) umma_commit(bar);
+        };
+        const uint64_t q_desc = umma_desc_sw128(smem_u32(sm.q));
+        int g = 0, it_n = 0;
+        for (int w = cta; w < total_items; w += ncta, ++it_n) {
+            auto issue_s = [&](int j) {                     // tile j of this item = running tile g + j
+                const int gj = g + j, s = gj % kStages, sb = gj & 1;
+                mbar_wait(&sm.k_full[s], (gj / kStages) & 1);
+                tc_fence_after();
+                const uint64_t k_desc = umma_desc_sw128(smem_u32(sm.k(s)));
+                const uint32_t dst = tmem_s + static_cast<uint32_t>(sb * kKeys);
+                for (int c = 0; c < dch; ++c) {             // 64-feature chunk c: 16 KB of Q, 8 KB of K (descriptor units of 16 B)
+                    const uint64_t ad = q_desc + static_cast<uint64_t>(c * (16384 >> 4));
+                    const uint64_t bd = k_desc + static_cast<uint64_t>(c * (8192 >> 4));
 #pragma unroll
-                        for (int k4 = 0; k4 < 4; ++k4) mma(dst, ad + 2 * k4, bd + 2 * k4, idesc_s, (c | k4) != 0);
-                    }
-                    commit(&sm.k_empty[s]);               // K_j can be overwritten as soon as S_j has retired
-                    commit(&sm.s_full[sb]);
-                    if (j == nt - 1) commit(sm.q_empty);    // ... and so can Q after the item's last S
-                };
-                mbar_wait(sm.q_full, it_n & 1);
-                // the S buffers are free: every softmax tile of the previous item was waited for below (p_full)
-                issue_s(0);
-                if (nt > 1) issue_s(1);                   // S is double-buffered: S_{j+1} is ready before softmax j ends
-                for (int j = 0; j < nt; ++j) {
-                    const int gj = g + j, s = gj % S, sb = gj & 1;
-                    mbar_wait(&sm.p_full[sb], (gj >> 1) & 1);   // P_j in smem, S_j consumed (its buffer is free), O rescaled if needed
-                    tc_fence_after();
-                    if (j + 2 < nt) issue_s(j + 2);
-                    if (j == 0 && it_n > 0) {               // O still holds the previous item until its rows have been read out
-                        mbar_wait(sm.o_empty, (it_n - 1) & 1);
-                        tc_fence_after();
-                    }
-                    mbar_wait(&sm.v_full[s], (gj / S) & 1);
-                    tc_fence_after();
-                    const uint64_t p_desc = umma_desc_sw128(smem_u32(sm.p(sb)));
-                    const uint64_t v_desc = umma_desc_sw128_mn(smem_u32(sm.v(s)), v_lbo);
-#pragma unroll
-                    for (int kk = 0; kk < kKeys / 16; ++kk)     // 16 keys: +32 bytes in a P row, +2048 bytes (16 rows) in V
-                        mma(tmem_o, p_desc + 2 * kk, v_desc + static_cast<uint64_t>(kk * (2048 >> 4)), idesc_o, (j | kk) != 0);
-                    commit(&sm.v_empty[s]);               // V_j / P_j free, O updated
+                    for (int k4 = 0; k4 < 4; ++k4) mma(dst, ad + 2 * k4, bd + 2 * k4, idesc_s, (c | k4) != 0);
                 }
-                g += nt;
+                commit(&sm.k_empty[s]);                   // K_j can be overwritten as soon as S_j has retired
+                commit(&sm.s_full[sb]);
+                if (j == nt - 1) commit(sm.q_empty);        // ... and so can Q after the item's last S
+            };
+            mbar_wait(sm.q_full, it_n & 1);
+            // the S buffers are free: every softmax tile of the previous item was waited for below (p_full)
+            issue_s(0);
+            if (nt > 1) issue_s(1);                       // S is double-buffered: S_{j+1} is ready before softmax j ends
+            for (int j = 0; j < nt; ++j) {
+                const int gj = g + j, s = gj % kStages, sb = gj & 1;
+                mbar_wait(&sm.p_full[sb], (gj >> 1) & 1);   // P_j in smem, S_j consumed (its buffer is free), O rescaled if needed
+                tc_fence_after();
+                if (j + 2 < nt) issue_s(j + 2);
+                if (j == 0 && it_n > 0) {                   // O still holds the previous item until its rows have been read out
+                    mbar_wait(sm.o_empty, (it_n - 1) & 1);
+                    tc_fence_after();
+                }
+                mbar_wait(&sm.v_full[s], (gj / kStages) & 1);
+                tc_fence_after();
+                const uint64_t p_desc = umma_desc_sw128(smem_u32(sm.p(sb)));
+                const uint64_t v_desc = umma_desc_sw128_mn(smem_u32(sm.v(s)), v_lbo);
+#pragma unroll
+                for (int kk = 0; kk < kKeys / 16; ++kk)         // 16 keys: +32 bytes in a P row, +2048 bytes (16 rows) in V
+                    mma(tmem_o, p_desc + 2 * kk, v_desc + static_cast<uint64_t>(kk * (2048 >> 4)), idesc_o, (j | kk) != 0);
+                commit(&sm.v_empty[s]);                   // V_j / P_j free, O updated
             }
+            g += nt;
         }
     } else if (warp < 10) {
         // ------------------------------------------------------------------ softmax + output
@@ -257,10 +229,9 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
         const int row_img = row / N;                        // only meaningful when packed
         int g = 0, it_n = 0;
         for (int w = cta; w < total_items; w += ncta, ++it_n) {
-            const Item it = decode_item(w, qsteps, p.heads, ipc);
-            const int qt = TWO ? 2 * it.qt + rank : it.qt;
-            const long long grow = static_cast<long long>(it.b0) * N + static_cast<long long>(qt) * kQRows + row;
-            const bool row_ok = (grow < static_cast<long long>(p.B) * N) && (packed || qt * kQRows + row < N);
+            const Item it = decode_item(w, qtiles, p.heads, ipc);
+            const long long grow = static_cast<long long>(it.b0) * N + static_cast<long long>(it.qt) * kQRows + row;
+            const bool row_ok = (grow < static_cast<long long>(p.B) * N) && (packed || it.qt * kQRows + row < N);
             float m_used = -INFINITY, l = 0.f;
             for (int j = 0; j < nt; ++j) {
                 const int gj = g + j, sb = gj & 1;
@@ -302,7 +273,7 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
                 }
                 if (__any_sync(0xffffffffu, need)) {
                     // O must be complete through PV_{j-1} before it is rescaled (need implies j >= 1)
-                    mbar_wait(&sm.v_empty[(gj - 1) % S], ((gj - 1) / S) & 1);
+                    mbar_wait(&sm.v_empty[(gj - 1) % kStages], ((gj - 1) / kStages) & 1);
                     tc_fence_after();
                     for (int c0 = half * dh; c0 < half * dh + dh; c0 += 32) {
                         uint32_t o[32];
@@ -331,7 +302,7 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
                 l += lsum;
                 // P_j goes into the buffer PV_{g-2} read (possibly the previous item's): S_j was issued before that
                 // MMA, so s_full alone does not order these stores after its operand reads
-                if (gj >= 2) mbar_wait(&sm.v_empty[(gj - 2) % S], ((gj - 2) / S) & 1);
+                if (gj >= 2) mbar_wait(&sm.v_empty[(gj - 2) % kStages], ((gj - 2) / kStages) & 1);
                 uint8_t* prow = sm.p(sb) + row * 128;
 #pragma unroll
                 for (int ch = 0; ch < 4; ++ch)
@@ -340,7 +311,7 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
                 fence_proxy_async_smem();
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) { if (TWO) mbar_arrive_cluster(&sm.p_full[sb], 0); else mbar_arrive(&sm.p_full[sb]); }
+                if (lane == 0) mbar_arrive(&sm.p_full[sb]);
             }
             // ---- final: O / l -> 16-bit.  The two threads of a row add their partial sums.  (The first barrier keeps a
             // fast thread from overwriting a row maximum of the last tile that its partner has not read yet.)
@@ -349,7 +320,7 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
             asm volatile("bar.sync %0, 64;" ::"r"(bar_id) : "memory");
             l += xch[(half ^ 1) * 128 + row];
             const int g_last = g + nt - 1;
-            mbar_wait(&sm.v_empty[g_last % S], (g_last / S) & 1);
+            mbar_wait(&sm.v_empty[g_last % kStages], (g_last / kStages) & 1);
             tc_fence_after();
             const float inv_l = (l > 0.f) ? 1.f / l : 0.f;
             for (int c0 = half * dh; c0 < half * dh + dh; c0 += 32) {
@@ -359,7 +330,7 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
                 if (c0 + 32 >= half * dh + dh) {            // this warp's last read of O: the next item may overwrite it
                     tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) { if (TWO) mbar_arrive_cluster_relaxed(sm.o_empty, 0); else mbar_arrive(sm.o_empty); }
+                    if (lane == 0) mbar_arrive(sm.o_empty);
                 }
                 if (row_ok) {
                     uint4* dst = reinterpret_cast<uint4*>(p.out + grow * p.hid + it.h * d + c0);
@@ -380,20 +351,10 @@ __device__ __forceinline__ void attention_body(const AttnParams& p) {
 
     tc_fence_before();
     __syncthreads();
-    if (TWO) cluster_sync_all();                            // no CTA exits while its peer may still signal it
     if (warp == 1) {
         tc_fence_after();
-        if (TWO) tmem_dealloc_2cta(tmem_base, tmem_cols); else tmem_dealloc(tmem_base, tmem_cols);
+        tmem_dealloc(tmem_base, tmem_cols);
     }
-}
-
-template <bool F16>
-__global__ void __launch_bounds__(kThreads, 1) attention_kernel(const __grid_constant__ AttnParams p) {
-    attention_body<F16, false>(p);
-}
-template <bool F16>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) attention_pair_kernel(const __grid_constant__ AttnParams p) {
-    attention_body<F16, true>(p);
 }
 
 }  // namespace
@@ -410,8 +371,6 @@ cudaError_t launch_attention(const AttnParams& p, int num_sms, cudaStream_t stre
     if (smem > smem_set[dev].load(std::memory_order_acquire)) {
         e = cudaFuncSetAttribute(attention_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return e;
         smem_set[dev].store(smem, std::memory_order_release);
     }
@@ -419,24 +378,10 @@ cudaError_t launch_attention(const AttnParams& p, int num_sms, cudaStream_t stre
     const int ipc = packed ? 2 : 1;
     const int qtiles = packed ? 1 : (p.N + kQRows - 1) / kQRows;
     const int groups = (p.B + ipc - 1) / ipc;
-    // CTA pairs (cta_group::2; needs an even number of query tiles per image and whole 64-feature chunks in each CTA's half
-    // of V) are OFF by default: measured slower than the single-CTA kernel (N = 1024: 1.71 vs 1.19 ms per 1024 images,
-    // N = 256: 0.175 vs 0.139 ms; profiles/r2i_attention_ab.txt) -- the limiter is the softmax warps' latency chain, not the
-    // K / V ring depth or the L2 -> smem traffic the pairing halves.  VDT_ATTN_PAIR=1 selects it (covered by the kernel test).
-    static int pair_ok = -1;
-    if (pair_ok < 0) { const char* ev = getenv("VDT_ATTN_PAIR"); pair_ok = (ev && ev[0] == '1') ? 1 : 0; }
-    const bool two = pair_ok && !packed && qtiles % 2 == 0 && p.d % 128 == 0;
-    const long long items = static_cast<long long>(groups) * p.heads * (two ? qtiles / 2 : qtiles);
+    const long long items = static_cast<long long>(groups) * p.heads * qtiles;
     if (items <= 0) return cudaSuccess;
-    // persistent: one CTA (or CTA pair) per SM (pair of SMs): the tiles of a 256-wide head fill the SM's shared memory;
-    // the register file holds one CTA of this kernel either way
-    if (two) {
-        long long pairs = num_sms / 2;
-        if (pairs > items) pairs = items;
-        if (p.f16) attention_pair_kernel<true><<<static_cast<unsigned>(2 * pairs), kThreads, smem, stream>>>(p);
-        else attention_pair_kernel<false><<<static_cast<unsigned>(2 * pairs), kThreads, smem, stream>>>(p);
-        return cudaGetLastError();
-    }
+    // persistent: one CTA per SM: the tiles of a 256-wide head fill the SM's shared memory; the register file holds one
+    // CTA of this kernel either way
     long long grid = num_sms;
     if (grid > items) grid = items;
     if (p.f16) attention_kernel<true><<<static_cast<unsigned>(grid), kThreads, smem, stream>>>(p);

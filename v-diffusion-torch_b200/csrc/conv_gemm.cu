@@ -285,18 +285,6 @@ conv_gemm_kernel(const __grid_constant__ ConvParams p) {
                 const WorkItem it = decode_item(p, w, rank);
                 const int n_tile = it.n_tile, py = it.par >> 1, px = it.par & 1;
                 const TileCoord o = tile_origin(p, it.m_tile);
-                if (p.prefetch_next && w + num_pairs_resident < total_items) {
-                    // (opt-in experiment, rejected: -3 % images/s) the next item's own rows (centre tap) into L2 a whole tile
-                    // ahead of the ring's ~2 us; the extra DRAM reads cost more than the first-touch latency they hide
-                    const WorkItem nx = decode_item(p, w + num_pairs_resident, rank);
-                    if (nx.par == 0 && nx.n_tile == 0 && nx.m_tile < p.num_m_tiles) {
-                        const TileCoord no = tile_origin(p, nx.m_tile);
-                        if (elect_one())
-                            for (int s = 0; s < p.num_segs; ++s)
-                                for (int kb = 0; kb < p.seg_kblocks[s]; ++kb) tma_prefetch_4d(&p.a_map[s], kb * kBK, no.c1, no.c2, no.c3);
-                        __syncwarp();
-                    }
-                }
                 int kcol = it.par * kblocks_total * kBK;   // sub-pixel conv: every parity class has its own weight columns
                 for (int s = 0; s < p.num_segs; ++s) {
                     const int taps = p.seg_taps[s];

@@ -14,9 +14,6 @@
 // group and every PPH-th pixel; private fp32 partials combined once through shared memory).
 // Optionally also writes the raw concat in 16 bits (operand of the 1x1 skip conv) and the resampled
 // raw input in fp32 (identity-skip residual of a resampling block).
-#include <atomic>
-#include <cstdlib>
-
 #include "kernels.cuh"
 #include "ptx.cuh"
 
@@ -419,39 +416,7 @@ __global__ void __launch_bounds__(1024, 1) groupnorm_kernel(const GroupNormParam
 
 }  // namespace
 
-// The SM's L1 / shared-memory split is configured per kernel, and two kernels only share an SM when they agree on it.  The
-// conv and attention kernels need (almost) all of it as shared memory; asking for the same carve-out here (VDT_GN_CARVEOUT=1)
-// lets GroupNorm CTAs of one lane run next to a resident conv CTA of the other lane (plan.cu: vdt_plan::lanes).  Measured on
-// one box (profiles/r2h_lanes_carveout_ab.txt): the kernel itself loses 12 % without its L1 (83.4 -> 93.5 ms per step),
-// which the overlap (+1.6 %) does not pay back, so the default keeps the driver's split.
-template <typename K>
-static cudaError_t prefer_smem_carveout(K kernel) {
-    return cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-}
-static cudaError_t configure_groupnorm_kernels() {
-    static std::atomic<bool> done[kMaxDevices];
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return e;
-    if (dev < 0 || dev >= kMaxDevices) return cudaErrorInvalidDevice;
-    if (done[dev].load(std::memory_order_acquire)) return cudaSuccess;
-    const char* on = getenv("VDT_GN_CARVEOUT");              // default: leave the driver's split
-    if (!(on && on[0] == '1')) { done[dev].store(true, std::memory_order_release); return cudaSuccess; }
-#define VDT_GN_CFG(V, FU, I16, F) if (e == cudaSuccess) e = prefer_smem_carveout(groupnorm_kernel<V, FU, I16, F>)
-    VDT_GN_CFG(4, true, true, true);   VDT_GN_CFG(4, true, true, false);  VDT_GN_CFG(4, true, false, true);  VDT_GN_CFG(4, true, false, false);
-    VDT_GN_CFG(2, true, true, true);   VDT_GN_CFG(2, true, true, false);  VDT_GN_CFG(2, true, false, true);  VDT_GN_CFG(2, true, false, false);
-    VDT_GN_CFG(4, false, false, true); VDT_GN_CFG(4, false, false, false); VDT_GN_CFG(2, false, false, true); VDT_GN_CFG(2, false, false, false);
-#undef VDT_GN_CFG
-    if (e == cudaSuccess) e = prefer_smem_carveout(groupnorm_finalize_kernel);
-    if (e == cudaSuccess) done[dev].store(true, std::memory_order_release);
-    return e;
-}
-
 cudaError_t launch_groupnorm(const GroupNormParams& p, cudaStream_t stream) {
-    {
-        const cudaError_t ce = configure_groupnorm_kernels();
-        if (ce != cudaSuccess) return ce;
-    }
     const int C = p.C1 + p.C2;
     if (C % kGroups != 0 || p.B <= 0) return cudaErrorInvalidValue;
     const int cpg = C / kGroups;
@@ -465,14 +430,9 @@ cudaError_t launch_groupnorm(const GroupNormParams& p, cudaStream_t stream) {
                   p.C1 % p.stat_cols != 0 || (p.C2 > 0 && p.stats2 == nullptr))) return cudaErrorInvalidValue;
     if (p.in16 && (p.C2 != 0 || !fused)) return cudaErrorInvalidValue;
     if (p.drop_p > 0.f && (p.resample != kResNone || p.drop_seed == nullptr || p.drop_p >= 1.f)) return cudaErrorInvalidValue;
-    // threads per CTA: 256 by default (16 K registers, ~1 KB of shared memory), so that a GroupNorm CTA fits on an SM next
-    // to a resident conv / attention CTA of the other lane (plan.cu: vdt_plan::lanes); VDT_GN_THREADS overrides
-    static int max_threads = 0;
-    if (max_threads == 0) {
-        const char* e = getenv("VDT_GN_THREADS");
-        max_threads = e ? atoi(e) : 256;
-        if (max_threads < 32 || max_threads > 1024) max_threads = 256;
-    }
+    // threads per CTA: 256 (16 K registers, ~1 KB of shared memory), so that a GroupNorm CTA fits on an SM next to a
+    // resident conv / attention CTA of the other lane (plan.cu: vdt_plan::kLanes)
+    constexpr int max_threads = 256;
     int PPH = (max_threads > CV ? max_threads : CV) / CV;
     const int work = (p.resample == kResDown) ? HW / 4 : HW;
     if (PPH > work) PPH = work;

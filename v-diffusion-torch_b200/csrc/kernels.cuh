@@ -45,7 +45,6 @@ struct alignas(64) ConvParams {
     int f16;                           // operand / 16-bit output format: 1 fp16, 0 bf16
     const float* bias;                 // [Cout]
     const float* residual;             // fp32 [M, ld] or null
-    int prefetch_next;                 // 1: the TMA warp prefetches the next work item's A rows into L2 (VDT_CONV_PREFETCH=1; measured slower, off by default)
     int pair_tiles;                    // tiles per image when a CTA pair works on the same tile of two consecutive images, else 0
     int resid_rep;                     // > 1: output image i adds residual image i / resid_rep ([M / resid_rep, ld]; CFG row pairs
                                        // share the residual computed before the first FiLM); power-of-two HW takes the fast epilogue
@@ -156,7 +155,6 @@ cudaError_t launch_groupnorm_backward(const GroupNormBwdParams& p, cudaStream_t 
 struct alignas(64) AttnParams {
     CUtensorMap q_map;                 // 2-D (3*hid, B*N) 16-bit, box (64, 128): q | k | v thirds, heads contiguous in each
     CUtensorMap kv_map;                // same tensor, box (64, 64): K tiles at column hid + h*d, V tiles at 2*hid + h*d
-    CUtensorMap k2_map;                // same tensor, box (64, 32): a CTA's half of a K tile in the CTA-pair variant
     int B, N, heads, d, hid;
     int f16;
     float scale_log2e;                 // log2(e) / sqrt(d)

@@ -359,7 +359,6 @@ struct vdt_plan {
     std::map<std::string, std::unique_ptr<Exec>> execs;
     uint64_t use_clock = 0;
     unsigned long long* sat_count = nullptr;  // device counter: fp16 operand packs that hit +-65504 (saturated)
-    bool use_graph = true;
     int f16 = 1;                          // GEMM operand format: 1 fp16 (default), 0 bf16
     int split = 0;                        // 1: split-precision validation mode (every operand as a hi/lo fp16 pair)
     int stat_cols = 4;                    // columns per GroupNorm statistics entry: 4, or 2 when some group is not a multiple of 4 channels
@@ -370,12 +369,11 @@ struct vdt_plan {
     // The chunks of a sampling batch are independent samples: they alternate between two lanes (streams, each with its
     // own workspace and step graph), so that one chunk's HBM-bound kernels (GroupNorm, small-N attention, 1x1 GEMMs)
     // can run on the SMs' spare warps while the other chunk's tensor-bound conv kernel holds the tensor cores.
-    int lanes = 2;                        // VDT_LANES = 1 .. kMaxLanes overrides
-    static constexpr int kMaxLanes = 4;
-    cudaStream_t lane_stream[kMaxLanes] = {};   // [0] unused: lane 0 is `work`
-    cudaEvent_t ev_fork = nullptr, ev_join[kMaxLanes] = {};
+    static constexpr int kLanes = 2;
+    cudaStream_t lane_stream[kLanes] = {};   // [0] unused: lane 0 is `work`
+    cudaEvent_t ev_fork = nullptr, ev_join[kLanes] = {};
     int sync_lanes() {
-        for (int l = 1; l < kMaxLanes; ++l)
+        for (int l = 1; l < kLanes; ++l)
             if (lane_stream[l] && cudaStreamSynchronize(lane_stream[l]) != cudaSuccess) return 1;
         return 0;
     }
@@ -387,7 +385,7 @@ struct vdt_plan {
         if (ev_in) cudaEventDestroy(ev_in);
         if (ev_out) cudaEventDestroy(ev_out);
         if (ev_fork) cudaEventDestroy(ev_fork);
-        for (int l = 1; l < kMaxLanes; ++l) {
+        for (int l = 1; l < kLanes; ++l) {
             if (ev_join[l]) cudaEventDestroy(ev_join[l]);
             if (lane_stream[l]) cudaStreamDestroy(lane_stream[l]);
         }
@@ -499,10 +497,6 @@ extern "C" int vdt_plan_create(const vdt_unet_config* cfg, vdt_plan** out) {
     if (c.operand_dtype < 0 || c.operand_dtype > 2) return fail("operand_dtype must be 0 (fp16), 1 (bf16) or 2 (fp16 x3 split)");
     p->f16 = c.operand_dtype != 1;
     p->split = c.operand_dtype == 2;
-    const char* ng = getenv("VDT_NO_GRAPH");
-    p->use_graph = !(ng && ng[0] == '1');
-    const char* ln = getenv("VDT_LANES");
-    if (ln && ln[0] >= '1' && ln[0] <= '0' + vdt_plan::kMaxLanes && ln[1] == 0) p->lanes = ln[0] - '0';
     int dev = 0;
     if (cudaGetDevice(&dev) == cudaSuccess) {
         int n = 0;
@@ -896,10 +890,6 @@ static int setup_conv(const ConvSpec& s, ConvParams* cp) {
     cp->ups = s.ups; cp->ups_w = s.w; cp->stat_slabs_img = slabs; cp->resid_up = s.resid_up; cp->out_w = s.w;
     cp->resid_rep = s.residual ? s.resid_rep : 0;
     {
-        const char* pf = getenv("VDT_CONV_PREFETCH");         // measured slower (-3 % images/s): opt-in only
-        cp->prefetch_next = (pf && pf[0] == '1') ? 1 : 0;
-    }
-    {
         const char* pt = getenv("VDT_PAIR_TILES");
         if (cp->resid_rep == 2 && !cp->pointwise && cp->box_n == 1 && cp->tiles_per_image >= 1 &&
             cp->num_m_tiles == s.n * cp->tiles_per_image && s.n % 2 == 0 && !(pt && pt[0] == '0'))
@@ -1106,7 +1096,6 @@ static int build_unet_steps(vdt_plan* p, Exec* ex, const float* film, const int*
                 memset(ap.get(), 0, sizeof(AttnParams));
                 CKI(make_map_2d(&ap->q_map, qkv, (long long)R * N, 3 * hidd, 3 * hidd, 128));
                 CKI(make_map_2d(&ap->kv_map, qkv, (long long)R * N, 3 * hidd, 3 * hidd, 64));
-                CKI(make_map_2d(&ap->k2_map, qkv, (long long)R * N, 3 * hidd, 3 * hidd, 32));
                 ap->B = R; ap->N = N; ap->heads = nh; ap->d = hd; ap->hid = hidd; ap->f16 = p->f16;
                 ap->scale_log2e = (float)(1.4426950408889634 / std::sqrt((double)hd));
                 ap->out = o;
@@ -1258,24 +1247,11 @@ static int run_steps_profiled(vdt_plan* p, Exec* ex, cudaStream_t st) {
     return rc;
 }
 
-// Measurement aid (VDT_IDLE_US=n): one thread sleeps n microseconds at the end of every step.  Tells a power-capped
-// step (the governor hands the idle time back as clock, throughput barely moves) from a time-bound one.
-__global__ void idle_kernel(unsigned long long ns) {
-    unsigned long long t0, t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-    do { __nanosleep(1000); asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); } while (t - t0 < ns);
-}
-static long long idle_us() {
-    static long long v = -1;
-    if (v < 0) { const char* e = getenv("VDT_IDLE_US"); v = e ? atoll(e) : 0; }
-    return v;
-}
-
-// Run the exec's step list, through a CUDA graph when enabled.
+// Run the exec's step list, through a CUDA graph once it has been captured.
 static int run_exec(vdt_plan* p, Exec* ex, cudaStream_t st) {
     if (g_profile.load()) { g_launches += ex->steps.size(); return run_steps_profiled(p, ex, st); }
     // first run is eager (sets function attributes, surfaces launch errors); the second run captures
-    if (p->use_graph && !ex->graph && !ex->graph_failed && ex->runs++ >= 1) {
+    if (!ex->graph && !ex->graph_failed && ex->runs++ >= 1) {
         cudaGraph_t g = nullptr;
         cudaError_t e = cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal);
         if (e == cudaSuccess) {
@@ -1299,13 +1275,14 @@ static int run_exec(vdt_plan* p, Exec* ex, cudaStream_t st) {
     } else {
         CKI(run_steps(p, ex, st));
     }
-    if (idle_us() > 0) idle_kernel<<<1, 1, 0, st>>>((unsigned long long)idle_us() * 1000ull);
     return 0;
 }
 
 // The plan keeps a handful of execs (workspace + captured graph per batch size / sampler signature).  A miss on a full
 // cache evicts the least recently used entry only; queued work may still use its buffers, hence the stream sync.
-constexpr size_t kMaxExecs = vdt_plan::kMaxLanes + 2;   // one sampler exec per lane + a ragged tail + a plain forward
+// Six entries: a sampling call uses up to three (a full chunk per lane and a ragged tail), which leaves room for plain
+// forwards and other batch sizes before an eviction makes a later call rebuild a workspace and re-capture its graph.
+constexpr size_t kMaxExecs = 6;
 static int exec_cache_lookup(vdt_plan* p, const std::string& key, Exec** out) {
     auto it = p->execs.find(key);
     if (it == p->execs.end()) { *out = nullptr; return 0; }
@@ -1682,7 +1659,7 @@ extern "C" int vdt_p_sample_range_inpaint(vdt_plan* p, const vdt_sampler_config*
     const int chunk = std::max(1, c.max_rows / rep);
     const int nchunks = (batch + chunk - 1) / chunk;
     // several lanes when there is more than one chunk (per-launch profiling needs a single ordered stream)
-    const int lanes = g_profile.load() ? 1 : std::max(1, std::min(p->lanes, nchunks));
+    const int lanes = g_profile.load() ? 1 : std::max(1, std::min(vdt_plan::kLanes, nchunks));
     if (lanes > 1) {
         if (!p->ev_fork) CK(cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming));
         CK(cudaEventRecord(p->ev_fork, p->work));
@@ -2162,7 +2139,6 @@ extern "C" int vdt_op_attention(const void* qkv, void* out, int32_t batch, int32
     memset(ap.get(), 0, sizeof(AttnParams));
     CKI(make_map_2d(&ap->q_map, qkv, (long long)batch * n, 3 * hid, 3 * hid, 128));
     CKI(make_map_2d(&ap->kv_map, qkv, (long long)batch * n, 3 * hid, 3 * hid, 64));
-    CKI(make_map_2d(&ap->k2_map, qkv, (long long)batch * n, 3 * hid, 3 * hid, 32));
     ap->B = batch; ap->N = n; ap->heads = heads; ap->d = d; ap->hid = hid; ap->f16 = f16;
     ap->scale_log2e = (float)(1.4426950408889634 / std::sqrt((double)d));
     ap->out = (h16*)out;

@@ -110,24 +110,10 @@ __device__ __forceinline__ void tma_load_4d_2cta(void* dst, const CUtensorMap* m
         "r"(c2), "r"(c3)
         : "memory");
 }
-// hint: bring a 4-D TMA box into L2 (no shared-memory destination, no completion to wait for)
-__device__ __forceinline__ void tma_prefetch_4d(const CUtensorMap* m, int c0, int c1, int c2, int c3) {
-    asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];"
-                 ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-// arrive on the mbarrier at this smem offset in CTA `cta` of the cluster
-__device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t cta) {
-    asm volatile(
-        "{\n\t.reg .b32 ra;\n\t"
-        "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-        "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
-        ::"r"(smem_u32(bar)), "r"(cta)
-        : "memory");
-}
-
-// Same without release semantics: no memory barrier is generated.  For hand-offs whose payload is not generic-proxy
-// memory (e.g. "this warp's tcgen05.ld of the accumulator have completed": ordered by tcgen05.wait::ld and
-// tcgen05.fence::before_thread_sync), where a release fence would only make the warp wait for its own global stores.
+// Arrive on the mbarrier at this smem offset in CTA `cta` of the cluster, without release semantics: no memory barrier
+// is generated.  For hand-offs whose payload is not generic-proxy memory (e.g. "this warp's tcgen05.ld of the
+// accumulator have completed": ordered by tcgen05.wait::ld and tcgen05.fence::before_thread_sync), where a release
+// fence would only make the warp wait for its own global stores.
 __device__ __forceinline__ void mbar_arrive_cluster_relaxed(uint64_t* bar, uint32_t cta) {
     asm volatile(
         "{\n\t.reg .b32 ra;\n\t"
