@@ -141,6 +141,31 @@ int vdt_p_sample_inpaint(vdt_plan* plan, const vdt_sampler_config* sc, const vdt
 int vdt_p_sample_range_inpaint(vdt_plan* plan, const vdt_sampler_config* sc, const vdt_inpaint* inpaint, float* x,
                                const void* label, const float* step_noise, int32_t batch, int32_t first_step,
                                int32_t num_steps, float* pred_x0, void* stream);
+/* Sampling from an intermediate time (SDEdit, Meng et al., 2022; re-sampling an inverted latent): x (in place, fp32
+ * [B, C, R, R]) is x at t = (first_step + 1) / T, and steps first_step ... 0 run as a fresh trajectory -- under
+ * DPM-Solver++(2M) step first_step is first-order, as step T-1 is for a whole trajectory.  DDIM, ancestral sampling, CFG and
+ * inpainting work unchanged; step_noise and known_noise stay [T, B, C, R, R], indexed by step.  first_step = T-1 is
+ * vdt_p_sample_inpaint (in place).  0 <= first_step < T. */
+int vdt_p_sample_from(vdt_plan* plan, const vdt_sampler_config* sc, const vdt_inpaint* inpaint /* nullable */, float* x,
+                      const void* label, const float* step_noise, int32_t batch, int32_t first_step, void* stream);
+/* DDIM inversion (Song et al., DDIM, section 4.3): the deterministic DDIM ODE walked forward in time to encode an image.
+ * Inversion step j (0 <= j < T) maps x at s = j/T to x at t = (j+1)/T, the (s, t) pair of sampler step j:
+ *   - the model is evaluated at the input's own time s (fp64 t = j/T; t = 0 at j = 0, where lambda = logsnr_max);
+ *   - x0 comes from the raw model output through the converters of every model_out_type at lambda_s, NOT clipped (a clip
+ *     would make the step impossible to invert); under CFG (w_guide > 0 and labels; rows 2i conditional, 2i+1
+ *     unconditional) the guided x0 = x0c + w (x0c - x0u) -- the step is linear in x0, so this is the sampler's guidance on
+ *     the means without its per-branch clip;
+ *   - x_t = c1' x_s + c2' x0, c1' = sigma_t / sigma_s = exp((logsigmoid(-l_t) - logsigmoid(-l_s)) / 2),
+ *     c2' = alpha_t - alpha_s c1' = -alpha_t expm1((l_s - l_t) / 2), in fp64 from the fp32-rounded log-SNRs, rounded once.
+ * For an x0-type model the first step multiplies the model's error at t = 0 by sigma_t / sigma_s (about 350 at T = 100 on
+ * the cosine +-20 schedule); v, eps and both are benign there, because x0 at lambda = logsnr_max reduces to x.
+ * Refused (vdt_last_error): use_ddim = 0, x0eps_coef = 1, solver != FIRST_ORDER, t_fp32 = 1, steps outside [0, T).
+ * vdt_invert_coefficients: out [T][16] in the vdt_step_coefficients layout -- slots 0-5 and 12-13 the converters at
+ * lambda_s, 6-7 c1' and c2', 10-11 l_s and l_t, every other slot 0.
+ * vdt_ddim_invert_range: in place on x (fp32 [B, C, R, R]), steps first_step ... first_step + num_steps - 1. */
+int vdt_invert_coefficients(const vdt_sampler_config* sc, float* out);
+int vdt_ddim_invert_range(vdt_plan* plan, const vdt_sampler_config* sc, float* x, const void* label, int32_t batch,
+                          int32_t first_step, int32_t num_steps, void* stream);
 /* Same with HOST buffers (pinned or pageable); copies in/out inside the call and synchronises. */
 int vdt_p_sample_host(vdt_plan* plan, const vdt_sampler_config* sc, const float* noise, const void* label,
                       const float* step_noise, float* out, int32_t batch);
@@ -331,6 +356,10 @@ int vdt_op_sampler_step_known(const float* model_out, const float* x_t, const fl
                               int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, int32_t step, const float* coef_host,
                               float w, float* pred_hist, const float* known, const float* mask, const float* known_noise,
                               uint64_t seed, const float* coef_prev_host, void* stream);
+/* One DDIM inversion step (vdt_ddim_invert_range) for a generic denoise_fn: x fp32 [B, C, H, W] at s -> x_next at t (may
+ * alias x); model_out as for vdt_op_sampler_step; coef_host = one row of vdt_invert_coefficients (host). */
+int vdt_op_invert_step(const float* model_out, const float* x, float* x_next, int32_t batch, int32_t c, int32_t hw, int32_t cfg,
+                       int32_t model_out_type, const float* coef_host, float w, void* stream);
 
 #ifdef __cplusplus
 }

@@ -212,7 +212,7 @@ cudaError_t launch_images_to_uint8(const float* x, uint8_t* out, int B, int C, i
 // Per-step device-side sampler state: everything that changes from step to step -- and everything that changes from
 // call to call (noise tensor, seed) -- lives here, so one captured CUDA graph is replayed for every step of every call.
 struct SamplerState {
-    int next_step;                     // step index the next begin_step will consume (T-1 .. 0)
+    int next_step;                     // step index the next begin_step will consume (T-1 .. 0; 0 .. T-1 for inversion)
     int step;                          // step index of the step in flight
     int img0;                          // first image of the current chunk (offset into injected noise)
     int t_fp32;                        // 1: t = (step+1)/T and the sinusoidal embedding are evaluated in fp32, as
@@ -228,12 +228,20 @@ struct SamplerState {
     const float* known;                // [Btotal, C, HW] known image in model space
     const float* mask;                 // [Btotal, C, HW] in [0, 1], 1 = known
     const float* known_noise;          // [T, Btotal, C, HW] injected z' or null
+    // first step of the call's trajectory: the begin-step zeroes c2k (slot 15) there, so DPM-Solver++(2M) starts with a
+    // first-order step when sampling starts at an intermediate time.  T-1 for a whole trajectory (where c2k is 0 already)
+    // and for a range of one.  Kept last: coef must stay 16-byte aligned for the step kernel's float4 reads.
+    int start_step;
 };
 constexpr int kCoefStride = 16;
 // single-thread kernel: st->step = st->next_step--, copies the coefficient row (and slots 0, 1 of row step - 1 into
-// known_a / known_s when step > 0), writes t_rows[r] = (step+1)/T
+// known_a / known_s when step > 0; c2k zeroed when step == start_step), writes t_rows[r] = (step+1)/T
 cudaError_t launch_sampler_begin_step(SamplerState* st, const float* coef_table, double* t_rows, int nrows, int T,
                                       cudaStream_t stream);
+// the same for DDIM inversion, which walks upwards: st->step = st->next_step++, copies row step of the inversion table
+// (vdt_invert_coefficients), writes t_rows[r] = step/T (fp64): the model sees the input's own time
+cudaError_t launch_invert_begin_step(SamplerState* st, const float* coef_table, double* t_rows, int nrows, int T,
+                                     cudaStream_t stream);
 
 struct SamplerStepParams {
     const float* model_out;            // fp32 NCHW [B*(1+cfg), Cm, HW]; cond rows even, uncond rows odd
@@ -251,6 +259,10 @@ struct SamplerStepParams {
     int x0eps;                         // posterior mean = c1 * eps + c2 * x0, eps re-derived from the clipped x0
 };
 cudaError_t launch_sampler_step(const SamplerStepParams& p, cudaStream_t stream);
+// One DDIM inversion step x_s -> x_t on the same parameters: x_t (the input, at s) -> x_s (the output, at t, may alias),
+// x_t = c1' x_s + c2' x0 with the unclipped (guided) x0 and the coefficient row in st->coef; pred_x0, x0eps and the state's
+// noise and inpainting fields are not read.
+cudaError_t launch_invert_step(const SamplerStepParams& p, cudaStream_t stream);
 
 // ------------------------------------------------------------------------------------------------
 // Training-step kernels (train.cu): GaussianDiffusion.train_loss around the model call (diffusion.py:492-545)

@@ -220,10 +220,10 @@ __global__ void multitag_rows_kernel(const float* __restrict__ label, float* __r
     y_rows[i] = (rep == 2 && (r & 1)) ? 0.f : label[(size_t)(r / rep) * ncls + k];
 }
 // every per-call field is written, the inpainting pointers too (null when the call has none): execs are reused across calls
-__global__ void sampler_init_state_kernel(SamplerState* st, int next_step, int img0, int t_fp32, const float* noise,
+__global__ void sampler_init_state_kernel(SamplerState* st, int next_step, int start_step, int img0, int t_fp32, const float* noise,
                                           long long noise_stride, unsigned long long seed, vdt_inpaint inp) {
     if (threadIdx.x == 0 && blockIdx.x == 0) {
-        st->next_step = next_step; st->step = next_step; st->img0 = img0; st->t_fp32 = t_fp32;
+        st->next_step = next_step; st->step = next_step; st->start_step = start_step; st->img0 = img0; st->t_fp32 = t_fp32;
         st->noise = noise; st->noise_step_stride = noise_stride; st->seed = seed;
         st->known_a = 0.f; st->known_s = 0.f;
         st->known = inp.known; st->mask = inp.mask; st->known_noise = inp.known_noise;
@@ -260,7 +260,8 @@ struct Block {
     float* bias2 = nullptr;   // conv2.bias (+ skip.bias)
 };
 
-enum StepKind { S_CONV, S_GN, S_ATTN, S_IM2COL, S_TEMB, S_LINEAR, S_CLSEMB, S_BEGIN, S_SAMPLE, S_ATTN_F32, S_TAPSUM };
+enum StepKind { S_CONV, S_GN, S_ATTN, S_IM2COL, S_TEMB, S_LINEAR, S_CLSEMB, S_BEGIN, S_SAMPLE, S_ATTN_F32, S_TAPSUM, S_BEGIN_INV,
+                S_INVERT };
 struct TapsumArgs { const float* y; const float* bias; float* out; int B, H, W, Cout, ld; };
 struct LinearArgs { const float *x, *W, *b; float* out; int rows, K, N, silu; };
 struct Im2colArgs { const float* x; h16* out; h16* out_lo; int B, rep, C, H, W, f16; };
@@ -1216,6 +1217,8 @@ static int run_steps(vdt_plan* p, Exec* ex, cudaStream_t st, std::vector<cudaEve
             }
             case S_BEGIN: { auto& a = ex->begins[s.idx]; e = launch_sampler_begin_step(a.st, a.table, a.t_rows, a.nrows, a.T, st); break; }
             case S_SAMPLE: e = launch_sampler_step(ex->samples[s.idx], st); break;
+            case S_BEGIN_INV: { auto& a = ex->begins[s.idx]; e = launch_invert_begin_step(a.st, a.table, a.t_rows, a.nrows, a.T, st); break; }
+            case S_INVERT: e = launch_invert_step(ex->samples[s.idx], st); break;
             case S_TAPSUM: { auto& a = ex->tapsums[s.idx]; e = launch_tapsum3x3(a.y, a.bias, a.out, a.B, a.H, a.W, a.Cout, a.ld, st); break; }
             case S_ATTN_F32: { auto& a = ex->attn32s[s.idx]; e = launch_attention_f32(a.qkv, a.hi, a.lo, a.B, a.N, a.heads, a.d, a.f16, st); break; }
         }
@@ -1405,6 +1408,21 @@ static int logsnr_d(const vdt_sampler_config& sc, double t, double* out) {
     return fail("unknown logsnr schedule %d", sc.logsnr_schedule);   // NotImplementedError, diffusion.py:96
 }
 
+// The prediction converters at one fp32 log-SNR l, fp32 math like the reference's TorchScript converters (diffusion.py:206-245):
+// slots 0-5 alpha, sigma, rsqrt(sigmoid l), exp(-l/2), sigmoid l, sigmoid -l and 12-13 rsqrt(sigmoid -l) (pred_eps_from_x0,
+// diffusion.py:222-223), exp(l/2) of a vdt_step_coefficients row.
+static void converter_slots(float l, float* o) {
+    const float sig_pos = 1.0f / (1.0f + std::exp(-l)), sig_neg = 1.0f / (1.0f + std::exp(l));
+    o[0] = std::sqrt(sig_pos);
+    o[1] = std::sqrt(sig_neg);
+    o[2] = 1.0f / std::sqrt(sig_pos);
+    o[3] = std::exp(-0.5f * l);
+    o[4] = sig_pos;
+    o[5] = sig_neg;
+    o[12] = 1.0f / std::sqrt(sig_neg);
+    o[13] = std::exp(0.5f * l);
+}
+
 // DPM-Solver++(2M) is defined here on the data prediction of the DDIM (eta = 0) step only.
 static int check_solver(const vdt_sampler_config& sc) {
     if (sc.solver == VDT_SOLVER_FIRST_ORDER) return 0;
@@ -1461,13 +1479,7 @@ extern "C" int vdt_step_coefficients(const vdt_sampler_config* scp, float* out) 
             else return fail("unknown model_var_type %d", sc.model_var_type);   // NotImplementedError, diffusion.py:161
         }
         float* o = out + (size_t)i * kCoefStride;
-        const float sig_pos = 1.0f / (1.0f + std::exp(-lt32)), sig_neg = 1.0f / (1.0f + std::exp(lt32));
-        o[0] = std::sqrt(sig_pos);
-        o[1] = std::sqrt(sig_neg);
-        o[2] = 1.0f / std::sqrt(sig_pos);
-        o[3] = std::exp(-0.5f * lt32);
-        o[4] = sig_pos;
-        o[5] = sig_neg;
+        converter_slots(lt32, o);
         o[6] = (float)c1;
         o[7] = (float)c2;
         const float lv32 = (float)logvar;
@@ -1475,8 +1487,6 @@ extern "C" int vdt_step_coefficients(const vdt_sampler_config* scp, float* out) 
         o[9] = lv32;
         o[10] = ls32;
         o[11] = lt32;
-        o[12] = 1.0f / std::sqrt(sig_neg);           // pred_eps_from_x0 (diffusion.py:222-223)
-        o[13] = std::exp(0.5f * lt32);
         o[14] = sc.x0eps_coef ? 1.0f : 0.0f;         // lets vdt_op_sampler_step pick the (eps, x0) form from the row alone
         o[15] = 0.0f;
         h[i] = 0.5 * (ls - lt);
@@ -1487,6 +1497,42 @@ extern "C" int vdt_step_coefficients(const vdt_sampler_config* scp, float* out) 
     // The first step (i = T-1) is DDIM; the last (i = 0) returns the guided x0 like DDIM.
     if (sc.solver == VDT_SOLVER_DPMPP_2M)
         for (int i = 1; i < T - 1; ++i) out[(size_t)i * kCoefStride + 15] = (float)(c2d[i] * (h[i] / (2.0 * h[i + 1])));
+    return 0;
+}
+
+// DDIM inversion runs the deterministic first-order step with the p_sample time grid (fp64 t) and the data-prediction form.
+static int check_invert(const vdt_sampler_config& sc) {
+    if (sc.sample_timesteps < 1) return fail("sample_timesteps must be >= 1");
+    if (!sc.use_ddim) return fail("DDIM inversion needs use_ddim = 1 (the ancestral step is not deterministic)");
+    if (sc.x0eps_coef)
+        return fail("DDIM inversion needs x0eps_coef = 0 (under DDIM the reference's (eps, x0) coefficients are logarithms)");
+    if (sc.solver != VDT_SOLVER_FIRST_ORDER) return fail("DDIM inversion is first-order: solver must be 0 (got %d)", sc.solver);
+    if (sc.t_fp32) return fail("DDIM inversion runs the fp64 time grid of p_sample: t_fp32 must be 0");
+    return 0;
+}
+
+// Row j maps x at s = j/T to x at t = (j+1)/T: converters at lambda_s (the model sees x_s at time s), c1' = sigma_t / sigma_s,
+// c2' = alpha_t - alpha_s c1' = -alpha_t expm1((l_s - l_t) / 2), in fp64 from the fp32-rounded log-SNRs and rounded once.
+extern "C" int vdt_invert_coefficients(const vdt_sampler_config* scp, float* out) {
+    if (!scp || !out) return fail("null argument");
+    const vdt_sampler_config& sc = *scp;
+    CKI(check_invert(sc));
+    const int T = sc.sample_timesteps;
+    for (int j = 0; j < T; ++j) {
+        double ls_d, lt_d;
+        CKI(logsnr_d(sc, (double)j / (double)T, &ls_d));
+        CKI(logsnr_d(sc, (double)(j + 1) / (double)T, &lt_d));
+        const float ls32 = (float)ls_d, lt32 = (float)lt_d;
+        const double ls = ls32, lt = lt32;
+        if (!(lt < ls)) return fail("log-SNR schedule is not strictly decreasing at step %d", j);
+        float* o = out + (size_t)j * kCoefStride;
+        for (int k = 0; k < kCoefStride; ++k) o[k] = 0.0f;
+        converter_slots(ls32, o);
+        o[6] = (float)std::exp(0.5 * (logsigmoid_d(-lt) - logsigmoid_d(-ls)));
+        o[7] = (float)(-std::exp(0.5 * logsigmoid_d(lt)) * std::expm1(0.5 * (ls - lt)));
+        o[10] = ls32;
+        o[11] = lt32;
+    }
     return 0;
 }
 
@@ -1504,11 +1550,8 @@ extern "C" int vdt_train_coefficients(const vdt_sampler_config* scp, const doubl
         const float l = (float)l_d;
         float* o = out + (size_t)i * kCoefStride;
         for (int k = 0; k < kCoefStride; ++k) o[k] = 0.f;
-        const float sp = 1.0f / (1.0f + std::exp(-l)), sn = 1.0f / (1.0f + std::exp(l));
-        o[0] = std::sqrt(sp); o[1] = std::sqrt(sn);
-        o[2] = 1.0f / std::sqrt(sp); o[3] = std::exp(-0.5f * l);
-        o[4] = sp; o[5] = sn; o[11] = l;
-        o[12] = 1.0f / std::sqrt(sn); o[13] = std::exp(0.5f * l);
+        converter_slots(l, o);
+        o[11] = l;
     }
     return 0;
 }
@@ -1562,14 +1605,15 @@ extern "C" int vdt_adamw_ema_step(float* param, const float* grad, float* exp_av
 }
 
 // ================================================================================================ sampler
-static int get_sampler_exec(vdt_plan* p, const vdt_sampler_config& sc, int imgs, bool has_label, int lane, Exec** out) {
+// invert: the DDIM inversion exec (ascending begin-step, invert_step_kernel, vdt_invert_coefficients), cached under its own key
+static int get_sampler_exec(vdt_plan* p, const vdt_sampler_config& sc, int imgs, bool has_label, int lane, bool invert, Exec** out) {
     const bool cfg = sc.w_guide > 0.0 && has_label;            // diffusion.py:368
     const int rep = cfg ? 2 : 1;
     // the key holds what shapes the workspace, the coefficient table and the kernel parameters baked into the graph;
     // per-call values (seed, injected-noise tensor, fp32-t mode of p_sample_progressive) live in the device-side
     // SamplerState and are rewritten before every call
     char key[208];
-    snprintf(key, sizeof(key), "smp%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%.17g:%.17g:%.17g:%.17g", lane, imgs, (int)has_label,
+    snprintf(key, sizeof(key), "%s%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%.17g:%.17g:%.17g:%.17g", invert ? "inv" : "smp", lane, imgs, (int)has_label,
              sc.sample_timesteps, sc.model_out_type, sc.model_var_type, sc.logsnr_schedule, sc.use_ddim, sc.x0eps_coef, sc.t_fp32,
              sc.solver, sc.intp_frac, sc.logsnr_min, sc.logsnr_max, sc.w_guide);
     CKI(exec_cache_lookup(p, key, out));
@@ -1600,13 +1644,13 @@ static int get_sampler_exec(vdt_plan* p, const vdt_sampler_config& sc, int imgs,
     iota_i64_kernel<<<(ex->emb_rows + 127) / 128, 128, 0, p->work>>>(ex->y_rows, ex->emb_rows);
     CK(cudaGetLastError());
     std::vector<float> coefs((size_t)T * kCoefStride);
-    CKI(vdt_step_coefficients(&sc, coefs.data()));
+    CKI(invert ? vdt_invert_coefficients(&sc, coefs.data()) : vdt_step_coefficients(&sc, coefs.data()));
     CK(cudaMemcpyAsync(ex->coef_table, coefs.data(), coefs.size() * 4, cudaMemcpyHostToDevice, p->work));
     CK(cudaStreamSynchronize(p->work));              // `coefs` is a host temporary
     float* film;
     CKI(ex->acquire((size_t)ex->emb_rows * p->film_total * 4, (void**)&film));
     ex->begins.push_back({ex->state, ex->coef_table, ex->t_rows, ex->emb_rows, T});
-    ex->steps.push_back({S_BEGIN, 0});
+    ex->steps.push_back({invert ? S_BEGIN_INV : S_BEGIN, 0});
     CKI(add_embedding_steps(p, ex.get(), film, cond_model));
     CKI(build_unet_steps(p, ex.get(), film, mt ? nullptr : ex->film_row));
     SamplerStepParams sp{};
@@ -1614,7 +1658,7 @@ static int get_sampler_exec(vdt_plan* p, const vdt_sampler_config& sc, int imgs,
     sp.st = ex->state; sp.B = imgs; sp.C = c.in_channels; sp.HW = (int)HW; sp.cfg = cfg ? 1 : 0;
     sp.model_out_type = sc.model_out_type; sp.w = (float)sc.w_guide; sp.x0eps = sc.x0eps_coef ? 1 : 0;
     ex->samples.push_back(sp);
-    ex->steps.push_back({S_SAMPLE, 0});
+    ex->steps.push_back({invert ? S_INVERT : S_SAMPLE, 0});
     *out = ex.get();
     p->execs[key] = std::move(ex);
     return 0;
@@ -1628,25 +1672,12 @@ static int check_inpaint(const float* known, const float* mask, const float* kno
     return 0;
 }
 
-extern "C" int vdt_p_sample_range_inpaint(vdt_plan* p, const vdt_sampler_config* scp, const vdt_inpaint* inpaint, float* x,
-                                          const void* label, const float* step_noise, int32_t batch, int32_t first_step,
-                                          int32_t num_steps, float* pred_x0, void* stream) {
-    if (!p || !scp || !x) return fail("null argument");
-    const vdt_inpaint inp = inpaint ? *inpaint : vdt_inpaint{nullptr, nullptr, nullptr};
-    CKI(check_inpaint(inp.known, inp.mask, inp.known_noise));
-    const vdt_sampler_config& sc = *scp;
-    const int T = sc.sample_timesteps;
-    CKI(check_solver(sc));
-    // DPM-Solver++(2M) steps after the first read the previous step's guided x0: a range that starts inside the trajectory
-    // takes it from pred_x0 (written by the call that ran step first_step + 1), since the exec's pred buffer is shared by
-    // every chunk of its lane
-    const bool carry_pred = sc.solver == VDT_SOLVER_DPMPP_2M && first_step < T - 1 && num_steps > 0;
-    if (carry_pred && !pred_x0)
-        return fail("DPM-Solver++(2M) from step %d < T-1 needs pred_x0 holding the guided x0 of step %d", first_step, first_step + 1);
-    if (!p->finalized) return fail("plan not finalized (load every state_dict key, then vdt_plan_finalize)");
-    if (sc.model_out_type < 0 || sc.model_out_type > 3) return fail("unknown model_out_type %d", sc.model_out_type);
-    if (first_step < 0 || first_step >= T || num_steps < 0 || first_step - num_steps < -1)
-        return fail("step range [%d, %d) steps leaves the trajectory of %d steps", first_step, num_steps, T);
+// The chunk and lane loop shared by sampling and inversion; its callers check every argument first.  Sampling runs steps
+// first_step, first_step - 1, ... (num_steps of them) with `start_step` as the first step of the trajectory (see SamplerState);
+// inversion (invert) runs first_step, first_step + 1, ...
+static int run_sampler_range(vdt_plan* p, const vdt_sampler_config& sc, const vdt_inpaint& inp, float* x, const void* label,
+                             const float* step_noise, int32_t batch, int32_t first_step, int32_t num_steps, float* pred_x0,
+                             bool carry_pred, int start_step, bool invert, void* stream) {
     cudaStream_t user = reinterpret_cast<cudaStream_t>(stream);
     CKI(enter_work(p, user));
     cudaStream_t st = p->work;
@@ -1676,7 +1707,7 @@ extern "C" int vdt_p_sample_range_inpaint(vdt_plan* p, const vdt_sampler_config*
         const int lane = ci % lanes;
         st = lane ? p->lane_stream[lane] : p->work;
         Exec* ex;
-        CKI(get_sampler_exec(p, sc, imgs, label != nullptr, lane, &ex));
+        CKI(get_sampler_exec(p, sc, imgs, label != nullptr, lane, invert, &ex));
         CK(cudaMemcpyAsync(ex->xin, x + (size_t)i0 * CHW, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
         if (carry_pred) CK(cudaMemcpyAsync(ex->pred, pred_x0 + (size_t)i0 * CHW, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
         if (mt) {
@@ -1688,7 +1719,7 @@ extern "C" int vdt_p_sample_range_inpaint(vdt_plan* p, const vdt_sampler_config*
                                                                      c.num_classes);
         }
         CK(cudaGetLastError());
-        sampler_init_state_kernel<<<1, 32, 0, st>>>(ex->state, first_step, i0, sc.t_fp32 ? 1 : 0, step_noise,
+        sampler_init_state_kernel<<<1, 32, 0, st>>>(ex->state, first_step, start_step, i0, sc.t_fp32 ? 1 : 0, step_noise,
                                                     (long long)batch * (long long)CHW, (unsigned long long)sc.seed, inp);
         CK(cudaGetLastError());
         g_launches += 2;
@@ -1702,6 +1733,62 @@ extern "C" int vdt_p_sample_range_inpaint(vdt_plan* p, const vdt_sampler_config*
         CK(cudaStreamWaitEvent(p->work, p->ev_join[l], 0));
     }
     return leave_work(p, user);
+}
+
+// checks shared by every fused sampling / inversion entry point, ahead of any CUDA call
+static int check_plan_for_sampler(const vdt_plan* p, const vdt_sampler_config& sc) {
+    if (!p->finalized) return fail("plan not finalized (load every state_dict key, then vdt_plan_finalize)");
+    if (sc.model_out_type < 0 || sc.model_out_type > 3) return fail("unknown model_out_type %d", sc.model_out_type);
+    return 0;
+}
+
+extern "C" int vdt_p_sample_range_inpaint(vdt_plan* p, const vdt_sampler_config* scp, const vdt_inpaint* inpaint, float* x,
+                                          const void* label, const float* step_noise, int32_t batch, int32_t first_step,
+                                          int32_t num_steps, float* pred_x0, void* stream) {
+    if (!p || !scp || !x) return fail("null argument");
+    const vdt_inpaint inp = inpaint ? *inpaint : vdt_inpaint{nullptr, nullptr, nullptr};
+    CKI(check_inpaint(inp.known, inp.mask, inp.known_noise));
+    const vdt_sampler_config& sc = *scp;
+    const int T = sc.sample_timesteps;
+    CKI(check_solver(sc));
+    // DPM-Solver++(2M) steps after the first read the previous step's guided x0: a range that starts inside the trajectory
+    // takes it from pred_x0 (written by the call that ran step first_step + 1), since the exec's pred buffer is shared by
+    // every chunk of its lane
+    const bool carry_pred = sc.solver == VDT_SOLVER_DPMPP_2M && first_step < T - 1 && num_steps > 0;
+    if (carry_pred && !pred_x0)
+        return fail("DPM-Solver++(2M) from step %d < T-1 needs pred_x0 holding the guided x0 of step %d", first_step, first_step + 1);
+    CKI(check_plan_for_sampler(p, sc));
+    if (first_step < 0 || first_step >= T || num_steps < 0 || first_step - num_steps < -1)
+        return fail("step range [%d, %d) steps leaves the trajectory of %d steps", first_step, num_steps, T);
+    return run_sampler_range(p, sc, inp, x, label, step_noise, batch, first_step, num_steps, pred_x0, carry_pred, T - 1, false,
+                             stream);
+}
+
+extern "C" int vdt_p_sample_from(vdt_plan* p, const vdt_sampler_config* scp, const vdt_inpaint* inpaint, float* x,
+                                 const void* label, const float* step_noise, int32_t batch, int32_t first_step, void* stream) {
+    if (!p || !scp || !x) return fail("null argument");
+    const vdt_inpaint inp = inpaint ? *inpaint : vdt_inpaint{nullptr, nullptr, nullptr};
+    CKI(check_inpaint(inp.known, inp.mask, inp.known_noise));
+    const vdt_sampler_config& sc = *scp;
+    CKI(check_solver(sc));
+    if (first_step < 0 || first_step >= sc.sample_timesteps)
+        return fail("first_step %d lies outside [0, %d)", first_step, sc.sample_timesteps);
+    CKI(check_plan_for_sampler(p, sc));
+    return run_sampler_range(p, sc, inp, x, label, step_noise, batch, first_step, first_step + 1, nullptr, false, first_step,
+                             false, stream);
+}
+
+extern "C" int vdt_ddim_invert_range(vdt_plan* p, const vdt_sampler_config* scp, float* x, const void* label, int32_t batch,
+                                     int32_t first_step, int32_t num_steps, void* stream) {
+    if (!p || !scp || !x) return fail("null argument");
+    const vdt_sampler_config& sc = *scp;
+    CKI(check_invert(sc));
+    const int T = sc.sample_timesteps;
+    if (first_step < 0 || first_step >= T || num_steps < 0 || num_steps > T - first_step)
+        return fail("inversion steps [%d, %d + %d) leave [0, %d)", first_step, first_step, num_steps, T);
+    CKI(check_plan_for_sampler(p, sc));
+    const vdt_inpaint none{nullptr, nullptr, nullptr};
+    return run_sampler_range(p, sc, none, x, label, nullptr, batch, first_step, num_steps, nullptr, false, T - 1, true, stream);
 }
 
 extern "C" int vdt_p_sample_range(vdt_plan* p, const vdt_sampler_config* scp, float* x, const void* label,
@@ -2214,6 +2301,29 @@ extern "C" int vdt_op_sampler_step_known(const float* model_out, const float* x_
                                          const float* known_noise, uint64_t seed, const float* coef_prev_host, void* stream) {
     return op_sampler_step_impl(model_out, x_t, noise, x_s, batch, c, hw, cfg, model_out_type, step, coef_host, w, pred_hist,
                                 known, mask, known_noise, seed, coef_prev_host, stream);
+}
+
+extern "C" int vdt_op_invert_step(const float* model_out, const float* x, float* x_next, int32_t batch, int32_t c, int32_t hw,
+                                  int32_t cfg, int32_t model_out_type, const float* coef_host, float w, void* stream) {
+    if (!model_out || !x || !x_next || !coef_host) return fail("null argument");
+    if (model_out_type < 0 || model_out_type > 3) return fail("unknown model_out_type %d", model_out_type);
+    if (batch < 0 || c < 1 || hw < 1) return fail("bad image shape (%d, %d, %d)", batch, c, hw);
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    SamplerState hs{};
+    for (int i = 0; i < kCoefStride; ++i) hs.coef[i] = coef_host[i];
+    SamplerState* ds = nullptr;
+    CK(cudaMalloc(&ds, sizeof(SamplerState)));
+    CK(cudaMemcpy(ds, &hs, sizeof(hs), cudaMemcpyHostToDevice));
+    SamplerStepParams sp{};
+    sp.model_out = model_out; sp.x_t = x; sp.x_s = x_next; sp.st = ds; sp.B = batch; sp.C = c; sp.HW = hw; sp.cfg = cfg ? 1 : 0;
+    sp.model_out_type = model_out_type; sp.w = w;
+    cudaError_t e = launch_invert_step(sp, st);
+    ++g_launches;
+    cudaError_t e2 = cudaStreamSynchronize(st);
+    cudaFree(ds);
+    if (e != cudaSuccess) return fail("invert_step launch failed: %s", cudaGetErrorString(e));
+    if (e2 != cudaSuccess) return fail("invert_step failed: %s", cudaGetErrorString(e2));
+    return 0;
 }
 
 // ---- entry points the composed training step (v-diffusion-torch_b200/training.py) adds to the kernel-level hooks ----------

@@ -198,6 +198,8 @@ __global__ void sampler_begin_step_kernel(SamplerState* st, const float* __restr
         st->step = step;
         st->next_step = step - 1;
         for (int i = 0; i < kCoefStride; ++i) st->coef[i] = coef_table[step * kCoefStride + i];
+        // a trajectory that starts at this step (sampling from an intermediate time) has no previous guided x0 for 2M
+        if (step == st->start_step) st->coef[15] = 0.f;
         // inpainting: the known image is diffused to this step's s = step / T, which is row step - 1's t (in both t modes)
         if (step > 0) {
             st->known_a = coef_table[(step - 1) * kCoefStride + 0];
@@ -206,6 +208,19 @@ __global__ void sampler_begin_step_kernel(SamplerState* st, const float* __restr
         // t = (step + 1) / T: fp64 in p_sample (diffusion.py:399, 364), fp32 in p_sample_progressive (diffusion.py:421)
         const double t = st->t_fp32 ? static_cast<double>(__fdiv_rn(static_cast<float>(step + 1), static_cast<float>(T)))
                                     : static_cast<double>(step + 1) / static_cast<double>(T);
+        for (int r = 0; r < nrows; ++r) t_rows[r] = t;
+    }
+}
+
+// Inversion walks the steps upwards: st->step = st->next_step++, and the model sees the input's own time s = step / T (fp64;
+// the table of an inversion exec is vdt_invert_coefficients, which refuses the fp32-t mode)
+__global__ void invert_begin_step_kernel(SamplerState* st, const float* __restrict__ coef_table, double* t_rows, int nrows, int T) {
+    if (threadIdx.x == 0 && blockIdx.x == 0) {
+        const int step = st->next_step;
+        st->step = step;
+        st->next_step = step + 1;
+        for (int i = 0; i < kCoefStride; ++i) st->coef[i] = coef_table[step * kCoefStride + i];
+        const double t = static_cast<double>(step) / static_cast<double>(T);
         for (int r = 0; r < nrows; ++r) t_rows[r] = t;
     }
 }
@@ -227,13 +242,18 @@ __device__ __forceinline__ float4 philox_normal4(unsigned long long seed, uint32
     return make_float4(ra * ca, ra * sa, rb * cb, rb * sb);
 }
 
-__device__ __forceinline__ float pred_x0(int type, float x, float o, float o2, const float* cf) {
+// x0 from the raw model output, unclipped: the inversion step needs it so (a clip would make the step impossible to invert)
+__device__ __forceinline__ float pred_x0_raw(int type, float x, float o, float o2, const float* cf) {
     float x0;
     if (type == 3) x0 = x * cf[0] - o * cf[1];                       // v   (diffusion.py:233-234)
     else if (type == 0) x0 = o;                                      // x0
     else if (type == 1) x0 = x * cf[2] - o * cf[3];                  // eps (diffusion.py:207-208)
     else { const float xe = x * cf[2] - o2 * cf[3]; x0 = o * cf[5] + xe * cf[4]; }   // both (211-214)
-    return fminf(fmaxf(x0, -1.f), 1.f);                              // clip_denoised (diffusion.py:327)
+    return x0;
+}
+
+__device__ __forceinline__ float pred_x0(int type, float x, float o, float o2, const float* cf) {
+    return fminf(fmaxf(pred_x0_raw(type, x, o, o2, cf), -1.f), 1.f);   // clip_denoised (diffusion.py:327)
 }
 
 template <int VEC> struct SVec;
@@ -366,6 +386,59 @@ __global__ void __launch_bounds__(256, 6) sampler_step_kernel(const SamplerStepP
     stv(p.x_s + i, out);
 }
 
+// DDIM inversion (Song et al., DDIM, section 4.3): one step of the deterministic DDIM ODE forward in time, x at s -> x at t,
+// x_t = c1' x_s + c2' x0 with the UNCLIPPED x0 at lambda_s and, under CFG, the guided x0c + w (x0c - x0u) (the step is linear in
+// x0).  A kernel of its own rather than a mode of sampler_step_kernel, whose register budget (six blocks per SM) a branch for
+// this caller would spend.  p.x_t is the input x_s, p.x_s the output x_t; the coefficient row is one of vdt_invert_coefficients.
+template <int VEC>
+__global__ void __launch_bounds__(256) invert_step_kernel(const SamplerStepParams p) {
+    typedef typename SVec<VEC>::type vec_t;
+    const long long n = static_cast<long long>(p.B) * p.C * p.HW;
+    const long long i = (blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x) * VEC;
+    if (i >= n) return;
+    float cf[kCoefStride];
+#pragma unroll
+    for (int k = 0; k < kCoefStride; k += 4) {
+        const float4 c4 = *reinterpret_cast<const float4*>(p.st->coef + k);
+        cf[k] = c4.x; cf[k + 1] = c4.y; cf[k + 2] = c4.z; cf[k + 3] = c4.w;
+    }
+    const int chw = p.C * p.HW;
+    const int b = static_cast<int>(i / chw), e = static_cast<int>(i % chw);
+    const int Cm = (p.model_out_type == 2) ? 2 * p.C : p.C;
+    const int rep = 1 + p.cfg;
+    const float* mo = p.model_out + static_cast<size_t>(b) * rep * Cm * p.HW + e;
+    const size_t second = static_cast<size_t>(p.C) * p.HW;           // "both": eps half follows the x0 half
+    float x[VEC], o[VEC], o2[VEC], u[VEC], u2[VEC], out[VEC];
+    auto ldv = [](const float* q, float (&v)[VEC]) {
+        const vec_t t = *reinterpret_cast<const vec_t*>(q);
+        const float* f = reinterpret_cast<const float*>(&t);
+#pragma unroll
+        for (int k = 0; k < VEC; ++k) v[k] = f[k];
+    };
+    ldv(p.x_t + i, x);
+    ldv(mo, o);
+    if (p.model_out_type == 2) ldv(mo + second, o2);
+    if (p.cfg) {
+        ldv(mo + static_cast<size_t>(Cm) * p.HW, u);
+        if (p.model_out_type == 2) ldv(mo + static_cast<size_t>(Cm) * p.HW + second, u2);
+    }
+    const float c1 = cf[6], c2 = cf[7];
+#pragma unroll
+    for (int k = 0; k < VEC; ++k) {
+        float x0 = pred_x0_raw(p.model_out_type, x[k], o[k], (p.model_out_type == 2) ? o2[k] : 0.f, cf);
+        if (p.cfg) {
+            const float x0u = pred_x0_raw(p.model_out_type, x[k], u[k], (p.model_out_type == 2) ? u2[k] : 0.f, cf);
+            x0 = x0 + p.w * (x0 - x0u);
+        }
+        out[k] = c1 * x[k] + c2 * x0;
+    }
+    vec_t t;
+    float* f = reinterpret_cast<float*>(&t);
+#pragma unroll
+    for (int k = 0; k < VEC; ++k) f[k] = out[k];
+    *reinterpret_cast<vec_t*>(p.x_s + i) = t;
+}
+
 // ------------------------------------------------------------------------------------------ out_conv tap sum
 // The network's last 3x3 conv has only Cout = out_channels (3 / 6 / 1) output channels: as an implicit GEMM its A operand
 // would be fetched nine times (once per tap) for an N tile of 16 columns.  It is computed instead as ONE pointwise GEMM
@@ -496,6 +569,23 @@ cudaError_t launch_class_embed_multitag_silu(const float* e, const float* y, con
 cudaError_t launch_sampler_begin_step(SamplerState* st, const float* coef_table, double* t_rows, int nrows, int T,
                                       cudaStream_t stream) {
     sampler_begin_step_kernel<<<1, 32, 0, stream>>>(st, coef_table, t_rows, nrows, T);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_invert_begin_step(SamplerState* st, const float* coef_table, double* t_rows, int nrows, int T,
+                                     cudaStream_t stream) {
+    invert_begin_step_kernel<<<1, 32, 0, stream>>>(st, coef_table, t_rows, nrows, T);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_invert_step(const SamplerStepParams& p, cudaStream_t stream) {
+    const long long n = static_cast<long long>(p.B) * p.C * p.HW;
+    if (n == 0) return cudaSuccess;
+    auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15u) == 0; };
+    // caller tensors at odd offsets (or planes of a size not divisible by 4) take the scalar kernel
+    const bool vec4 = (p.HW % 4 == 0) && al16(p.model_out) && al16(p.x_t) && al16(p.x_s);
+    if (vec4) invert_step_kernel<4><<<static_cast<unsigned>((n / 4 + 255) / 256), 256, 0, stream>>>(p);
+    else invert_step_kernel<1><<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(p);
     return cudaGetLastError();
 }
 

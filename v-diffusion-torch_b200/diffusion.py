@@ -175,19 +175,46 @@ class GaussianDiffusion:
         _lib.check(_lib.lib().vdt_step_coefficients(C.byref(sc), _lib.ptr(out)))
         return out
 
+    def invert_coefficients(self):
+        """[T, 16] fp32 host table of DDIM inversion (include/vdt_b200.h: vdt_invert_coefficients): row j maps x at j/T to
+        x at (j+1)/T."""
+        self._check_invertible()
+        sc = self.sampler_config(True)
+        out = torch.empty((self.sample_timesteps, _lib.COEF_STRIDE), dtype=torch.float32)
+        _lib.check(_lib.lib().vdt_invert_coefficients(C.byref(sc), _lib.ptr(out)))
+        return out
+
+    def _check_invertible(self):
+        if self.x0eps_coef:
+            raise NotImplementedError("DDIM inversion needs x0eps_coef=False (under DDIM the reference's (eps, x0) "
+                                      "coefficients are logarithms, diffusion.py:180-182)")
+
+    def _check_start_step(self, start_step):
+        """``start_step`` k of p_sample: None means T (a whole trajectory), else an int in [1, T]."""
+        T = self.sample_timesteps
+        if start_step is None:
+            return T
+        if isinstance(start_step, bool) or not isinstance(start_step, int) or not 1 <= start_step <= T:
+            raise ValueError(f"start_step must be an int in [1, {T}] (x is given at t = start_step / T), got {start_step!r}")
+        return start_step
+
     # ------------------------------------------------------------------ p_sample (diffusion.py:394-414)
     @torch.no_grad()
     def p_sample(self, denoise_fn, shape, noise=None, label=None, device="cpu", seed=None, use_ddim=False,
-                 step_noise=None, solver=None, known=None, mask=None, known_noise=None):
+                 step_noise=None, solver=None, known=None, mask=None, known_noise=None, start_step=None):
         """``step_noise`` (extension): optional (T, B, C, H, W) tensor of the per-step normal draws the
         reference takes from its generator (diffusion.py:389), so both sides inject identical noise.
         ``solver`` (extension): None (the reference's step) or "dpmpp_2m" (DPM-Solver++(2M), with use_ddim=True).
         ``known``, ``mask``, ``known_noise`` (extension): inpainting by replacement.  After every step the pixels with mask 1
         are set to ``known`` diffused to the step's time (alpha_s known + sigma_s z'), and the last step sets them to ``known``;
         a soft mask blends.  z' comes from ``known_noise`` or else from the library's noise stream keyed by ``seed`` (a fresh
-        seed when None, under DDIM too).  See include/vdt_b200.h vdt_inpaint."""
+        seed when None, under DDIM too).  See include/vdt_b200.h vdt_inpaint.
+        ``start_step`` (extension): k in [1, T]; ``noise`` is then x at t = k/T (e.g. an inverted latent, or an image diffused
+        to k/T for SDEdit) and steps k-1 ... 0 run as a fresh trajectory (DPM-Solver++(2M) starts first-order).  None means T,
+        the reference's loop.  ``step_noise`` and ``known_noise`` keep their (T, ...) shapes, indexed by step."""
         self._check_solver(solver, use_ddim)
         inp = self._check_inpaint(shape, known, mask, known_noise)
+        k = self._check_start_step(start_step)
         device = torch.device(device)
         if device.type != "cuda":
             raise RuntimeError("v_diffusion_b200 samples on CUDA (sm_100a) only; there is no CPU fallback")
@@ -219,7 +246,12 @@ class GaussianDiffusion:
             plan = denoise_fn.plan_for(shape[2], device)
             out = torch.empty_like(x_t)
             with torch.cuda.device(device):
-                if inp is None:
+                if start_step is not None:
+                    held, ip = self._inpaint_on(inp, shape, device) if inp is not None else (None, None)   # kept alive
+                    out.copy_(x_t)
+                    _lib.check(L.vdt_p_sample_from(plan, C.byref(sc), None if ip is None else C.byref(ip), _lib.ptr(out),
+                                                   _lib.ptr(label), _lib.ptr(step_noise), B, k - 1, _lib.current_stream_ptr()))
+                elif inp is None:
                     _lib.check(L.vdt_p_sample(plan, C.byref(sc), _lib.ptr(x_t), _lib.ptr(label), _lib.ptr(step_noise),
                                               _lib.ptr(out), B, _lib.current_stream_ptr()))
                 else:
@@ -231,7 +263,7 @@ class GaussianDiffusion:
         # that produced x_T, like the reference's single generator (diffusion.py:401-405, 389)
         sc = self.sampler_config(use_ddim, self._noise_seed(seed) if inp_seed else seed, solver=solver)
         held = None if inp is None else self._inpaint_on(inp, shape, device)[0]
-        return self._p_sample_generic(denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver, held).cpu()
+        return self._p_sample_generic(denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver, held, k).cpu()
 
     @torch.no_grad()
     def p_sample_progressive(self, denoise_fn, shape, noise=None, label=None, device="cpu", seed=None, use_ddim=False,
@@ -286,6 +318,64 @@ class GaussianDiffusion:
                 first = stop - 1
         return x.cpu(), preds
 
+    # ------------------------------------------------------------------ DDIM inversion (extension)
+    @torch.no_grad()
+    def ddim_invert(self, denoise_fn, x_0, label=None, device="cuda", num_steps=None, w_guide=None):
+        """DDIM inversion (Song et al., DDIM, section 4.3): runs the deterministic DDIM ODE forward in time from the image
+        ``x_0`` (model space, (B, C, R, R)) and returns x at t = num_steps / T on the CPU, like p_sample.  ``num_steps=None``
+        means T (a full encoding); ``p_sample(..., noise=latent, start_step=num_steps, use_ddim=True)`` decodes it again.
+        Step j evaluates the model at j/T and uses its unclipped x0; under CFG (``w_guide`` > 0 and labels, ``w_guide=None``
+        meaning ``self.w_guide``) the guided x0c + w (x0c - x0u).  The UNet runs on the fused path; any other callable goes
+        one step at a time through vdt_op_invert_step.  See include/vdt_b200.h vdt_ddim_invert_range.
+
+        For an "x0" model the first step multiplies the model's error at t = 0 by sigma_t / sigma_s (about 350 at T = 100 on
+        the cosine +-20 schedule), so an untrained x0 network's latents grow large; "v", "eps" and "both" are benign there."""
+        self._check_invertible()
+        T = self.sample_timesteps
+        n = T if num_steps is None else num_steps
+        if isinstance(n, bool) or not isinstance(n, int) or not 0 <= n <= T:
+            raise ValueError(f"num_steps must be an int in [0, {T}], got {num_steps!r}")
+        w = float(self.w_guide if w_guide is None else w_guide)
+        device = torch.device(device)
+        if device.type != "cuda":
+            raise RuntimeError("v_diffusion_b200 samples on CUDA (sm_100a) only; there is no CPU fallback")
+        if device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        x = x_0.to(device=device, dtype=torch.float32).contiguous().clone()
+        if x.ndim != 4:
+            raise ValueError(f"x_0 must have shape (B, C, R, R), got {tuple(x.shape)}")
+        B = x.shape[0]
+        if B == 0 or n == 0:
+            return x.cpu()
+        label = self._prepare_label(denoise_fn, label, B, device)
+        sc = self.sampler_config(True)
+        sc.w_guide = w
+        L = _lib.lib()
+        with torch.cuda.device(device):
+            if isinstance(denoise_fn, UNet):
+                plan = denoise_fn.plan_for(x.shape[2], device)
+                _lib.check(L.vdt_ddim_invert_range(plan, C.byref(sc), _lib.ptr(x), _lib.ptr(label), B, 0, n,
+                                                   _lib.current_stream_ptr()))
+                return x.cpu()
+            coefs = self.invert_coefficients()
+            use_cfg = (w > 0) and (label is not None)              # the sampler's rule (diffusion.py:368)
+            hw = x.shape[2] * x.shape[3]
+            for j in range(n):
+                t = torch.full((B,), j / T, dtype=torch.float64, device=device)
+                if use_cfg:
+                    xin, tin = x.repeat_interleave(2, dim=0), t.repeat_interleave(2)
+                    yin = label.repeat_interleave(2, dim=0)
+                    yin[1::2] = 0
+                else:
+                    xin, tin, yin = x, t, label
+                model_out = denoise_fn(xin, tin, yin).to(torch.float32).contiguous()
+                x_next = torch.empty_like(x)
+                _lib.check(L.vdt_op_invert_step(_lib.ptr(model_out), _lib.ptr(x), _lib.ptr(x_next), B, x.shape[1], hw,
+                                                int(use_cfg), sc.model_out_type, _lib.ptr(coefs[j].contiguous()), w,
+                                                _lib.current_stream_ptr()))
+                x = x_next
+        return x.cpu()
+
     # ------------------------------------------------------------------ train_loss (diffusion.py:492-545)
     @torch.no_grad()
     def train_loss(self, denoise_fn, x_0, t, y, noise=None, return_grad=False):
@@ -337,17 +427,20 @@ class GaussianDiffusion:
                                         _lib.REWEIGHT_TYPES[self.reweight_type], _lib.current_stream_ptr()))
         return (loss, grad) if return_grad else loss
 
-    def _p_sample_generic(self, denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver=None, inp=None):
+    def _p_sample_generic(self, denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver=None, inp=None,
+                          start_step=None):
         L = _lib.lib()
         B = shape[0]
+        T = self.sample_timesteps
+        k = T if start_step is None else start_step
         coefs = self.step_coefficients(use_ddim, solver)
+        coefs[k - 1, 15] = 0.                                       # the trajectory's first step has no 2M history
         # DPM-Solver++(2M): the guided x0 of the previous step, read by every step whose c2k is non-zero
         hist = torch.empty_like(x_t) if solver is not None else None
         use_cfg = (self.w_guide > 0) and (label is not None)        # diffusion.py:368
-        T = self.sample_timesteps
         hw = shape[2] * shape[3]
         with torch.cuda.device(device):
-            for ti in reversed(range(T)):
+            for ti in reversed(range(k)):
                 t = torch.full((B,), (ti + 1) / T, dtype=torch.float64, device=device)
                 if use_cfg:
                     xin, tin = x_t.repeat_interleave(2, dim=0), t.repeat_interleave(2)
