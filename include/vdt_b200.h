@@ -166,6 +166,43 @@ int vdt_p_sample_from(vdt_plan* plan, const vdt_sampler_config* sc, const vdt_in
 int vdt_invert_coefficients(const vdt_sampler_config* sc, float* out);
 int vdt_ddim_invert_range(vdt_plan* plan, const vdt_sampler_config* sc, float* x, const void* label, int32_t batch,
                           int32_t first_step, int32_t num_steps, void* stream);
+/* Likelihood evaluation: the negative ELBO in bits per dimension (Ho et al., 2020, section 3.3; Nichol & Dhariwal, 2021,
+ * _vb_terms_bpd / calc_bpd_loop), on this library's time grid and coefficient table.  It follows that standard definition;
+ * it is not pinned to the reference's own likelihood code, which could not be compared.  For step i = 0 ... T-1 with
+ * s = i/T, t = (i+1)/T (the sampler's pair of step i) and x0 in model space ([-1, 1]):
+ *   - eps_i ~ N(0, I), fresh per step: noise[i] (injected, fp32 [T, B, C, R, R]) or else this library's Philox4x32-10 stream
+ *     keyed by sc->seed with counter word 3 = 2 (0 is the ancestral noise, 1 inpainting's z');
+ *   - x_t = alpha_t x0 + sigma_t eps_i (two fp32 products and a sum, rounded like vdt_q_sample); the model sees x_t at
+ *     fp64 time t, as p_sample's does;
+ *   - x0_hat from the raw output at lambda_t through the converters of every model_out_type, clipped to [-1, 1] iff
+ *     clip_denoised; mse_i = mean over C*H*W of (x0_hat - x0)^2 (fp32 products, per-tile sums in fp64);
+ *   - i > 0: term_i = KL(q(x_s | x_t, x0) || p(x_s | x_t)) / ln 2 as a mean over C*H*W.  Both are Gaussians with means
+ *     c1 x_t + c2 x0 and c1 x_t + c2 x0_hat (c1, c2 the ancestral posterior's), log-variances lv_q = fixed_small's and
+ *     lv_p = the configured model_var_type's, so term_i = K_i + k_i mse_i with K_i = (-1 + lv_p - lv_q + e^(lv_q - lv_p)) /
+ *     (2 ln 2) and k_i = c2^2 e^(-lv_p) / (2 ln 2) (K_i = 0 under fixed_small);
+ *   - i = 0: term_0 = -mean over C*H*W of log p(x0 | x0_hat) / ln 2 for the 8-bit discretized Gaussian decoder with
+ *     log-scale lv_p(row 0) / 2: bins of half-width 1/255, CDF 0.5 (1 + tanh(sqrt(2/pi) (u + 0.044715 u^3))), open edge
+ *     bins (x0 < -0.999: log CDF(plus); x0 > 0.999: log(1 - CDF(min))), every log clamped at 1e-12, in fp32.  Under
+ *     fixed_small lv_p(row 0) is about -20 on the +-20 cosine schedule, so the decoder is a near-delta and term_0 is large
+ *     unless x0_hat is within a bin of x0; IDDPM's clip of that variance is not reproduced;
+ *   - prior_bpd = mean over C*H*W of (-1 - lv_1 + e^(lv_1) + alpha_1^2 x0^2) / (2 ln 2), alpha_1^2 = sigmoid(l1),
+ *     lv_1 = logsigmoid(-l1), l1 = lambda(1) rounded to fp32;
+ *   - total_bpd = sum over i of term_i (in order, fp64) + prior_bpd (the Python layer adds them).
+ * Guidance plays no part (a guided model has no ELBO): labels condition the model, w_guide is ignored, as are use_ddim and
+ * solver.  Refused (vdt_last_error): x0eps_coef = 1, t_fp32 = 1, model_var_type outside the three fixed types, steps outside
+ * [0, T).
+ * vdt_bpd_coefficients: out [T][16] in the vdt_step_coefficients layout with use_ddim = 0 -- slots 0-5 and 12-13 the
+ * converters at lambda_t, 6-7 c1 and c2, 8-11 as in vdt_step_coefficients (9 = lv_p) -- with slot 14 = K_i and slot 15 = k_i
+ * in place of the x0eps flag and c2k, which this path never uses.  Row 0's K_0, k_0 are the formula's and unused.
+ * vdt_calc_bpd_range: x0 fp32 [B, C, R, R] (read only), label as for vdt_p_sample; fills columns first_step ...
+ * first_step + num_steps - 1 of terms and mse, fp64 [B, T].  Each step is independent of the others, and per-sample sums run
+ * over fixed tiles, so results are bit-identical however the range is split and the batch chunked.
+ * vdt_bpd_prior: out fp64 [B], x0 fp32 [B, chw]. */
+int vdt_bpd_coefficients(const vdt_sampler_config* sc, float* out);
+int vdt_calc_bpd_range(vdt_plan* plan, const vdt_sampler_config* sc, const float* x0, const void* label,
+                       const float* noise /* nullable, [T, B, C, R, R] */, int32_t clip_denoised, int32_t batch,
+                       int32_t first_step, int32_t num_steps, double* terms, double* mse, void* stream);
+int vdt_bpd_prior(const vdt_sampler_config* sc, const float* x0, int32_t batch, int32_t chw, double* out, void* stream);
 /* Same with HOST buffers (pinned or pageable); copies in/out inside the call and synchronises. */
 int vdt_p_sample_host(vdt_plan* plan, const vdt_sampler_config* sc, const float* noise, const void* label,
                       const float* step_noise, float* out, int32_t batch);
@@ -360,6 +397,12 @@ int vdt_op_sampler_step_known(const float* model_out, const float* x_t, const fl
  * alias x); model_out as for vdt_op_sampler_step; coef_host = one row of vdt_invert_coefficients (host). */
 int vdt_op_invert_step(const float* model_out, const float* x, float* x_next, int32_t batch, int32_t c, int32_t hw, int32_t cfg,
                        int32_t model_out_type, const float* coef_host, float w, void* stream);
+/* One step of vdt_calc_bpd_range for a generic denoise_fn: model_out fp32 [B, Cm, H, W] (no CFG rows) computed from x_t fp32
+ * [B, C, H, W], x0 fp32 [B, C, H, W]; coef_host = row `step` of vdt_bpd_coefficients (host).  Writes terms[b][step] and
+ * mse[b][step] of fp64 [B, num_steps] outputs.  Any 4-byte alignment. */
+int vdt_op_bpd_term(const float* model_out, const float* x_t, const float* x0, int32_t batch, int32_t c, int32_t hw,
+                    int32_t model_out_type, int32_t step, int32_t num_steps, const float* coef_host, int32_t clip_denoised,
+                    double* terms, double* mse, void* stream);
 
 #ifdef __cplusplus
 }

@@ -121,6 +121,10 @@ def lib():
     L.vdt_ddim_invert_range.argtypes = [vp, C.POINTER(SamplerConfig), vp, vp, i32, i32, i32, vp]
     L.vdt_invert_coefficients.argtypes = [C.POINTER(SamplerConfig), vp]
     L.vdt_op_invert_step.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, vp, C.c_float, vp]
+    L.vdt_bpd_coefficients.argtypes = [C.POINTER(SamplerConfig), vp]
+    L.vdt_calc_bpd_range.argtypes = [vp, C.POINTER(SamplerConfig), vp, vp, vp, i32, i32, i32, i32, vp, vp, vp]
+    L.vdt_bpd_prior.argtypes = [C.POINTER(SamplerConfig), vp, i32, i32, vp, vp]
+    L.vdt_op_bpd_term.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, i32, vp, vp, vp]
     L.vdt_plan_flops.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double)]
     L.vdt_profile_enable.argtypes = [C.c_int]
     L.vdt_profile_read.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_uint64)]
@@ -165,7 +169,8 @@ EXPORTS = ["vdt_last_error", "vdt_version", "vdt_kernel_launches", "vdt_plan_cre
            "vdt_plan_num_weights", "vdt_plan_weight_name", "vdt_plan_weight_shape", "vdt_plan_load_weight",
            "vdt_plan_finalize", "vdt_unet_forward", "vdt_p_sample", "vdt_p_sample_range", "vdt_p_sample_host",
            "vdt_p_sample_inpaint", "vdt_p_sample_range_inpaint", "vdt_p_sample_from", "vdt_ddim_invert_range",
-           "vdt_invert_coefficients", "vdt_op_invert_step",
+           "vdt_invert_coefficients", "vdt_op_invert_step", "vdt_bpd_coefficients", "vdt_calc_bpd_range", "vdt_bpd_prior",
+           "vdt_op_bpd_term",
            "vdt_step_coefficients", "vdt_plan_flops", "vdt_profile_enable", "vdt_profile_read",
            "vdt_op_conv", "vdt_op_conv_ex", "vdt_op_in_conv", "vdt_op_out_conv", "vdt_op_groupnorm", "vdt_op_attention", "vdt_op_sampler_step", "vdt_op_sampler_step_hist",
            "vdt_op_sampler_step_known",           "vdt_stat_slabs_per_image",

@@ -232,6 +232,12 @@ struct SamplerState {
     // first-order step when sampling starts at an intermediate time.  T-1 for a whole trajectory (where c2k is 0 already)
     // and for a range of one.  Kept last: coef must stay 16-byte aligned for the step kernel's float4 reads.
     int start_step;
+    // likelihood evaluation (vdt_calc_bpd_range; the fields above keep their offsets): 1 = x0 clipped to [-1, 1], and the
+    // caller's fp64 [Btotal, ld] outputs that the finalize writes at [img0 + b, step]
+    int bpd_clip;
+    int bpd_ld;
+    double* bpd_terms;
+    double* bpd_mse;
 };
 constexpr int kCoefStride = 16;
 // single-thread kernel: st->step = st->next_step--, copies the coefficient row (and slots 0, 1 of row step - 1 into
@@ -263,6 +269,27 @@ cudaError_t launch_sampler_step(const SamplerStepParams& p, cudaStream_t stream)
 // x_t = c1' x_s + c2' x0 with the unclipped (guided) x0 and the coefficient row in st->coef; pred_x0, x0eps and the state's
 // noise and inpainting fields are not read.
 cudaError_t launch_invert_step(const SamplerStepParams& p, cudaStream_t stream);
+
+// Likelihood evaluation (bpd.cu; include/vdt_b200.h vdt_calc_bpd_range).  One step i = st->step per launch, with the row of
+// vdt_bpd_coefficients in st->coef.  Per-sample sums run over fixed tiles of kBpdTile elements, so the result does not
+// depend on how a batch is chunked.
+constexpr int kBpdTile = 4096;
+inline int bpd_tiles(long long chw) { return static_cast<int>((chw + kBpdTile - 1) / kBpdTile); }
+struct BpdParams {
+    const float* x0;                   // fp32 [B, C, HW] data in model space
+    float* x_t;                        // fp32 [B, C, HW] the UNet input
+    const float* model_out;            // fp32 [B, Cm, HW]
+    double* partial;                   // [B, bpd_tiles(C*HW), 2] per-tile sums of (x0_hat - x0)^2 and the decoder log-likelihood
+    const SamplerState* st;
+    int B, C, HW;
+    int model_out_type;
+};
+// x_t = alpha_t x0 + sigma_t eps, eps = st->noise[step] (injected) or Philox stream 2 of st->seed
+cudaError_t launch_bpd_qsample(const BpdParams& p, cudaStream_t stream);
+// the per-tile sums, then the finalize: terms[img0 + b][step] and mse[img0 + b][step] through st->bpd_terms / bpd_mse
+cudaError_t launch_bpd_term(const BpdParams& p, cudaStream_t stream);
+// out[b] = c0 + c1 * mean over C*HW of x0^2 (fp64), fixed-order per-sample sums
+cudaError_t launch_bpd_prior(const float* x0, int B, int chw, double c0, double c1, double* out, cudaStream_t stream);
 
 // ------------------------------------------------------------------------------------------------
 // Training-step kernels (train.cu): GaussianDiffusion.train_loss around the model call (diffusion.py:492-545)

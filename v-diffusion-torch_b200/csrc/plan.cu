@@ -229,6 +229,12 @@ __global__ void sampler_init_state_kernel(SamplerState* st, int next_step, int s
         st->known = inp.known; st->mask = inp.mask; st->known_noise = inp.known_noise;
     }
 }
+// the per-call fields of a likelihood evaluation, written after sampler_init_state_kernel
+__global__ void bpd_init_state_kernel(SamplerState* st, double* terms, double* mse, int ld, int clip) {
+    if (threadIdx.x == 0 && blockIdx.x == 0) {
+        st->bpd_terms = terms; st->bpd_mse = mse; st->bpd_ld = ld; st->bpd_clip = clip;
+    }
+}
 __global__ void set_u64_kernel(unsigned long long* p, unsigned long long v) {
     if (threadIdx.x == 0 && blockIdx.x == 0) *p = v;
 }
@@ -261,7 +267,7 @@ struct Block {
 };
 
 enum StepKind { S_CONV, S_GN, S_ATTN, S_IM2COL, S_TEMB, S_LINEAR, S_CLSEMB, S_BEGIN, S_SAMPLE, S_ATTN_F32, S_TAPSUM, S_BEGIN_INV,
-                S_INVERT };
+                S_INVERT, S_BPD_QSAMPLE, S_BPD_TERM };
 struct TapsumArgs { const float* y; const float* bias; float* out; int B, H, W, Cout, ld; };
 struct LinearArgs { const float *x, *W, *b; float* out; int rows, K, N, silu; };
 struct Im2colArgs { const float* x; h16* out; h16* out_lo; int B, rep, C, H, W, f16; };
@@ -292,6 +298,7 @@ struct Exec {
     std::vector<BeginArgs> begins;
     std::vector<TapsumArgs> tapsums;
     std::vector<SamplerStepParams> samples;
+    std::vector<BpdParams> bpds;
     // fixed I/O staging
     float* xin = nullptr;        // forward: fp32 NCHW [rows, Cin, HW] | sampler: x_t [rows/rep, C, HW]
     float* yout = nullptr;       // fp32 NCHW [rows, Cout, HW]
@@ -303,6 +310,7 @@ struct Exec {
     unsigned long long* drop_seed = nullptr;   // training forward: seed of this call's dropout masks (device word read by the graph)
     float drop_p = 0.f;
     float* pred = nullptr;       // sampler: (guided) x0 prediction of the last executed step [rows/rep, C, HW]
+    float* x0 = nullptr;         // likelihood evaluation: the chunk's data [rows, C, HW] (xin holds x_t)
     float* coef_table = nullptr; // [T][kCoefStride] (sampler)
     // sampler signature this exec was built for
     vdt_sampler_config sc{};
@@ -1219,6 +1227,8 @@ static int run_steps(vdt_plan* p, Exec* ex, cudaStream_t st, std::vector<cudaEve
             case S_SAMPLE: e = launch_sampler_step(ex->samples[s.idx], st); break;
             case S_BEGIN_INV: { auto& a = ex->begins[s.idx]; e = launch_invert_begin_step(a.st, a.table, a.t_rows, a.nrows, a.T, st); break; }
             case S_INVERT: e = launch_invert_step(ex->samples[s.idx], st); break;
+            case S_BPD_QSAMPLE: e = launch_bpd_qsample(ex->bpds[s.idx], st); break;
+            case S_BPD_TERM: e = launch_bpd_term(ex->bpds[s.idx], st); break;
             case S_TAPSUM: { auto& a = ex->tapsums[s.idx]; e = launch_tapsum3x3(a.y, a.bias, a.out, a.B, a.H, a.W, a.Cout, a.ld, st); break; }
             case S_ATTN_F32: { auto& a = ex->attn32s[s.idx]; e = launch_attention_f32(a.qkv, a.hi, a.lo, a.B, a.N, a.heads, a.d, a.f16, st); break; }
         }
@@ -1536,6 +1546,64 @@ extern "C" int vdt_invert_coefficients(const vdt_sampler_config* scp, float* out
     return 0;
 }
 
+// ================================================================================================ likelihood (bits/dim)
+// The bound runs the p_sample time grid (fp64 t) with the ancestral posterior; the sampler-only fields of the config
+// (use_ddim, solver, w_guide) play no part and are ignored.
+static int check_bpd(const vdt_sampler_config& sc) {
+    if (sc.sample_timesteps < 1) return fail("sample_timesteps must be >= 1");
+    if (sc.x0eps_coef)
+        return fail("the likelihood bound needs x0eps_coef = 0 (the reference's (eps, x0) posterior coefficients are another "
+                    "parameterisation of the mean, and under DDIM logarithms)");
+    if (sc.t_fp32) return fail("the likelihood bound runs the fp64 time grid of p_sample: t_fp32 must be 0");
+    if (sc.model_var_type < VDT_VAR_FIXED_SMALL || sc.model_var_type > VDT_VAR_FIXED_MEDIUM)
+        return fail("the likelihood bound needs a fixed model_var_type (0, 1 or 2), got %d", sc.model_var_type);
+    return 0;
+}
+
+static vdt_sampler_config bpd_config(const vdt_sampler_config& sc) {
+    vdt_sampler_config c = sc;
+    c.use_ddim = 0; c.solver = VDT_SOLVER_FIRST_ORDER; c.w_guide = 0.0;
+    return c;
+}
+
+// vdt_step_coefficients with use_ddim = 0, slots 14-15 replaced by K_i and k_i of term_i = K_i + k_i mse_i: the KL between
+// the true posterior (fixed_small's log-variance lv_q) and the model's (the configured lv_p) with means c2 apart per unit
+// of x0 error, in bits, fp64 from the fp32-rounded log-SNRs (slots 10, 11) and rounded once.
+extern "C" int vdt_bpd_coefficients(const vdt_sampler_config* scp, float* out) {
+    if (!scp || !out) return fail("null argument");
+    CKI(check_bpd(*scp));
+    const vdt_sampler_config sc = bpd_config(*scp);
+    CKI(vdt_step_coefficients(&sc, out));
+    const double ln2 = std::log(2.0);
+    for (int i = 0; i < sc.sample_timesteps; ++i) {
+        float* o = out + (size_t)i * kCoefStride;
+        const double ls = o[10], lt = o[11];
+        const double l1mr = log1mexp_d(lt - ls);
+        const double lo = l1mr + logsigmoid_d(-ls), hi = l1mr + logsigmoid_d(-lt);
+        const double lv_q = lo;
+        const double lv_p = sc.model_var_type == VDT_VAR_FIXED_SMALL ? lo
+                          : sc.model_var_type == VDT_VAR_FIXED_LARGE ? hi : lo + sc.intp_frac * (hi - lo);
+        const double c2 = std::exp(l1mr + 0.5 * logsigmoid_d(ls));
+        const double dlv = lv_p - lv_q;                  // -1 + dlv + e^(-dlv), written so that dlv = 0 gives exactly 0
+        o[14] = (float)(0.5 * (std::expm1(-dlv) + dlv) / ln2);
+        o[15] = (float)(0.5 * c2 * c2 * std::exp(-lv_p) / ln2);
+    }
+    return 0;
+}
+
+// prior_bpd = c0 + c1 mean(x0^2): KL(q(x_1 | x0) || N(0, I)) per dimension in bits, alpha_1^2 = sigmoid(l1),
+// lv_1 = logsigmoid(-l1) at the fp32-rounded l1 = lambda(1)
+static int bpd_prior_constants(const vdt_sampler_config& sc, double* c0, double* c1) {
+    double l1_d;
+    CKI(logsnr_d(sc, 1.0, &l1_d));
+    const double l1 = (float)l1_d;
+    const double ln2 = std::log(2.0);
+    const double lv1 = logsigmoid_d(-l1);
+    *c0 = 0.5 * (-1.0 - lv1 + std::exp(lv1)) / ln2;
+    *c1 = 0.5 * std::exp(logsigmoid_d(l1)) / ln2;
+    return 0;
+}
+
 // ================================================================================================ training step
 // Per-sample scalars of GaussianDiffusion.train_loss from the continuous times t (host, fp64): the log-SNR is evaluated in
 // fp64 and rounded to fp32 by broadcast_to (diffusion.py:23-26, 293-295); every derived scalar is then fp32 math on that
@@ -1605,15 +1673,20 @@ extern "C" int vdt_adamw_ema_step(float* param, const float* grad, float* exp_av
 }
 
 // ================================================================================================ sampler
-// invert: the DDIM inversion exec (ascending begin-step, invert_step_kernel, vdt_invert_coefficients), cached under its own key
-static int get_sampler_exec(vdt_plan* p, const vdt_sampler_config& sc, int imgs, bool has_label, int lane, bool invert, Exec** out) {
+// EX_INVERT: the DDIM inversion exec (ascending begin-step, invert_step_kernel, vdt_invert_coefficients); EX_BPD: the likelihood
+// exec (descending begin-step, q-sample of the exec's x0 before the UNet, the bound's terms after it, vdt_bpd_coefficients).
+// Each kind is cached under its own key.
+enum ExecKind { EX_SAMPLE, EX_INVERT, EX_BPD };
+static int get_sampler_exec(vdt_plan* p, const vdt_sampler_config& sc, int imgs, bool has_label, int lane, ExecKind kind,
+                            Exec** out) {
+    const bool invert = kind == EX_INVERT, bpd = kind == EX_BPD;
     const bool cfg = sc.w_guide > 0.0 && has_label;            // diffusion.py:368
     const int rep = cfg ? 2 : 1;
     // the key holds what shapes the workspace, the coefficient table and the kernel parameters baked into the graph;
     // per-call values (seed, injected-noise tensor, fp32-t mode of p_sample_progressive) live in the device-side
     // SamplerState and are rewritten before every call
     char key[208];
-    snprintf(key, sizeof(key), "%s%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%.17g:%.17g:%.17g:%.17g", invert ? "inv" : "smp", lane, imgs, (int)has_label,
+    snprintf(key, sizeof(key), "%s%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%d:%.17g:%.17g:%.17g:%.17g", invert ? "inv" : bpd ? "bpd" : "smp", lane, imgs, (int)has_label,
              sc.sample_timesteps, sc.model_out_type, sc.model_var_type, sc.logsnr_schedule, sc.use_ddim, sc.x0eps_coef, sc.t_fp32,
              sc.solver, sc.intp_frac, sc.logsnr_min, sc.logsnr_max, sc.w_guide);
     CKI(exec_cache_lookup(p, key, out));
@@ -1638,19 +1711,34 @@ static int get_sampler_exec(vdt_plan* p, const vdt_sampler_config& sc, int imgs,
     CKI(ex->acquire(ex->emb_rows * sizeof(int64_t), (void**)&ex->y_rows));
     CKI(ex->acquire(ex->rows * sizeof(int), (void**)&ex->film_row));
     CKI(ex->acquire(sizeof(SamplerState), (void**)&ex->state));
-    CKI(ex->acquire(imgs * HW * c.in_channels * 4, (void**)&ex->pred));
+    CKI(ex->acquire(imgs * HW * c.in_channels * 4, bpd ? (void**)&ex->x0 : (void**)&ex->pred));
     CKI(ex->acquire((size_t)T * kCoefStride * 4, (void**)&ex->coef_table));
     // on the plan's own stream: the legacy default stream does not order against a non-blocking stream
     iota_i64_kernel<<<(ex->emb_rows + 127) / 128, 128, 0, p->work>>>(ex->y_rows, ex->emb_rows);
     CK(cudaGetLastError());
     std::vector<float> coefs((size_t)T * kCoefStride);
-    CKI(invert ? vdt_invert_coefficients(&sc, coefs.data()) : vdt_step_coefficients(&sc, coefs.data()));
+    CKI(invert ? vdt_invert_coefficients(&sc, coefs.data()) : bpd ? vdt_bpd_coefficients(&sc, coefs.data())
+                                                                  : vdt_step_coefficients(&sc, coefs.data()));
     CK(cudaMemcpyAsync(ex->coef_table, coefs.data(), coefs.size() * 4, cudaMemcpyHostToDevice, p->work));
     CK(cudaStreamSynchronize(p->work));              // `coefs` is a host temporary
     float* film;
     CKI(ex->acquire((size_t)ex->emb_rows * p->film_total * 4, (void**)&film));
     ex->begins.push_back({ex->state, ex->coef_table, ex->t_rows, ex->emb_rows, T});
     ex->steps.push_back({invert ? S_BEGIN_INV : S_BEGIN, 0});
+    if (bpd) {
+        BpdParams bp{};
+        bp.x0 = ex->x0; bp.x_t = ex->xin; bp.model_out = ex->yout; bp.st = ex->state;
+        bp.B = imgs; bp.C = c.in_channels; bp.HW = (int)HW; bp.model_out_type = sc.model_out_type;
+        CKI(ex->acquire((size_t)imgs * bpd_tiles((long long)HW * c.in_channels) * 2 * sizeof(double), (void**)&bp.partial));
+        ex->bpds.push_back(bp);
+        ex->steps.push_back({S_BPD_QSAMPLE, 0});
+        CKI(add_embedding_steps(p, ex.get(), film, cond_model));
+        CKI(build_unet_steps(p, ex.get(), film, mt ? nullptr : ex->film_row));
+        ex->steps.push_back({S_BPD_TERM, 0});
+        *out = ex.get();
+        p->execs[key] = std::move(ex);
+        return 0;
+    }
     CKI(add_embedding_steps(p, ex.get(), film, cond_model));
     CKI(build_unet_steps(p, ex.get(), film, mt ? nullptr : ex->film_row));
     SamplerStepParams sp{};
@@ -1672,12 +1760,16 @@ static int check_inpaint(const float* known, const float* mask, const float* kno
     return 0;
 }
 
-// The chunk and lane loop shared by sampling and inversion; its callers check every argument first.  Sampling runs steps
-// first_step, first_step - 1, ... (num_steps of them) with `start_step` as the first step of the trajectory (see SamplerState);
-// inversion (invert) runs first_step, first_step + 1, ...
+// Per-call outputs of a likelihood evaluation (vdt_calc_bpd_range)
+struct BpdCall { double* terms; double* mse; int ld; int clip; };
+
+// The chunk and lane loop shared by sampling, inversion and the likelihood evaluation; its callers check every argument
+// first.  Sampling runs steps first_step, first_step - 1, ... (num_steps of them) with `start_step` as the first step of the
+// trajectory (see SamplerState); inversion (invert) runs first_step, first_step + 1, ...  With `bpd`, x is the data x0, read
+// only: each chunk's x0 goes to the exec, steps run downwards as in sampling and write their terms through the state.
 static int run_sampler_range(vdt_plan* p, const vdt_sampler_config& sc, const vdt_inpaint& inp, float* x, const void* label,
                              const float* step_noise, int32_t batch, int32_t first_step, int32_t num_steps, float* pred_x0,
-                             bool carry_pred, int start_step, bool invert, void* stream) {
+                             bool carry_pred, int start_step, bool invert, void* stream, const BpdCall* bpd = nullptr) {
     cudaStream_t user = reinterpret_cast<cudaStream_t>(stream);
     CKI(enter_work(p, user));
     cudaStream_t st = p->work;
@@ -1707,8 +1799,8 @@ static int run_sampler_range(vdt_plan* p, const vdt_sampler_config& sc, const vd
         const int lane = ci % lanes;
         st = lane ? p->lane_stream[lane] : p->work;
         Exec* ex;
-        CKI(get_sampler_exec(p, sc, imgs, label != nullptr, lane, invert, &ex));
-        CK(cudaMemcpyAsync(ex->xin, x + (size_t)i0 * CHW, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
+        CKI(get_sampler_exec(p, sc, imgs, label != nullptr, lane, bpd ? EX_BPD : invert ? EX_INVERT : EX_SAMPLE, &ex));
+        CK(cudaMemcpyAsync(bpd ? ex->x0 : ex->xin, x + (size_t)i0 * CHW, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
         if (carry_pred) CK(cudaMemcpyAsync(ex->pred, pred_x0 + (size_t)i0 * CHW, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
         if (mt) {
             const int n = ex->rows * c.num_classes;
@@ -1723,8 +1815,13 @@ static int run_sampler_range(vdt_plan* p, const vdt_sampler_config& sc, const vd
                                                     (long long)batch * (long long)CHW, (unsigned long long)sc.seed, inp);
         CK(cudaGetLastError());
         g_launches += 2;
+        if (bpd) {
+            bpd_init_state_kernel<<<1, 32, 0, st>>>(ex->state, bpd->terms, bpd->mse, bpd->ld, bpd->clip);
+            CK(cudaGetLastError());
+            ++g_launches;
+        }
         for (int step = 0; step < num_steps; ++step) CKI(run_exec(p, ex, st));
-        CK(cudaMemcpyAsync(x + (size_t)i0 * CHW, ex->xin, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
+        if (!bpd) CK(cudaMemcpyAsync(x + (size_t)i0 * CHW, ex->xin, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
         if (pred_x0 && num_steps > 0)
             CK(cudaMemcpyAsync(pred_x0 + (size_t)i0 * CHW, ex->pred, imgs * CHW * 4, cudaMemcpyDeviceToDevice, st));
     }
@@ -1789,6 +1886,37 @@ extern "C" int vdt_ddim_invert_range(vdt_plan* p, const vdt_sampler_config* scp,
     CKI(check_plan_for_sampler(p, sc));
     const vdt_inpaint none{nullptr, nullptr, nullptr};
     return run_sampler_range(p, sc, none, x, label, nullptr, batch, first_step, num_steps, nullptr, false, T - 1, true, stream);
+}
+
+extern "C" int vdt_calc_bpd_range(vdt_plan* p, const vdt_sampler_config* scp, const float* x0, const void* label,
+                                  const float* noise, int32_t clip_denoised, int32_t batch, int32_t first_step, int32_t num_steps,
+                                  double* terms, double* mse, void* stream) {
+    if (!p || !scp || !x0 || !terms || !mse) return fail("null argument");
+    CKI(check_bpd(*scp));
+    const vdt_sampler_config sc = bpd_config(*scp);
+    const int T = sc.sample_timesteps;
+    if (batch < 0) return fail("batch must be >= 0 (got %d)", batch);
+    if (first_step < 0 || first_step >= T || num_steps < 0 || num_steps > T - first_step)
+        return fail("bound steps [%d, %d + %d) leave [0, %d)", first_step, first_step, num_steps, T);
+    CKI(check_plan_for_sampler(p, sc));
+    const vdt_inpaint none{nullptr, nullptr, nullptr};
+    const BpdCall call{terms, mse, T, clip_denoised ? 1 : 0};
+    // steps first_step + num_steps - 1 ... first_step (each is independent of the others); start_step -1 keeps slot 15 (k_i),
+    // which the sampler's begin-step zeroes at the first step of a trajectory; x0 is only read
+    return run_sampler_range(p, sc, none, const_cast<float*>(x0), label, noise, batch, first_step + num_steps - 1, num_steps,
+                             nullptr, false, -1, false, stream, &call);
+}
+
+extern "C" int vdt_bpd_prior(const vdt_sampler_config* scp, const float* x0, int32_t batch, int32_t chw, double* out, void* stream) {
+    if (!scp || !x0 || !out) return fail("null argument");
+    CKI(check_bpd(*scp));
+    if (batch < 0 || chw < 1) return fail("bad image shape (%d, %d)", batch, chw);
+    double c0, c1;
+    CKI(bpd_prior_constants(*scp, &c0, &c1));
+    cudaError_t e = launch_bpd_prior(x0, batch, chw, c0, c1, out, reinterpret_cast<cudaStream_t>(stream));
+    ++g_launches;
+    if (e != cudaSuccess) return fail("bpd_prior launch failed: %s", cudaGetErrorString(e));
+    return 0;
 }
 
 extern "C" int vdt_p_sample_range(vdt_plan* p, const vdt_sampler_config* scp, float* x, const void* label,
@@ -2323,6 +2451,38 @@ extern "C" int vdt_op_invert_step(const float* model_out, const float* x, float*
     cudaFree(ds);
     if (e != cudaSuccess) return fail("invert_step launch failed: %s", cudaGetErrorString(e));
     if (e2 != cudaSuccess) return fail("invert_step failed: %s", cudaGetErrorString(e2));
+    return 0;
+}
+
+extern "C" int vdt_op_bpd_term(const float* model_out, const float* x_t, const float* x0, int32_t batch, int32_t c, int32_t hw,
+                               int32_t model_out_type, int32_t step, int32_t num_steps, const float* coef_host,
+                               int32_t clip_denoised, double* terms, double* mse, void* stream) {
+    if (!model_out || !x_t || !x0 || !coef_host || !terms || !mse) return fail("null argument");
+    if (model_out_type < 0 || model_out_type > 3) return fail("unknown model_out_type %d", model_out_type);
+    if (batch < 0 || c < 1 || hw < 1) return fail("bad image shape (%d, %d, %d)", batch, c, hw);
+    if (step < 0 || step >= num_steps) return fail("step %d lies outside [0, %d)", step, num_steps);
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    SamplerState hs{};
+    for (int i = 0; i < kCoefStride; ++i) hs.coef[i] = coef_host[i];
+    hs.step = step; hs.bpd_clip = clip_denoised ? 1 : 0; hs.bpd_ld = num_steps; hs.bpd_terms = terms; hs.bpd_mse = mse;
+    SamplerState* ds = nullptr;
+    double* partial = nullptr;
+    CK(cudaMalloc(&ds, sizeof(SamplerState)));
+    cudaError_t e = cudaMalloc(&partial, (size_t)std::max(batch, 1) * bpd_tiles((long long)c * hw) * 2 * sizeof(double));
+    if (e != cudaSuccess) { cudaFree(ds); return fail("cudaMalloc failed: %s", cudaGetErrorString(e)); }
+    e = cudaMemcpy(ds, &hs, sizeof(hs), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) {
+        BpdParams bp{};
+        bp.x0 = x0; bp.x_t = const_cast<float*>(x_t); bp.model_out = model_out; bp.partial = partial; bp.st = ds;
+        bp.B = batch; bp.C = c; bp.HW = hw; bp.model_out_type = model_out_type;
+        e = launch_bpd_term(bp, st);
+        g_launches += 2;
+    }
+    cudaError_t e2 = cudaStreamSynchronize(st);
+    cudaFree(partial);
+    cudaFree(ds);
+    if (e != cudaSuccess) return fail("bpd_term launch failed: %s", cudaGetErrorString(e));
+    if (e2 != cudaSuccess) return fail("bpd_term failed: %s", cudaGetErrorString(e2));
     return 0;
 }
 

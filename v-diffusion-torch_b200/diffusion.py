@@ -376,6 +376,94 @@ class GaussianDiffusion:
                 x = x_next
         return x.cpu()
 
+    # ------------------------------------------------------------------ likelihood in bits/dim (extension)
+    def _check_bpd(self):
+        if self.x0eps_coef:
+            raise NotImplementedError("the likelihood bound needs x0eps_coef=False (the reference's (eps, x0) posterior "
+                                      "coefficients are another parameterisation of the mean, and under DDIM logarithms)")
+        if self.model_var_type not in _lib.VAR_TYPES:
+            raise NotImplementedError(f"the likelihood bound needs a fixed model_var_type, got {self.model_var_type!r}")
+
+    def bpd_coefficients(self):
+        """[T, 16] fp32 host table of the likelihood bound (include/vdt_b200.h: vdt_bpd_coefficients): the ancestral row of
+        step i with slot 14 = K_i and slot 15 = k_i, term_i = K_i + k_i mse_i for i > 0."""
+        self._check_bpd()
+        sc = self.sampler_config(False)
+        out = torch.empty((self.sample_timesteps, _lib.COEF_STRIDE), dtype=torch.float32)
+        _lib.check(_lib.lib().vdt_bpd_coefficients(C.byref(sc), _lib.ptr(out)))
+        return out
+
+    @torch.no_grad()
+    def calc_all_bpd(self, denoise_fn, x_0, y=None, clip_denoised=True, device="cuda", seed=None, noise=None):
+        """Negative ELBO in bits per dimension of the images ``x_0`` (model space [-1, 1], (B, C, R, R)), the standard
+        variational bound of Ho et al. (2020, section 3.3) as Nichol & Dhariwal's calc_bpd_loop computes it, on this
+        library's time grid t = (i+1)/T and coefficient table.  The definition is written out in include/vdt_b200.h
+        (vdt_calc_bpd_range); it is not pinned to the reference's own likelihood code, and the name and return layout follow
+        the reference family without its exact signature having been checked.
+
+        Returns ``(total_bpd [B], terms_bpd [B, T], prior_bpd [B], mse [B, T])``, fp64 on the CPU: term i is the KL of step i
+        (i > 0) or the 8-bit decoder's negative log-likelihood (i = 0), mse[:, i] the mean squared error of the (clipped iff
+        ``clip_denoised``) x0 prediction, and total = terms.sum(1) + prior.  ``y``: labels as in p_sample; guidance plays no
+        part.  The q-sample draws eps_i come from ``noise`` ((T, B, C, R, R), indexed by step) or else from a stream keyed by
+        ``seed`` (a fresh seed when None): the library's own on the fused path (the UNet), a torch generator for any other
+        callable, which runs one step at a time through vdt_op_bpd_term."""
+        self._check_bpd()
+        T = self.sample_timesteps
+        device = torch.device(device)
+        if device.type != "cuda":
+            raise RuntimeError("v_diffusion_b200 evaluates on CUDA (sm_100a) only; there is no CPU fallback")
+        if device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        x0 = x_0.to(device=device, dtype=torch.float32).contiguous()
+        if x0.ndim != 4 or x0.shape[2] != x0.shape[3]:
+            raise ValueError(f"x_0 must have shape (B, C, R, R), got {tuple(x0.shape)}")
+        B, Cc, R = x0.shape[0], x0.shape[1], x0.shape[2]
+        if noise is not None:
+            noise = noise.to(device=device, dtype=torch.float32).contiguous()
+            if tuple(noise.shape) != (T,) + tuple(x0.shape):
+                raise ValueError(f"noise has shape {tuple(noise.shape)}, expected {(T,) + tuple(x0.shape)}")
+        if B == 0:
+            return (torch.zeros(0, dtype=torch.float64), torch.zeros((0, T), dtype=torch.float64),
+                    torch.zeros(0, dtype=torch.float64), torch.zeros((0, T), dtype=torch.float64))
+        flags = [torch.isfinite(x0).all()] + ([torch.isfinite(noise).all()] if noise is not None else [])
+        ok = torch.stack(flags).tolist()
+        if not ok[0]:
+            raise ValueError("x_0 must be finite")
+        if noise is not None and not ok[1]:
+            raise ValueError("noise must be finite")
+        label = self._prepare_label(denoise_fn, y, B, device)
+        sc = self.sampler_config(False, self._noise_seed(seed) if noise is None else seed)
+        terms = torch.empty((B, T), dtype=torch.float64, device=device)
+        mse = torch.empty((B, T), dtype=torch.float64, device=device)
+        prior = torch.empty((B,), dtype=torch.float64, device=device)
+        chw, clip = Cc * R * R, int(bool(clip_denoised))
+        L = _lib.lib()
+        with torch.cuda.device(device):
+            _lib.check(L.vdt_bpd_prior(C.byref(sc), _lib.ptr(x0), B, chw, _lib.ptr(prior), _lib.current_stream_ptr()))
+            if isinstance(denoise_fn, UNet):
+                plan = denoise_fn.plan_for(R, device)
+                _lib.check(L.vdt_calc_bpd_range(plan, C.byref(sc), _lib.ptr(x0), _lib.ptr(label), _lib.ptr(noise), clip, B, 0, T,
+                                                _lib.ptr(terms), _lib.ptr(mse), _lib.current_stream_ptr()))
+            else:
+                coefs = self.bpd_coefficients()
+                coef_dev = coefs.to(device)
+                gen = torch.Generator(device).manual_seed(sc.seed) if noise is None else None
+                want = (B, (2 if self.model_out_type == "both" else 1) * Cc, R, R)
+                for i in reversed(range(T)):                   # the fused path's order (and the generator's)
+                    eps = noise[i] if noise is not None else torch.randn(tuple(x0.shape), device=device, generator=gen)
+                    x_t = torch.empty_like(x0)
+                    _lib.check(L.vdt_q_sample(_lib.ptr(x0), _lib.ptr(eps), _lib.ptr(coef_dev[i].expand(B, -1).contiguous()),
+                                              _lib.ptr(x_t), B, chw, _lib.current_stream_ptr()))
+                    t = torch.full((B,), (i + 1) / T, dtype=torch.float64, device=device)
+                    out = denoise_fn(x_t, t, label).to(torch.float32).contiguous()
+                    if tuple(out.shape) != want:
+                        raise ValueError(f"model output has shape {tuple(out.shape)}, expected {want}")
+                    _lib.check(L.vdt_op_bpd_term(_lib.ptr(out), _lib.ptr(x_t), _lib.ptr(x0), B, Cc, R * R, sc.model_out_type, i, T,
+                                                 _lib.ptr(coefs[i].contiguous()), clip, _lib.ptr(terms), _lib.ptr(mse),
+                                                 _lib.current_stream_ptr()))
+        terms, mse, prior = terms.cpu(), mse.cpu(), prior.cpu()
+        return terms.sum(dim=1) + prior, terms, prior, mse
+
     # ------------------------------------------------------------------ train_loss (diffusion.py:492-545)
     @torch.no_grad()
     def train_loss(self, denoise_fn, x_0, t, y, noise=None, return_grad=False):
