@@ -367,6 +367,28 @@ int vdt_op_linear(const float* x, const float* w, const float* b, float* out, in
                   int32_t silu_out, void* stream);
 /* get_timestep_embedding(t, dim) (functions.py:10-29) for fp64 t [rows] -> fp32 [rows, dim] (sin | cos halves). */
 int vdt_op_timestep_embedding(const double* t, float* out, int32_t rows, int32_t dim, void* stream);
+/* The conditioning path one kernel at a time, as the plan launches it (refused before any CUDA call: null pointers, shapes
+ * outside the ranges below, element counts past 2^31 - 1).
+ * vdt_op_timestep_embedding_ex: the same with the plan's fp32-t switch (vdt_sampler_config.t_fp32): fp32_t = 1 rounds every
+ *   op of functions.py:20-25 to fp32, as p_sample_progressive's fp32 step tensor does; 0 is vdt_op_timestep_embedding.
+ * vdt_op_class_embed: out [rows, E] = SiLU(e + class term) with e [rows, E] (the time MLP's output), w [E, num_classes],
+ *   b [E]; exactly one label form: y int64 [rows] (OneHot(exclude_zero=True) + Linear: id c in 1..num_classes adds
+ *   b + w[:, c-1], id 0 adds b; ids below 0 add b and ids above num_classes are clamped to num_classes) or y_multihot fp32
+ *   [rows, num_classes] (adds w y / sqrt(max(1, nonzeros of y)) + b, unet.py:290-294).
+ * vdt_op_film_rows: the sampler's FiLM-table row per UNet row: out int32 [rows], row i reads label[i / rep], except that the
+ *   odd rows of rep = 2 (CFG's unconditional half) and a NULL label give 0; ids are clamped to [0, ncls].
+ * vdt_op_multitag_rows: its multitag twin: out fp32 [rows, ncls] = label[i / rep] (fp32 [rows / rep, ncls]), odd rows of
+ *   rep = 2 all zero.
+ * vdt_op_attention_f32: the split-precision mode's attention (operand_dtype 2), fp32 on CUDA cores: qkv fp32 [B*N, 3*hid]
+ *   in vdt_op_attention's layout, d in {64, 128, 192, 256} -> out_hi 16-bit [B*N, hid] = round16(o), out_lo 16-bit =
+ *   round16(o - out_hi). */
+int vdt_op_timestep_embedding_ex(const double* t, float* out, int32_t rows, int32_t dim, int32_t fp32_t, void* stream);
+int vdt_op_class_embed(const float* e, const int64_t* y, const float* y_multihot, const float* w, const float* b,
+                       int32_t num_classes, float* out, int32_t rows, int32_t E, void* stream);
+int vdt_op_film_rows(const int64_t* label, int32_t rows, int32_t rep, int32_t ncls, int32_t* out, void* stream);
+int vdt_op_multitag_rows(const float* label, int32_t rows, int32_t rep, int32_t ncls, float* out, void* stream);
+int vdt_op_attention_f32(const float* qkv, void* out_hi, void* out_lo, int32_t batch, int32_t n, int32_t heads, int32_t d,
+                         int32_t f16, void* stream);
 /* attention on qkv 16-bit [B*N, 3*hid] (q | k | v thirds, heads contiguous inside each, the layout proj_in writes)
  * -> 16-bit [B*N, hid]; any N >= 1 (ragged last key / query tiles are masked) */
 int vdt_op_attention(const void* qkv_16, void* out_16, int32_t batch, int32_t n, int32_t heads,

@@ -161,6 +161,11 @@ def lib():
     L.vdt_op_groupnorm_train.argtypes = [vp, i32, i32, i32, i32, vp, vp, vp, i32, i32, i32, vp, i32, C.c_float, C.c_uint64, i32, vp]
     L.vdt_op_linear.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, vp]
     L.vdt_op_timestep_embedding.argtypes = [vp, vp, i32, i32, vp]
+    L.vdt_op_timestep_embedding_ex.argtypes = [vp, vp, i32, i32, i32, vp]
+    L.vdt_op_class_embed.argtypes = [vp, vp, vp, vp, vp, i32, vp, i32, i32, vp]
+    L.vdt_op_film_rows.argtypes = [vp, i32, i32, i32, vp, vp]
+    L.vdt_op_multitag_rows.argtypes = [vp, i32, i32, i32, vp, vp]
+    L.vdt_op_attention_f32.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, vp]
     _lib = L
     return L
 
@@ -178,7 +183,9 @@ EXPORTS = ["vdt_last_error", "vdt_version", "vdt_kernel_launches", "vdt_plan_cre
            "vdt_train_coefficients", "vdt_q_sample", "vdt_train_loss", "vdt_unet_forward_train", "vdt_op_groupnorm_dropout",
            "vdt_op_conv_dgrad", "vdt_op_conv_wgrad", "vdt_op_groupnorm_backward",
            "vdt_plan_conv_flops_executed", "vdt_grad_sq_scratch_bytes", "vdt_grad_sq_accumulate", "vdt_adamw_ema_step",
-           "vdt_op_attention_backward", "vdt_op_groupnorm_train", "vdt_op_linear", "vdt_op_timestep_embedding"]
+           "vdt_op_attention_backward", "vdt_op_groupnorm_train", "vdt_op_linear", "vdt_op_timestep_embedding",
+           "vdt_op_timestep_embedding_ex", "vdt_op_class_embed", "vdt_op_film_rows", "vdt_op_multitag_rows",
+           "vdt_op_attention_f32"]
 
 
 def check(rc):

@@ -2523,11 +2523,88 @@ extern "C" int vdt_op_linear(const float* x, const float* W, const float* b, flo
 }
 
 // get_timestep_embedding(t, dim) (functions.py:20-25) for fp64 t: sin | cos halves of 1000 t exp(-k log(1e4) / (dim/2 - 1)).
-extern "C" int vdt_op_timestep_embedding(const double* t, float* out, int32_t rows, int32_t dim, void* stream) {
+static int check_embedding_shape(const double* t, const float* out, int32_t rows, int32_t dim) {
     if (!t || !out) return fail("null argument");
     if (rows < 0 || dim < 4) return fail("bad embedding shape (%d, %d)", rows, dim);
+    if ((int64_t)rows * dim > INT32_MAX) return fail("embedding of %d x %d elements exceeds 2^31 - 1", rows, dim);
+    return 0;
+}
+
+extern "C" int vdt_op_timestep_embedding(const double* t, float* out, int32_t rows, int32_t dim, void* stream) {
+    CKI(check_embedding_shape(t, out, rows, dim));
     cudaError_t e = launch_timestep_embedding(t, out, rows, dim, nullptr, reinterpret_cast<cudaStream_t>(stream));
     ++g_launches;
     if (e != cudaSuccess) return fail("timestep embedding launch failed: %s", cudaGetErrorString(e));
+    return 0;
+}
+
+// ---- kernel-level hooks of the conditioning path: (t, y) -> FiLM table, and the validation mode's fp32 attention ------------
+// The sampler reads the fp32-t flag from its device state (SamplerState::t_fp32); here it sits in a device int of its own.
+extern "C" int vdt_op_timestep_embedding_ex(const double* t, float* out, int32_t rows, int32_t dim, int32_t fp32_t, void* stream) {
+    CKI(check_embedding_shape(t, out, rows, dim));
+    if (fp32_t != 0 && fp32_t != 1) return fail("fp32_t must be 0 or 1 (got %d)", fp32_t);
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    int* flag = nullptr;
+    CK(cudaMalloc(&flag, sizeof(int)));
+    cudaError_t e = cudaMemcpy(flag, &fp32_t, sizeof(int), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) {
+        e = launch_timestep_embedding(t, out, rows, dim, flag, st);
+        ++g_launches;
+    }
+    cudaError_t e2 = cudaStreamSynchronize(st);
+    cudaFree(flag);
+    if (e != cudaSuccess) return fail("timestep embedding launch failed: %s", cudaGetErrorString(e));
+    if (e2 != cudaSuccess) return fail("timestep embedding failed: %s", cudaGetErrorString(e2));
+    return 0;
+}
+
+extern "C" int vdt_op_class_embed(const float* e, const int64_t* y, const float* y_multihot, const float* w, const float* b,
+                                  int32_t num_classes, float* out, int32_t rows, int32_t E, void* stream) {
+    if (!e || !w || !b || !out) return fail("null argument");
+    if ((y != nullptr) == (y_multihot != nullptr)) return fail("give exactly one of y (int64 ids) and y_multihot (fp32 rows)");
+    if (rows < 0 || E < 1 || num_classes < 1) return fail("bad class embedding shape (%d, %d, %d classes)", rows, E, num_classes);
+    if ((int64_t)rows * E > INT32_MAX) return fail("class embedding of %d x %d elements exceeds 2^31 - 1", rows, E);
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    cudaError_t err = y_multihot ? launch_class_embed_multitag_silu(e, y_multihot, w, b, num_classes, out, rows, E, st)
+                                 : launch_class_embed_silu(e, y, w, b, num_classes, out, rows, E, st);
+    ++g_launches;
+    if (err != cudaSuccess) return fail("class embedding launch failed: %s", cudaGetErrorString(err));
+    return 0;
+}
+
+extern "C" int vdt_op_film_rows(const int64_t* label, int32_t rows, int32_t rep, int32_t ncls, int32_t* out, void* stream) {
+    if (!out) return fail("null argument");
+    if (rows < 0 || ncls < 0) return fail("bad FiLM row shape (%d rows, %d classes)", rows, ncls);
+    if (rep != 1 && rep != 2) return fail("rep must be 1 or 2 (got %d)", rep);
+    if (rows == 0) return 0;
+    film_rows_kernel<<<(rows + 127) / 128, 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(label, out, rows, rep, ncls);
+    ++g_launches;
+    CK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int vdt_op_multitag_rows(const float* label, int32_t rows, int32_t rep, int32_t ncls, float* out, void* stream) {
+    if (!label || !out) return fail("null argument");
+    if (rows < 0 || ncls < 1) return fail("bad multitag row shape (%d rows, %d classes)", rows, ncls);
+    if (rep != 1 && rep != 2) return fail("rep must be 1 or 2 (got %d)", rep);
+    if ((int64_t)rows * ncls > INT32_MAX) return fail("multitag rows of %d x %d elements exceed 2^31 - 1", rows, ncls);
+    const int n = rows * ncls;
+    if (n == 0) return 0;
+    multitag_rows_kernel<<<(n + 127) / 128, 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(label, out, rows, rep, ncls);
+    ++g_launches;
+    CK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int vdt_op_attention_f32(const float* qkv, void* out_hi, void* out_lo, int32_t batch, int32_t n, int32_t heads, int32_t d,
+                                    int32_t f16, void* stream) {
+    if (!qkv || !out_hi || !out_lo) return fail("null argument");
+    if (batch < 1 || n < 1 || heads < 1) return fail("empty input (%d x %d, %d heads)", batch, n, heads);
+    if (d != 64 && d != 128 && d != 192 && d != 256) return fail("fp32 attention takes head dims 64, 128, 192 or 256 (got %d)", d);
+    if (f16 != 0 && f16 != 1) return fail("f16 must be 0 or 1 (got %d)", f16);
+    if ((int64_t)batch * n * heads > (int64_t)INT32_MAX * 8) return fail("%d x %d x %d query rows exceed one grid", batch, n, heads);
+    cudaError_t e = launch_attention_f32(qkv, (h16*)out_hi, (h16*)out_lo, batch, n, heads, d, f16, reinterpret_cast<cudaStream_t>(stream));
+    ++g_launches;
+    if (e != cudaSuccess) return fail("fp32 attention launch failed: %s", cudaGetErrorString(e));
     return 0;
 }

@@ -163,7 +163,10 @@ __global__ void class_embed_silu_kernel(const float* __restrict__ e, const int64
     const int r = idx / E, j = idx % E;
     float v = e[idx];
     if (y != nullptr) {
-        const long long cls = y[r];
+        // ids above num_classes are clamped like film_rows_kernel's (plan.cu), so that a C caller's label never reads past
+        // w_cls; ids <= 0 add the bias only
+        const long long id = y[r];
+        const long long cls = id > num_classes ? num_classes : id;
         float add = b_cls[j];
         if (cls > 0) add += w_cls[static_cast<size_t>(j) * num_classes + (cls - 1)];
         v += add;
