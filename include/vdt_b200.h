@@ -221,6 +221,40 @@ int vdt_train_loss(const float* model_out, const float* x0, const float* noise, 
                    float* loss, float* grad_out, int32_t batch, int32_t c, int32_t hw, int32_t model_out_type,
                    int32_t reweight_type, void* stream);
 
+/* ---- progressive distillation (Salimans & Ho, 2022, Algorithm 2) ------------------------------------------------------
+ * A student sampled with N DDIM steps learns to match a teacher with 2N.  Per sample a step index i in [0, N) gives the times
+ * t = (i+1)/N, t' = (2i+1)/(2N), t'' = i/N (fp64: the sampler's (t, s) grid at N and at 2N) and z_t = alpha_t x + sigma_t eps.
+ * The teacher takes two DDIM steps t -> t' -> t'', each the fused sampler's DDIM step with this sample's coefficients:
+ *   x1 = the guided x0 at t (per branch clipped to [-1, 1], then x0c + w (x0c - x0u); rows 2b conditional, 2b+1
+ *   unconditional), z_t' = c1 z_t + c2 x1; x2 = the same at t' from z_t', z_t'' = c1' z_t' + c2' x2 (= x2 when t'' = 0).
+ * Algorithm 2's target x~ = (z_t'' - (sigma_t''/sigma_t) z_t) / (alpha_t'' - (sigma_t''/sigma_t) alpha_t), the x0 with which one
+ * student DDIM step from z_t lands on z_t''.  Substituting the two steps, z_t cancels exactly:
+ *   z_t'' = (sigma_t''/sigma_t) z_t + sigma_t'' (alpha_t'/sigma_t' - alpha_t/sigma_t) x1 + (alpha_t'' - sigma_t'' alpha_t'/sigma_t') x2,
+ * and with alpha/sigma = e^(l/2) (l = log-SNR) and every term divided by alpha_t'':
+ *   x~ = c_a x1 + c_b x2,  c_b = expm1((l_t' - l_t'')/2) / expm1((l_t - l_t'')/2),
+ *                          c_a = 1 - c_b = e^((l_t' - l_t'')/2) expm1((l_t - l_t')/2) / expm1((l_t - l_t'')/2),
+ * both in [0, 1] since l_t < l_t' < l_t''.  At t'' = 0 the student's own last step returns its x0, so c_a = 0, c_b = 1.
+ * The form never subtracts nearly equal z's, so the low-SNR end (sigma_t''/sigma_t -> 1) stays well conditioned.  The student
+ * loss is vdt_train_loss unchanged with x0 := x~, noise := eps~ = z_t / sigma_t - x~ alpha_t / sigma_t, x_t := z_t and plane 0
+ * below as its table, so every model_out_type and reweight_type works as in training.
+ * vdt_distill_coefficients: sc->sample_timesteps is the student's N; only it, x0eps_coef and the schedule fields are read.
+ * step_host HOST int32 [B]; out HOST [2][B][16]:
+ *   plane 0 (t):  vdt_train_coefficients at t bit for bit, with slots 6-7 = the DDIM c1, c2 of t -> t' (sampler row 2i+1 at
+ *                 2N).  It also serves vdt_q_sample and vdt_train_loss;
+ *   plane 1 (t'): vdt_train_coefficients at t', with slots 6-7 = c1, c2 of t' -> t'' (sampler row 2i at 2N; 0 and 1 when
+ *                 t'' = 0), 8-9 = c_a, c_b and 10 = l_t''.
+ * c_a, c_b are fp64 from the fp32-rounded log-SNRs, rounded once.  Refused (vdt_last_error): x0eps_coef = 1, N < 1, steps
+ * outside [0, N).
+ * vdt_op_distill_step: teacher_out fp32 [B*(1+cfg), Cm, H, W] at t, z_t fp32 [B, C, H, W] -> z_mid = z_t', x0_hat = x1.
+ * vdt_op_distill_target: teacher_out at t', z_mid, x0_hat, z_t -> x_target = x~, eps_target = eps~.
+ * coef_dev: the table above on the device (16-byte aligned).  Image tensors at any 4-byte alignment; asynchronous on stream. */
+int vdt_distill_coefficients(const vdt_sampler_config* sc, const int32_t* step_host, int32_t batch, float* out);
+int vdt_op_distill_step(const float* teacher_out, const float* z_t, float* z_mid, float* x0_hat, const float* coef_dev,
+                        int32_t batch, int32_t c, int32_t hw, int32_t cfg, int32_t model_out_type, float w, void* stream);
+int vdt_op_distill_target(const float* teacher_out, const float* z_mid, const float* x0_hat, const float* z_t, float* x_target,
+                          float* eps_target, const float* coef_dev, int32_t batch, int32_t c, int32_t hw, int32_t cfg,
+                          int32_t model_out_type, float w, void* stream);
+
 /* The tail of generate.py's batch loop (generate.py:149): fp32 NCHW samples -> uint8 NHWC pixels,
  * (x * 127.5 + 127.5).clamp(0, 255).to(uint8).permute(0, 2, 3, 1).  x fp32 [B, C, HW], out uint8 [B, HW, C]; device pointers. */
 int vdt_images_to_uint8(const float* x_nchw, uint8_t* out_nhwc, int32_t batch, int32_t c, int32_t hw, void* stream);

@@ -156,6 +156,9 @@ def lib():
     L.vdt_train_coefficients.argtypes = [C.POINTER(SamplerConfig), vp, i32, vp]
     L.vdt_q_sample.argtypes = [vp, vp, vp, vp, i32, i32, vp]
     L.vdt_train_loss.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
+    L.vdt_distill_coefficients.argtypes = [C.POINTER(SamplerConfig), vp, i32, vp]
+    L.vdt_op_distill_step.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, C.c_float, vp]
+    L.vdt_op_distill_target.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, C.c_float, vp]
     L.vdt_images_to_uint8.argtypes = [vp, vp, i32, i32, i32, vp]
     L.vdt_plan_saturations.argtypes = [vp, C.POINTER(C.c_uint64), C.c_int]
     L.vdt_op_groupnorm_train.argtypes = [vp, i32, i32, i32, i32, vp, vp, vp, i32, i32, i32, vp, i32, C.c_float, C.c_uint64, i32, vp]
@@ -180,7 +183,8 @@ EXPORTS = ["vdt_last_error", "vdt_version", "vdt_kernel_launches", "vdt_plan_cre
            "vdt_op_conv", "vdt_op_conv_ex", "vdt_op_in_conv", "vdt_op_out_conv", "vdt_op_groupnorm", "vdt_op_attention", "vdt_op_sampler_step", "vdt_op_sampler_step_hist",
            "vdt_op_sampler_step_known",           "vdt_stat_slabs_per_image",
            "vdt_plan_saturations", "vdt_images_to_uint8",
-           "vdt_train_coefficients", "vdt_q_sample", "vdt_train_loss", "vdt_unet_forward_train", "vdt_op_groupnorm_dropout",
+           "vdt_train_coefficients", "vdt_q_sample", "vdt_train_loss", "vdt_distill_coefficients", "vdt_op_distill_step",
+           "vdt_op_distill_target", "vdt_unet_forward_train", "vdt_op_groupnorm_dropout",
            "vdt_op_conv_dgrad", "vdt_op_conv_wgrad", "vdt_op_groupnorm_backward",
            "vdt_plan_conv_flops_executed", "vdt_grad_sq_scratch_bytes", "vdt_grad_sq_accumulate", "vdt_adamw_ema_step",
            "vdt_op_attention_backward", "vdt_op_groupnorm_train", "vdt_op_linear", "vdt_op_timestep_embedding",

@@ -327,4 +327,9 @@ int wgrad_splits(const WgradParams& p, int num_sms);
 // runs the GEMM, the fixed-order split reduction into dw (fp32 OIHW) and, when dbias is given, db[co] = sum_p dY[p][co]
 cudaError_t launch_wgrad(const WgradParams& p, float* dw, float* dbias, const h16* dy, long long rows, cudaStream_t stream);
 
+// The C ABI's error message (vdt_last_error) and launch counter (vdt_kernel_launches) live in plan.cu; entry points defined
+// in other translation units (distill.cu) report through these.  api_fail returns 1, the ABI's error code.
+int api_fail(const char* fmt, ...);
+void api_count_launch();
+
 }  // namespace vdt

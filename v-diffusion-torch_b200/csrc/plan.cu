@@ -31,6 +31,14 @@ static int fail(const char* fmt, ...) {
     va_end(ap);
     return 1;
 }
+int vdt::api_fail(const char* fmt, ...) {
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(g_err, sizeof(g_err), fmt, ap);
+    va_end(ap);
+    return 1;
+}
+void vdt::api_count_launch() { ++g_launches; }
 #define CK(expr)                                                                                         \
     do {                                                                                                 \
         cudaError_t _e = (expr);                                                                         \

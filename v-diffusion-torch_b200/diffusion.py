@@ -515,6 +515,97 @@ class GaussianDiffusion:
                                         _lib.REWEIGHT_TYPES[self.reweight_type], _lib.current_stream_ptr()))
         return (loss, grad) if return_grad else loss
 
+    # ------------------------------------------------------------------ progressive distillation (extension)
+    def distill_coefficients(self, step):
+        """[2, B, 16] fp32 host table of progressive distillation (include/vdt_b200.h: vdt_distill_coefficients) for the
+        student step indices ``step`` (B,) in [0, sample_timesteps): plane 0 at t = (i+1)/N, plane 1 at t' = (2i+1)/(2N)."""
+        step_host = torch.as_tensor(step).detach().to(device="cpu", dtype=torch.int32).reshape(-1).contiguous()
+        sc = self.sampler_config(use_ddim=True)
+        out = torch.empty((2, step_host.numel(), _lib.COEF_STRIDE), dtype=torch.float32)
+        _lib.check(_lib.lib().vdt_distill_coefficients(C.byref(sc), _lib.ptr(step_host), step_host.numel(), _lib.ptr(out)))
+        return out
+
+    @staticmethod
+    def _teacher_rows(z, t, y, use_cfg):
+        """The sampler's CFG layout (diffusion.py:368-372): rows 2b conditional, 2b+1 unconditional."""
+        if not use_cfg:
+            return z, t, y
+        yin = y.repeat_interleave(2, dim=0)
+        yin[1::2] = 0
+        return z.repeat_interleave(2, dim=0), t.repeat_interleave(2), yin
+
+    @torch.no_grad()
+    def distill_loss(self, teacher_fn, student_fn, x_0, step, y, noise=None, w_guide=0., return_grad=False):
+        """Progressive distillation (Salimans & Ho, 2022, Algorithm 2; include/vdt_b200.h vdt_distill_coefficients): the
+        student, sampled with N = ``self.sample_timesteps`` DDIM steps, learns in one step from t = (i+1)/N to t'' = i/N what
+        the teacher does in two DDIM steps on the 2N grid.  ``step``: the student step index i per sample, (B,) in [0, N).
+
+        q_sample at t -> teacher at t -> vdt_op_distill_step (z_t', x1) -> teacher at t' -> vdt_op_distill_target (x~, eps~) ->
+        student at t -> vdt_train_loss with x~ and eps~ as the targets, so every model_out_type and reweight_type works as in
+        train_loss.  The teacher runs with CFG (2B interleaved rows) when ``w_guide`` > 0 and labels are given; the student
+        sees the labels as given.  Both networks may be any callable ``(x, t, y) -> output``.  Returns the per-sample loss (B,)
+        and, with ``return_grad``, d loss.mean() / d student output."""
+        if self.loss_type != "mse":
+            raise NotImplementedError("distillation trains with the mse loss")
+        if self.model_var_type == "learned":
+            raise AssertionError("mse loss needs a fixed variance type")
+        if self.reweight_type not in _lib.REWEIGHT_TYPES:
+            raise AssertionError(self.reweight_type)
+        if x_0.device.type != "cuda":
+            raise RuntimeError("v_diffusion_b200 trains on CUDA (sm_100a) only; there is no CPU fallback")
+        if x_0.ndim != 4:
+            raise ValueError(f"x_0 must have shape (B, C, H, W), got {tuple(x_0.shape)}")
+        dev, B, N = x_0.device, x_0.shape[0], int(self.sample_timesteps)
+        x_0 = x_0.to(torch.float32).contiguous()
+        noise = torch.randn_like(x_0) if noise is None else noise.to(device=dev, dtype=torch.float32).contiguous()
+        if noise.shape != x_0.shape:
+            raise ValueError(f"noise has shape {tuple(noise.shape)}, expected {tuple(x_0.shape)}")
+        step = torch.as_tensor(step).reshape(-1)
+        if step.numel() != B:
+            raise ValueError("step must have one entry per sample")
+        coef = self.distill_coefficients(step).to(dev)                 # refuses steps outside [0, N)
+        step = step.to(device=dev, dtype=torch.float64)
+        t = (step + 1) / N                                              # the sampler's t at N, fp64
+        t_mid = (2 * step + 1) / (2 * N)                                # its t at 2N
+        w = float(w_guide)
+        use_cfg = w > 0 and y is not None
+        out_type = _lib.OUT_TYPES[self.model_out_type]
+        Cc, hw = x_0.shape[1], x_0.shape[2] * x_0.shape[3]
+        Cm = (2 if self.model_out_type == "both" else 1) * Cc
+        L = _lib.lib()
+        if y is not None:
+            y = y.to(dev)
+
+        def teacher(z, tt):
+            out = teacher_fn(*self._teacher_rows(z, tt, y, use_cfg)).to(torch.float32).contiguous()
+            want = (B * (2 if use_cfg else 1), Cm) + tuple(x_0.shape[2:])
+            if tuple(out.shape) != want:
+                raise ValueError(f"teacher output has shape {tuple(out.shape)}, expected {want}")
+            return out
+
+        z_t = torch.empty_like(x_0)
+        with torch.cuda.device(dev):
+            st = _lib.current_stream_ptr()
+            _lib.check(L.vdt_q_sample(_lib.ptr(x_0), _lib.ptr(noise), _lib.ptr(coef), _lib.ptr(z_t), B, Cc * hw, st))
+            out1 = teacher(z_t, t)
+            z_mid, x1 = torch.empty_like(x_0), torch.empty_like(x_0)
+            _lib.check(L.vdt_op_distill_step(_lib.ptr(out1), _lib.ptr(z_t), _lib.ptr(z_mid), _lib.ptr(x1), _lib.ptr(coef), B, Cc, hw,
+                                             int(use_cfg), out_type, w, st))
+            out2 = teacher(z_mid, t_mid)
+            x_tgt, eps_tgt = torch.empty_like(x_0), torch.empty_like(x_0)
+            _lib.check(L.vdt_op_distill_target(_lib.ptr(out2), _lib.ptr(z_mid), _lib.ptr(x1), _lib.ptr(z_t), _lib.ptr(x_tgt),
+                                               _lib.ptr(eps_tgt), _lib.ptr(coef), B, Cc, hw, int(use_cfg), out_type, w, st))
+        model_out = student_fn(z_t, t, y).to(torch.float32).contiguous()
+        if tuple(model_out.shape) != (B, Cm) + tuple(x_0.shape[2:]):
+            raise ValueError(f"student output has shape {tuple(model_out.shape)}, expected {(B, Cm) + tuple(x_0.shape[2:])}")
+        loss = torch.empty((B,), dtype=torch.float32, device=dev)
+        grad = torch.empty_like(model_out) if return_grad else None
+        with torch.cuda.device(dev):
+            _lib.check(L.vdt_train_loss(_lib.ptr(model_out), _lib.ptr(x_tgt), _lib.ptr(eps_tgt), _lib.ptr(z_t), _lib.ptr(coef),
+                                        _lib.ptr(loss), _lib.ptr(grad), B, Cc, hw, out_type, _lib.REWEIGHT_TYPES[self.reweight_type],
+                                        _lib.current_stream_ptr()))
+        return (loss, grad) if return_grad else loss
+
     def _p_sample_generic(self, denoise_fn, shape, x_t, label, step_noise, sc, device, gen, use_ddim, solver=None, inp=None,
                           start_step=None):
         L = _lib.lib()

@@ -696,3 +696,47 @@ class TrainingStep:
             if hasattr(self.model, "mark_weights_changed"):
                 self.model.mark_weights_changed()                       # sampling plans re-pack the updated weights
         return loss
+
+
+class DistillationStep(TrainingStep):
+    """One stage of progressive distillation (Salimans & Ho, 2022): ``student`` learns to sample in N =
+    ``diffusion.sample_timesteps`` DDIM steps what ``teacher`` does in 2N (GaussianDiffusion.distill_loss).  Only ``draw`` and
+    ``loss_and_grads`` differ from TrainingStep, so ``step()``, gradient accumulation, the all-reduce, clip + AdamW + EMA and the
+    checkpoints are the training step's own.
+
+        ds = DistillationStep(student, teacher, diffusion, w_guide=0., lr=1e-4, ema_decay=0.9995)
+        loss = ds.step(x, y)
+
+    The teacher runs in ``.eval()`` on the sampling (plan) path.  With ``w_guide`` = 0 the labels are dropped (set to 0, "no
+    class") with probability ``diffusion.p_uncond`` before either network sees them, so the student keeps its unconditional
+    branch and can still be sampled with CFG.  With ``w_guide`` > 0 the teacher is guided, no label is dropped, and the student
+    learns the guided prediction: sample it with ``w_guide`` = 0."""
+
+    def __init__(self, student, teacher, diffusion, w_guide=0., **kwargs):
+        super().__init__(student, diffusion, **kwargs)
+        self.teacher = teacher.eval()
+        self.w_guide = float(w_guide)
+        if self.w_guide < 0:
+            raise ValueError(f"w_guide must be >= 0, got {w_guide}")
+
+    def draw(self, x):
+        """From the step's generator, in this order: the student step indices i ~ U{0 .. N-1}, the noise, then the label-keep
+        mask (uniforms >= p_uncond; drawn every step, so the stream does not depend on the labels or on w_guide)."""
+        B, N = x.shape[0], int(self.diffusion.sample_timesteps)
+        step = torch.randint(N, size=(B,), device=self.device, generator=self.generator)
+        noise = torch.empty_like(x).normal_(generator=self.generator)
+        keep = torch.rand((B,), device=self.device, generator=self.generator) >= float(self.diffusion.p_uncond or 0.)
+        return step, noise, keep
+
+    @torch.no_grad()
+    def loss_and_grads(self, x, y, step=None, noise=None, keep=None):
+        """Per-sample distillation loss (B,) and the gradients of ``loss.mean()`` w.r.t. every student parameter."""
+        x = x.to(device=self.device, dtype=torch.float32).contiguous()
+        if step is None or noise is None or keep is None:
+            step, noise, keep = self.draw(x)
+        if y is not None and self.w_guide == 0:
+            y = y.to(self.device)
+            y = y * keep.to(y.dtype).reshape((-1,) + (1,) * (y.ndim - 1))
+        loss, grad_out = self.diffusion.distill_loss(self.teacher, self.graph.forward, x, step, y, noise=noise,
+                                                     w_guide=self.w_guide, return_grad=True)
+        return loss, self.graph.backward(grad_out)
